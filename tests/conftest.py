@@ -1,3 +1,4 @@
+import hashlib
 import json
 import os
 import sys
@@ -25,9 +26,44 @@ def pytest_collection_modifyitems(config, items):
             item.add_marker(skip)
 
 
+def fingerprint(a):
+    """sha256 of an array's dtype, shape and bytes (tests/golden/make_golden.py records these for the arrays it does not store)."""
+    a = np.ascontiguousarray(a)
+    return hashlib.sha256(f"{a.dtype.str}{a.shape}".encode() + a.tobytes()).hexdigest()
+
+
+def seeded_draws(seed, B, J, H):
+    """The inputs tests/golden/make_golden.py draws from RandomState(seed) for the reference, in the order it draws them."""
+    rs = np.random.RandomState(seed)
+    d = {}
+    d["a5_uvd"] = rs.uniform(-0.9, 0.9, (B, J, 3))
+    d["a10_joint"] = rs.uniform(-0.7, 0.7, (B, J, 3))
+    d["a16_feature2joint_in_w"] = rs.standard_normal((B, J, H, H))
+    d["a13_anchor"] = rs.standard_normal((B, J, 128))
+    d["a13_key"] = rs.standard_normal((B, J, 128))
+    d["a13_mha_q"] = rs.standard_normal((J, B, 128))
+    d["a13_mha_k"] = rs.standard_normal((9, B, 128))
+    for name in ("rgbd", "ac"):
+        d[f"a14_{name}_rgb"] = rs.standard_normal((B, 64, 8, 8))
+        d[f"a14_{name}_depth"] = rs.standard_normal((B, 64, 8, 8))
+    return {k: v.astype(np.float32) for k, v in d.items()}
+
+
 @pytest.fixture(scope="session")
-def golden():
-    return dict(np.load(os.path.join(GOLDEN, "golden_path.npz")))
+def golden(golden_meta):
+    """The reference's outputs (golden_path.npz, golden_maps.npz) plus the seeded inputs it was fed, regenerated here, and the
+    copies it produced bit-identically twice, stored once; both are checked against the fingerprints of what the reference saw."""
+    m = golden_meta
+    d = {}
+    for name in ("golden_path.npz", "golden_maps.npz"):
+        d.update(np.load(os.path.join(GOLDEN, name)))
+    for k, v in seeded_draws(m["seed"], m["B"], m["J"], m["S"] // 4).items():
+        assert fingerprint(v) == m["seeded_sha256"][k], f"seeded draw {k} differs from the one the reference was fed"
+        d[k] = v
+    for k, (src, sha) in m["copies_sha256"].items():
+        assert fingerprint(d[src]) == sha, f"{k} is not a bit-identical copy of {src}"
+        d[k] = d[src]
+    return d
 
 
 @pytest.fixture(scope="session")

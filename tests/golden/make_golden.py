@@ -191,6 +191,18 @@ def main():
         out[f"b{i}_cross"] = npy(caps[f"b{i}_cross"])
         jx = r2d
 
+    # stored compactly, no fixture file above 1 MB: the inputs drawn from `rs` above are regenerated by tests/conftest.py, the
+    # outputs the reference computes identically twice are stored once, and the per-cell joint maps go to a file of their own
+    sys.path.insert(0, os.path.dirname(HERE))
+    from conftest import fingerprint, seeded_draws
+    meta["seeded_sha256"] = {}
+    for k, v in seeded_draws(SEED, B, J, H).items():
+        assert np.array_equal(out[k], v) and out[k].dtype == v.dtype, k
+        meta["seeded_sha256"][k] = fingerprint(out.pop(k))
+    meta["copies_sha256"] = {}
+    for k, src in (("a4_joint_uvd_gfm", "a4_joint_uvd"), ("a7_pcl_offset_gfm", "a7_pcl_offset"), ("a16_joint2feature", "a16_joint2offset_gfm")):
+        meta["copies_sha256"][k] = [src, fingerprint(out.pop(k))]
+    np.savez_compressed(os.path.join(HERE, "golden_maps.npz"), **{k: out.pop(k) for k in ("a10_hm_s1", "a10_hm_default", "a11_gam")})
     np.savez_compressed(os.path.join(HERE, "golden_path.npz"), **out)
     with open(os.path.join(HERE, "golden_meta.json"), "w") as f:
         json.dump(meta, f, indent=0, sort_keys=True)
