@@ -191,7 +191,7 @@ int kpf_token_stack(const float* x, const float* y, const float* r3d, const floa
                     const void* wseq, const float* wvec, int n_weights, int cross, int pre, int B, int J, int D, int L, int F, int Fc,
                     int fmt, float* tokens_out, float* pred_out, float* out_cj, float* out_jc, int out_jc_stride, int out_jc_c0,
                     const void* peer_bases, const int* xstep, int world, int row0, int rows_total /* fused exchange step, see below */,
-                    long long* dbg /* NULL, or 64 x int64 device: clock64 stamps of CTA 0 (profiling aid) */, cudaStream_t stream);
+                    cudaStream_t stream);
 
 /* ---- the path's one exchange step, fused into the kernel that produces the joints (SURVEY.md 2b row C1; the reference gathers through
  * DataParallel, train.py:81).  Every rank owns an exchange buffer at the SAME offsets in peer-accessible (symmetric) memory:
@@ -230,7 +230,7 @@ int kpf_point_embed(const void* feat_hi, const void* feat_lo, const int32_t* idx
                     const int32_t* order, const void* wmat, const float* wvec, int B, int N, int J, int HW, float kernel_size, int fmt,
                     void* e_out,
                     long long e_batch_stride /* 16-bit elements between samples of e_out, >= N*256; (N+J)*256 or more when kpf_desa_fused follows */,
-                    float* part_acc, float* part_ms, void* stage_out, const void* stage_in, int num_sms, long long* dbg, cudaStream_t stream);
+                    float* part_acc, float* part_ms, void* stage_out, const void* stage_in, int num_sms, cudaStream_t stream);
 
 /* ---- 8f-1 DESA on tensor cores (csrc/desa_fused.cu), model/model.py:129-204 + joint embeddings :323-325 ---------------
  * e / part_acc / part_ms: outputs of kpf_point_embed; pcl [B,N,3]; joint [B,J,3]; S scales with radii r0..r3 and
@@ -247,7 +247,7 @@ int kpf_desa_fused(void* e, long long e_batch_stride, const float* part_acc, con
                    const void* wmat, const float* wvec, int B, int N, int J, int S, int nsample, float r0, float r1, float r2, float r3,
                    int fmt, const float* jf_in /* NULL, or [B,J,128]: joint features given (stand-alone DESA.forward, model.py:166); the
                    joint embedding is skipped and part_acc / part_ms may be NULL */,
-                   float* desa_part, float* jf_out, void* scratch, int num_sms, long long* dbg, cudaStream_t stream);
+                   float* desa_part, float* jf_out, void* scratch, int num_sms, cudaStream_t stream);
 
 /* ---- a12 on tensor cores (csrc/spatial_agg_tc.cu): same contract as kpf_spatial_aggregate for feat_rgb [B,128,fs,fs] with
  * fs*fs % 128 == 0, given as bf16 (feat_rgb_lo = NULL: exact in one plane) or as the two bf16 planes of an fp32 map
@@ -260,7 +260,7 @@ int kpf_spatial_aggregate_tc(const void* feat_rgb, const void* feat_rgb_lo, cons
                              const void* wa_packed, const float* ba, const float* weight_dis, const float* fc_w, const float* fc_b,
                              const float* prev, int B, int C, int J, int fs, float img_size, float flip, float hm_std, float hm_sigma,
                              float gamma, int fmt, float* sw_out, float* feat_j_out, float* scratch, int* counters, int split,
-                             long long* dbg, cudaStream_t stream);
+                             cudaStream_t stream);
 
 /* x [n] f32 -> hi [n] bf16 = rn(x), lo [n] bf16 = rn(x - hi): how an fp32 feature map enters the split-precision kernels. n % 4 == 0. */
 int kpf_split_planes(const float* x, long long n, void* hi, void* lo, cudaStream_t stream);
@@ -293,22 +293,6 @@ int kpf_umma_selftest(const void* A, const void* B, float* D, int N, int K, int 
  * cycles (2 x int64 device, may be NULL): one GEMM issue -> completion, eight GEMMs back to back. */
 int kpf_umma_split_selftest(const float* A, const float* B, float* D, int N, int K, int fmt, int a_tmem, int a_exact, long long* cycles,
                             cudaStream_t stream);
-
-/* TMA row gather self-test (csrc/tma_gather.cuh): table = [rows][256] 16-bit ([hi 128 | lo 128] fp16 planes of a [rows][128] fp32
- * matrix X), idx [N] i32 -> D[128,N] f32 = A[128,128] X[idx]^T.  The rows are fetched with cp.async.bulk.tensor ... tile::gather4
- * (four rows per instruction, 128-byte swizzle) and consumed as a SWIZZLE_128B K-major operand.  N % 16 == 0, N <= 256.
- * a_tmem: A operand planes read from tensor memory instead of shared memory.
- * cycles (4 x int64 device, may be NULL): the gather (cold), one GEMM (24 MMAs), the gather repeated (L2-hot), eight GEMMs. */
-int kpf_tma_gather_selftest(const void* table, long long rows, const float* A, const int* idx, float* D, int N, int a_tmem, long long* cycles,
-                            cudaStream_t stream);
-
-/* cycle probe of 512-byte row gathers into shared memory (profiles/probe_gather.py): every one of `ctas` CTAs gathers n_rows rows
- * (idx [ctas][n_rows] i32) four times; out[cta] = cycles of the last repetition.  mode 0 TMA gather4, 1 bulk 512 B copies,
- * 2 cp.async (128-byte requests), 3 LDG.128 + STS, 4 cp.async (a row per warp instruction). */
-int kpf_gather_probe(const void* table, long long rows, const int* idx, int n_rows, int ctas, int mode, long long* out, cudaStream_t stream);
-
-/* cycle micro-benchmarks of the tcgen05 building blocks (out: 8 x int64 device; see csrc/umma_probe.cu) */
-int kpf_umma_probe(long long* out, int N, int K, int reps, cudaStream_t stream);
 
 #ifdef __cplusplus
 }

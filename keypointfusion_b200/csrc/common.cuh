@@ -34,13 +34,6 @@ namespace kpf {
 __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
 __device__ __forceinline__ void pdl_launch_dependents() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
 
-inline bool pdl_enabled() {
-    static const bool on = [] {
-        const char* e = getenv("KPF_PDL");
-        return !(e && e[0] == '0');
-    }();
-    return on;
-}
 template <typename... KArgs, typename... Args>
 inline cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t stream, Args... args) {
     cudaLaunchConfig_t cfg = {};
@@ -52,7 +45,7 @@ inline cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, s
     attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     attr[0].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = attr;
-    cfg.numAttrs = pdl_enabled() ? 1 : 0;
+    cfg.numAttrs = 1;
     return cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...);
 }
 }  // namespace kpf

@@ -45,10 +45,7 @@ struct DesaParams {
     uint16_t* idx;            // scratch [B,S,J,nsample] ball-query indices (>= N: one of the joints)
     int* gw;                  // scratch [B,S]: the largest ball population (capped at nsample) among the sample's J balls of a scale
     int B, N, J, T, S, nsample, fmt;
-    int probe;                // profiling aid (KPF_DESA_PROBE): bit 0 = skip the row copies, bit 1 = skip the MMAs (results are garbage),
-                              //   bit 2 = row copy as one burst, bit 3 = always group nsample rows per joint (no narrow groups)
     float radius[4];
-    long long* dbg;
 };
 
 constexpr int DS_NT = 512;
@@ -64,12 +61,6 @@ __global__ void __launch_bounds__(DS_NT, 1) desa_prep_kernel(const DesaParams p)
     extern __shared__ __align__(128) unsigned char ds_smem[];
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     const int J = p.J, N = p.N, T = p.T, NS = p.nsample, S = p.S;
-    int n_stamp = 0;
-    auto stamp = [&]() {
-        if (p.dbg && (blockIdx.x == 0 || (int)blockIdx.x == p.B) && tid == 0 && n_stamp < 8) p.dbg[(blockIdx.x == 0 ? 0 : 8) + n_stamp] = clock64();
-        ++n_stamp;
-    };
-    stamp();
     pdl_launch_dependents();
 
     if ((int)blockIdx.x >= p.B) {
@@ -87,7 +78,6 @@ __global__ void __launch_bounds__(DS_NT, 1) desa_prep_kernel(const DesaParams p)
         }
         __syncthreads();
         for (int i = tid; i < N + J; i += DS_NT) p.xyz4[(size_t)b * (N + 32) + i] = sPcl[i];
-        stamp();
         // Phase 1: thread = (32-point word, centre): lane = centre j, warp = word.  Every lane walks the word's 32 points (one
         // broadcast shared-memory read per point), computes d2 ONCE in the exact fp32 op order and sets the point's bit in the hit
         // word of every scale whose r^2 it is under.  No ballots, no cross-lane traffic; hit word layout sMask[(sc J + j) NW + word].
@@ -118,7 +108,6 @@ __global__ void __launch_bounds__(DS_NT, 1) desa_prep_kernel(const DesaParams p)
             }
         }
         __syncthreads();
-        stamp();
         // Phase 2: one warp per centre: popcount prefix over its hit words, then every lane expands the set bits of its word(s)
         // into their slots
         for (int pj = warp; pj < S * J; pj += DS_NT / 32) {   // pj = sc * J + j: the layout of sMask and of idx[b]
@@ -158,7 +147,6 @@ __global__ void __launch_bounds__(DS_NT, 1) desa_prep_kernel(const DesaParams p)
         // the widest ball of each scale: the tile kernel groups only as many rows per joint as the widest ball of the launch needs
         __syncthreads();
         if (tid < S) p.gw[(size_t)b * S + tid] = sGw[tid];
-        stamp();
         return;
     }
 
@@ -217,7 +205,6 @@ __global__ void __launch_bounds__(DS_NT, 1) desa_prep_kernel(const DesaParams p)
         sMS[T * 64 + tid] = den;
     }
     __syncthreads();
-    stamp();
     // ---- joint_agg[c][j] (softmax over all N points of the gathered weight map): 8 lanes read one channel's 128-byte row of
     //      a partial per load (4 L1 wavefronts per warp load); thread = (channel, 4 joints), two channel halves
     if (!given) {
@@ -259,7 +246,6 @@ __global__ void __launch_bounds__(DS_NT, 1) desa_prep_kernel(const DesaParams p)
             __syncwarp();
         }
     }
-    stamp();
     if (!given) {
         mbar_wait(&mma_bar, mph);
         mph ^= 1;
@@ -367,7 +353,6 @@ __global__ void __launch_bounds__(DS_NT, 1) desa_prep_kernel(const DesaParams p)
             if (j < J) p.cj[(((size_t)b * S + 3) * J + j) * 128 + ch] = d[i];
         }
     }
-    stamp();
     tc_fence_before();
     __syncthreads();
     if (warp == 0) tmem_dealloc(tmem0, 128);
@@ -412,12 +397,6 @@ __global__ void __launch_bounds__(DS_TILE_NT, 1) desa_tile_kernel(const DesaPara
     int ns_shift = 31 - __clz(NS);                                // NS is a power of two: joint of tile row x = x >> ns_shift
     const uint32_t ACC1 = 0, ACC2 = 128, TW1_HI = 256, TW1_LO = 320, TW2_HI = 384, TW2_LO = 448;   // TMEM columns
     constexpr int fmt = FMT;
-    int n_stamp = 0;
-    auto stamp = [&]() {
-        if (p.dbg && blockIdx.x == 0 && tid == 0 && n_stamp < 48) p.dbg[16 + n_stamp] = clock64();
-        ++n_stamp;
-    };
-    stamp();
     pdl_launch_dependents();
     if (warp == 0) tmem_alloc(&tmem_slot, 512);
     if (tid == 0) {
@@ -441,7 +420,7 @@ __global__ void __launch_bounds__(DS_TILE_NT, 1) desa_tile_kernel(const DesaPara
         for (int sc = 0; sc < S; ++sc) {
             int n = 16;
             while (n < sGw[sc]) n <<= 1;
-            if (n > NSTRIDE || (p.probe & 8)) n = NSTRIDE;
+            if (n > NSTRIDE) n = NSTRIDE;
             sNs[sc] = n;
             sBase[sc] = base;
             const int jpt = 128 / n;
@@ -503,9 +482,8 @@ __global__ void __launch_bounds__(DS_TILE_NT, 1) desa_tile_kernel(const DesaPara
     // next shared-memory / TMEM / global instruction -- i.e. the epilogues -- queues up behind it.  Measured per launch, the kernel alone
     // over L2-resident rows (profiles/probe_kernels.py, same box): one burst 84.1 us, two halves 81, four parts 77.0, eight parts 74.8
     // (with the copy switched off: 57 us).  Inside the running step (four steps in flight, rows partly from DRAM) the gain is within
-    // the run-to-run noise: 0.497 vs 0.501 ms per step, means of three alternating runs (KPF_DESA_PROBE=4 restores the burst).
+    // the run-to-run noise: 0.497 vs 0.501 ms per step, means of three alternating runs.
     DesaItem it_copy = {0, 0, 0};
-    const bool burst = (p.probe & 4) != 0;   // A/B switch (KPF_DESA_PROBE=4): the whole copy at the point of part 0, as one burst
     auto copy_one = [&](int item, int part) {
         if (part == 0) {
             it_copy = c_rows;
@@ -520,8 +498,7 @@ __global__ void __launch_bounds__(DS_TILE_NT, 1) desa_tile_kernel(const DesaPara
         // 16-byte chunk 8k + g8 of the 512-byte row [hi 128 | lo 128]: k-chunk (8k + g8) & 15 of plane k >> 1; the eight g8 lanes of a row
         // read 128 contiguous bytes = ONE request.  (.cg: the rows stream through L2 only -- measured 9 % faster than .ca, whose L1 is
         // ~30 KB next to 225 KB of shared memory.)  Rows beyond the last joint are zero filled (src-size 0).
-        if (!(p.probe & 1))
-            asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;" ::"r"(smem_u32(X + (k >> 1) * 2048 + (k & 1) * 64)), "l"(src + 64 * k), "r"(nbytes) : "memory");
+        asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;" ::"r"(smem_u32(X + (k >> 1) * 2048 + (k & 1) * 64)), "l"(src + 64 * k), "r"(nbytes) : "memory");
         if (k == 0 && g8 == 0) {   // xyz of the row's point and of its centre -> staging; the tail is built from it one iteration later
             const float4* tab = p.xyz4 + (size_t)it_copy.b * (N + 32);
             float4* st = sXyz + ((item & 1) * 128 + row) * 2;
@@ -530,14 +507,6 @@ __global__ void __launch_bounds__(DS_TILE_NT, 1) desa_tile_kernel(const DesaPara
             tail_ok[h] = ok;
         }
         if (part == 7) asm volatile("cp.async.commit_group;" ::: "memory");
-    };
-    auto copy_part = [&](int item, int part) {
-        if (!burst) {
-            copy_one(item, part);
-        } else if (part == 0) {
-#pragma unroll
-            for (int q8 = 0; q8 < 8; ++q8) copy_one(item, q8);
-        }
     };
     auto store_tail = [&](int item) {   // group_xyz_norm = (xyz[idx] - centre) / radius   model.py:177
         if (g8 != 0) return;
@@ -629,10 +598,10 @@ __global__ void __launch_bounds__(DS_TILE_NT, 1) desa_tile_kernel(const DesaPara
                             a.hi = tmem0 + TW1_HI; a.lo = tmem0 + TW1_LO;
                             SmemOp xb, ta, tb;
                             xb.hi = X; xb.lo = X + 2048 * 16; xb.lbo = 128; xb.sbo = 2048;
-                            if (!(p.probe & 2)) umma_gemm3_ts(tmem0 + ACC1, a, xb, id128, 128, false);
+                            umma_gemm3_ts(tmem0 + ACC1, a, xb, id128, 128, false);
                             ta.hi = smem_u32(sW1t); ta.lo = ta.hi + 256 * 16; ta.lbo = 2048; ta.sbo = 128;
                             tb.hi = X + 4096 * 16; tb.lo = tb.hi + 128 * 16; tb.lbo = 0; tb.sbo = 128;   // lbo 0: k-chunk 1 (zero weights) re-reads chunk 0
-                            if (!(p.probe & 2)) umma_gemm3_ss(tmem0 + ACC1, ta, tb, id128, 16, true);
+                            umma_gemm3_ss(tmem0 + ACC1, ta, tb, id128, 16, true);
                             umma_commit(&g1_bar);
                         }
                         if (s >= i0) {   // layer 2 of tile s: D2[c][row] = W2 h
@@ -640,7 +609,7 @@ __global__ void __launch_bounds__(DS_TILE_NT, 1) desa_tile_kernel(const DesaPara
                             a.hi = tmem0 + TW2_HI; a.lo = tmem0 + TW2_LO;
                             SmemOp hb;
                             hb.hi = smem_u32(sX + (s % 3) * DS_XBUF); hb.lo = hb.hi + 2048 * 16; hb.lbo = 2048; hb.sbo = 128;
-                            if (!(p.probe & 2)) umma_gemm3_ts(tmem0 + ACC2, a, hb, umma_idesc_f16(128, 128, false, true, fmt, fmt), 128, false);
+                            umma_gemm3_ts(tmem0 + ACC2, a, hb, umma_idesc_f16(128, 128, false, true, fmt, fmt), 128, false);
                             umma_commit(&g2_bar);
                         }
                     }
@@ -652,8 +621,8 @@ __global__ void __launch_bounds__(DS_TILE_NT, 1) desa_tile_kernel(const DesaPara
             if (!issuer) {
                 // gather side: rows of tile s + 2 (its buffer held tile s - 1, whose layer 2 every thread waited for in the previous
                 // iteration), indices of s + 3
-                const bool fine = s + 2 < i1;   // tile s + 2 exists: its row copy is issued in eight parts across this iteration (copy_part)
-                if (fine) copy_part(s + 2, 0);
+                const bool fine = s + 2 < i1;   // tile s + 2 exists: its row copy is issued in eight parts across this iteration (copy_one)
+                if (fine) copy_one(s + 2, 0);
                 // layer-1 bias of tile s + 1 minus the W1 jf term of the joint this thread's 32 rows belong to
                 float cjv[2] = {0.f, 0.f};   // per 16-row half (two joints when NS = 16); loaded here, consumed after the layer-2 epilogue
                 if (s >= i0 - 1 && s + 1 < i1) {
@@ -664,8 +633,8 @@ __global__ void __launch_bounds__(DS_TILE_NT, 1) desa_tile_kernel(const DesaPara
                     advance(c_epi);
                 }
                 if (fine) {
-                    copy_part(s + 2, 1);
-                    copy_part(s + 2, 2);
+                    copy_one(s + 2, 1);
+                    copy_one(s + 2, 2);
                 }
                 if (s >= i0 - 1 && s + 1 < i1) {   // layer-1 epilogue of tile s + 1: h[c][row] = relu(D1 + b1) -> MN-major B operand, in place
                     mbar_wait(&g1_bar, g1_phase);
@@ -686,11 +655,11 @@ __global__ void __launch_bounds__(DS_TILE_NT, 1) desa_tile_kernel(const DesaPara
                             H[(ch >> 3) * 128 + (4 * cg + 2 * hf + c) * 8 + (ch & 7)] = hh;
                             H[2048 + (ch >> 3) * 128 + (4 * cg + 2 * hf + c) * 8 + (ch & 7)] = hl;
                         }
-                        if (fine) copy_part(s + 2, 3 + hf);
+                        if (fine) copy_one(s + 2, 3 + hf);
                     }
                 } else if (fine) {
-                    copy_part(s + 2, 3);
-                    copy_part(s + 2, 4);
+                    copy_one(s + 2, 3);
+                    copy_one(s + 2, 4);
                 }
                 if (s >= i0) {   // layer-2 epilogue of tile s: max over this thread's 32 grouped points  (model.py:197-198)
                     mbar_wait(&g2_bar, g2_phase);
@@ -703,7 +672,7 @@ __global__ void __launch_bounds__(DS_TILE_NT, 1) desa_tile_kernel(const DesaPara
                         tmem_ld<16>(tmem + ACC2 + 32 * cg + 16 * hf, a);
 #pragma unroll
                         for (int i = 0; i < 16; ++i) mx[hf] = fmaxf(mx[hf], a[i]);
-                        if (fine) copy_part(s + 2, 5 + hf);
+                        if (fine) copy_one(s + 2, 5 + hf);
                     }
                     if (!direct) {
                         sPart[(s & 1) * 512 + cg * 128 + ch] = fmaxf(fmaxf(mx[0], mx[1]) + b2, 0.f);   // max_i relu(a_i + b2)
@@ -721,19 +690,17 @@ __global__ void __launch_bounds__(DS_TILE_NT, 1) desa_tile_kernel(const DesaPara
                     }
                     tc_fence_before();
                 } else if (fine) {
-                    copy_part(s + 2, 5);
-                    copy_part(s + 2, 6);
+                    copy_one(s + 2, 5);
+                    copy_one(s + 2, 6);
                 }
-                if (fine) copy_part(s + 2, 7);
+                if (fine) copy_one(s + 2, 7);
                 if (s + 3 < i1) fetch_idx();
             }
-            if (s <= i0 + 3) stamp();
         }
         __syncthreads();
         if (!direct) store_max(i1 - 1);
         w_phase ^= 1;
         i0 = i1;
-        stamp();
     }
     tc_fence_before();
     __syncthreads();
@@ -745,7 +712,7 @@ __global__ void __launch_bounds__(DS_TILE_NT, 1) desa_tile_kernel(const DesaPara
 extern "C" int kpf_desa_fused(void* e, long long e_batch_stride, const float* part_acc, const float* part_ms, const float* pcl, const float* joint,
                               const void* wmat, const float* wvec, int B, int N, int J, int S, int nsample, float r0, float r1, float r2,
                               float r3, int fmt, const float* jf_in, float* desa_part, float* jf_out, void* scratch, int num_sms,
-                              long long* dbg, cudaStream_t stream) {
+                              cudaStream_t stream) {
     using namespace kpf;
     KPF_REQUIRE(B >= 0 && N >= 64 && N % 64 == 0 && N + J <= 65535 && J >= 1 && J <= 32 && S >= 1 && S <= 4);
     KPF_REQUIRE(nsample == 32 || nsample == 64 || nsample == 128);
@@ -757,13 +724,8 @@ extern "C" int kpf_desa_fused(void* e, long long e_batch_stride, const float* pa
     KPF_REQUIRE(e_batch_stride >= (long long)(N + J) * 256 && e_batch_stride % 8 == 0);
     KPF_REQUIRE(jf_in != nullptr || (part_acc != nullptr && part_ms != nullptr));
     p.fmt = fmt; p.jf_in = jf_in;
-    {
-        const char* pe = getenv("KPF_DESA_PROBE");   // read per call (a captured graph keeps the value of its capture)
-        p.probe = pe ? atoi(pe) : 0;
-    }
     p.e = (uint16_t*)e; p.e_bs = e_batch_stride; p.part_acc = part_acc; p.part_ms = part_ms; p.pcl = pcl; p.joint = joint; p.wmat = (const uint4*)wmat;
     p.wvec = wvec; p.desa_part = desa_part; p.jf_out = jf_out; p.B = B; p.N = N; p.J = J; p.T = N / 64;   /* kpf_point_embed's tile = 64 points */ p.S = S; p.nsample = nsample;
-    p.dbg = dbg;
     p.radius[0] = r0; p.radius[1] = r1; p.radius[2] = r2; p.radius[3] = r3;
     p.cj = (float*)scratch;
     p.xyz4 = (float4*)((char*)scratch + (size_t)B * S * J * 128 * 4);

@@ -628,24 +628,16 @@ extern "C" int kpf_img2pcl_index(const float* pcl, const float* depth, long long
     // (row quarters per point group, threads per CTA): measured at batch 64, S = 128, K = 4 (profiles/probe_k2.py): (1, 256) 43.4 us,
     // (2, 256) 39.4, (2, 512) 36.7, (4, 512) 49.9, (4, 1024) 48.8 -- two warps per point group pay for their second window seeding and
     // the merge, four do not; seeding each warp only from the window rows it scans itself (no redundant seeding) loosens the bound and
-    // is far slower (49 / 86 us with two / four warps).  KPF_K2_VARIANT=1 selects (1, 256) for comparison (the other variants are not compiled in).
-    static const int variant = [] { const char* e = getenv("KPF_K2_VARIANT"); return e ? atoi(e) : 0; }();
-    const int RQ = variant == 1 ? 1 : 2;
-    const int NT = variant == 1 ? 256 : 512;
-    const int PTS = NT / RQ;
+    // is far slower (49 / 86 us with two / four warps).
+    constexpr int RQ = 2, NT = 512, PTS = NT / RQ;
     dim3 grid((N + PTS - 1) / PTS, B);
     const size_t smem = ((size_t)fs * fs + 2 * (size_t)fs) * sizeof(float4) + (size_t)(NT / 32 / RQ) * (RQ - 1) * K * 32 * 8;
-#define KPF_LAUNCH_K2V(KK, RQV, NTV)                                                                                         \
-    {                                                                                                                        \
-        cudaError_t e = kpf::set_smem(nearest_cells_kernel<KK, RQV, NTV>, smem);                                             \
-        if (e != cudaSuccess) return (int)e;                                                                                 \
-        nearest_cells_kernel<KK, RQV, NTV><<<grid, NTV, smem, stream>>>(pcl, depth, depth_bs, depth_rs, depth_cs, center, M, cube, cam, N, \
-                                                                       fs, img_size, flip, order, closeness, index64, index32); \
-    }
 #define KPF_LAUNCH_K2(KK)                                                                                                    \
     case KK: {                                                                                                               \
-        if (variant == 1) KPF_LAUNCH_K2V(KK, 1, 256)                                                                         \
-        else KPF_LAUNCH_K2V(KK, 2, 512)                                                                                      \
+        cudaError_t e = kpf::set_smem(nearest_cells_kernel<KK, RQ, NT>, smem);                                               \
+        if (e != cudaSuccess) return (int)e;                                                                                 \
+        nearest_cells_kernel<KK, RQ, NT><<<grid, NT, smem, stream>>>(pcl, depth, depth_bs, depth_rs, depth_cs, center, M, cube, cam, N, \
+                                                                     fs, img_size, flip, order, closeness, index64, index32);   \
     } break;
     switch (K) {
         KPF_LAUNCH_K2(1)
@@ -662,7 +654,6 @@ extern "C" int kpf_img2pcl_index(const float* pcl, const float* depth, long long
             return KPF_ERR_UNSUPPORTED;
     }
 #undef KPF_LAUNCH_K2
-#undef KPF_LAUNCH_K2V
     KPF_CHECK_LAUNCH();
     return 0;
 }
@@ -678,14 +669,13 @@ extern "C" int kpf_offset2joint_weight(const void* offset, int dtype, const floa
     } else if (dtype == KPF_BF16 && fs * fs == 8 * 128 && fs % 8 == 0 && ((uintptr_t)offset % 16) == 0) {
         // joints per CTA: 7 amortise the per-CTA setup best once the grid fills the GPU several times over (batch 512: 37 us vs 41 us,
         // 3.0 TB/s); 3 keep enough CTAs at small batches (batch 64: 8.7 us vs 10.1 us) -- profiles/probe_k4a.py
-        static const int variant = [] { const char* e = getenv("KPF_K4A_VARIANT"); return e ? atoi(e) : 0; }();   // tuning aid: 1 / 2 force
 #define KPF_K4A(JPC, MINB)                                                                                                   \
     do {                                                                                                                     \
         kpf::set_smem(offset2joint_bf16x8_kernel<JPC, MINB>, 0);                                                             \
         grid.x = (J + JPC - 1) / JPC;                                                                                        \
         offset2joint_bf16x8_kernel<JPC, MINB><<<grid, 128, 0, stream>>>((const __nv_bfloat16*)offset, depth, S, J, fs, kernel_vec, joint_out); \
     } while (0)
-        const bool big = variant == 2 || (variant == 0 && (long long)B * ((J + 6) / 7) >= 4 * 148);
+        const bool big = (long long)B * ((J + 6) / 7) >= 4 * 148;
         if (big) KPF_K4A(7, 4);
         else KPF_K4A(3, 5);
 #undef KPF_K4A

@@ -108,9 +108,7 @@ struct PointParams {
     unsigned char* stage_out;
     const unsigned char* stage_in;
     int B, N, J, HW, fmt;
-    int probe;               // profiling aid (KPF_PE_PROBE): bit 0 = gather from row 0 only (L1 hits), bit 1 = skip the main MMAs
     float kernel_size;
-    long long* dbg;
 };
 
 __device__ __forceinline__ void bf16x8_fma(float* acc, const uint4& v, float w) {
@@ -207,13 +205,6 @@ __global__ void __launch_bounds__(PE_NT, 1) point_embed_kernel(const PointParams
         tmem_wait_st();
     }
     uint32_t phase = 0;
-    const float inv_ks = 1.f / p.kernel_size;
-    int n_stamp = 0;
-    auto stamp = [&]() {
-        if (p.dbg && blockIdx.x == 0 && tid == 0 && n_stamp < 64) p.dbg[n_stamp] = clock64();
-        ++n_stamp;
-    };
-    stamp();
 
     // per-point inputs of the tile about to be gathered (prefetched during the previous tile's MMAs)
     int4 id = make_int4(0, 0, 0, 0);
@@ -252,12 +243,6 @@ __global__ void __launch_bounds__(PE_NT, 1) point_embed_kernel(const PointParams
     for (int tile = blockIdx.x; tile < p.B * T; tile += gridDim.x) {
         const int b = tile / T, t = tile - b * T;
         __syncthreads();  // previous tile's readers of sJ / sRed / sT / sE are done (its MMAs were waited for)
-        if (tid < J) {
-            sJ[4 * tid] = p.joint[((size_t)b * J + tid) * 3];
-            sJ[4 * tid + 1] = p.joint[((size_t)b * J + tid) * 3 + 1];
-            sJ[4 * tid + 2] = p.joint[((size_t)b * J + tid) * 3 + 2];
-        }
-        stamp();
         // ---- K3: 4-tap gathers of this thread's chunks of the 36-chunk row: grp 0 -> depth 0-15 (A1 chunks 0-15) and weight map
         //      32-35 (A1 chunks 16-19 and the softmax); grp 1 -> rgb 16-31 (A2 chunks 0-15)
         float wraw[8];   // grp 0: gathered weight-map channels [8 sub, 8 sub + 8) of this point
@@ -272,7 +257,6 @@ __global__ void __launch_bounds__(PE_NT, 1) point_embed_kernel(const PointParams
             }
         } else {
             const size_t rb = (size_t)b * p.HW;
-            if (p.probe & 1) id = make_int4(0, 0, 0, 0);
             const uint4 *h0 = p.feat_hi + (rb + id.x) * PE_CH, *h1 = p.feat_hi + (rb + id.y) * PE_CH, *h2 = p.feat_hi + (rb + id.z) * PE_CH,
                         *h3 = p.feat_hi + (rb + id.w) * PE_CH;
             const int nload = grp == 0 ? 5 : 4, c_base = grp == 0 ? 0 : 16;
@@ -331,13 +315,19 @@ __global__ void __launch_bounds__(PE_NT, 1) point_embed_kernel(const PointParams
 #pragma unroll
             for (int k = 0; k < 8; ++k) wraw[k] = acc[4][k];
         }
+        // the sample's joints for K4b, stored after the gather: the gather runs at the 128-register cap, and values held across it
+        // (these, 1 / kernel_size) spill
+        if (tid < J) {
+            sJ[4 * tid] = p.joint[((size_t)b * J + tid) * 3];
+            sJ[4 * tid + 1] = p.joint[((size_t)b * J + tid) * 3 + 1];
+            sJ[4 * tid + 2] = p.joint[((size_t)b * J + tid) * 3 + 2];
+        }
         // softmax over the tile's points, step 1: the gathered weights, transposed, for the per-joint maxima
         if (grp == 0 && !ST_IN) {
 #pragma unroll
             for (int k = 0; k < 8; ++k)
                 if (8 * sub + k < J) sT[(8 * sub + k) * 65 + r] = wraw[k];
         }
-        stamp();
         if (ST_OUT) fence_proxy_async();   // the operand chunks and sT are read by the bulk stores below (async proxy)
         __syncthreads();  // sJ, sT visible
         if (ST_OUT && warp == 0 && lane < 18) {   // store this tile's gathered image for a later launch (the 18 runs load_stage reads)
@@ -352,6 +342,7 @@ __global__ void __launch_bounds__(PE_NT, 1) point_embed_kernel(const PointParams
         //      chunk lanes x two groups) take three items each.  fp32-exact sqrt / divisions: the values feed a split-precision operand.
         {
             const int u = sub + 4 * grp;
+            const float inv_ks = 1.f / p.kernel_size;
 #pragma unroll
             for (int jj = 0; jj < 3; ++jj) {
                 const int j = 3 * u + jj;
@@ -390,7 +381,6 @@ __global__ void __launch_bounds__(PE_NT, 1) point_embed_kernel(const PointParams
             for (int o = 1; o < 16; o <<= 1) m = fmaxf(m, __shfl_xor_sync(0xffffffffu, m, o));
             if (rs == 0) sRed[rj] = rj < J ? m : -INFINITY;
         }
-        stamp();
         // the bulk stores have read their sources: sT is rewritten after the barrier below, the operands by the next tile
         if (ST_OUT && warp == 0 && lane < 18) asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
         fence_proxy_async();
@@ -405,10 +395,10 @@ __global__ void __launch_bounds__(PE_NT, 1) point_embed_kernel(const PointParams
                 // B operands: 128 B between k-chunks, 4096 / 2048 B between 8-point groups
                 a.hi = tmem0 + PE_W1H; a.lo = tmem0 + PE_W1L;
                 xb.hi = smem_u32(sX1); xb.lo = xb.hi + 2048 * 16; xb.lbo = 128; xb.sbo = 4096;
-                if (!(p.probe & 2)) umma_gemm3_ts(tmem0 + PE_ACC1, a, xb, id64, 256, false);
+                umma_gemm3_ts(tmem0 + PE_ACC1, a, xb, id64, 256, false);
                 a.hi = tmem0 + PE_W2H; a.lo = tmem0 + PE_W2L;
                 xb.hi = smem_u32(sX2); xb.lo = xb.hi + 1024 * 16; xb.lbo = 128; xb.sbo = 2048;
-                if (!(p.probe & 2)) umma_gemm3_ts(tmem0 + PE_ACC2, a, xb, id64, 128, false);
+                umma_gemm3_ts(tmem0 + PE_ACC2, a, xb, id64, 128, false);
                 umma_commit(&mma_bar);
             }
             __syncwarp();
@@ -443,11 +433,9 @@ __global__ void __launch_bounds__(PE_NT, 1) point_embed_kernel(const PointParams
             for (int o = 1; o < 8; o <<= 1) sm_ += __shfl_xor_sync(0xffffffffu, sm_, o);
             if (rs == 0) ms[32 + rj] = rj < J ? sm_ : 0.f;
         }
-        stamp();
         mbar_wait(&mma_bar, phase);
         phase ^= 1;
         tc_fence_after();
-        stamp();
         // ---- epilogue: e = relu(relu(acc1 + b1) + acc2 + b2) for channel ch, points [16cg, 16cg + 16)
         uint32_t eh[8], el[8];
         {
@@ -481,7 +469,6 @@ __global__ void __launch_bounds__(PE_NT, 1) point_embed_kernel(const PointParams
         tmem_st_nw<8>(tmem + PE_EH + 8 * cg, reinterpret_cast<const float*>(eh));
         tmem_st_nw<8>(tmem + PE_EL + 8 * cg, reinterpret_cast<const float*>(el));
         tmem_wait_st();
-        stamp();
         fence_proxy_async();
         tc_fence_before();
         __syncthreads();
@@ -515,7 +502,6 @@ __global__ void __launch_bounds__(PE_NT, 1) point_embed_kernel(const PointParams
         }
         tc_fence_before();
         tile_par ^= 1;
-        stamp();
     }
     if (ST_OUT && warp == 0 && lane < 18) asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");   // the staged images are written
     __syncthreads();
@@ -556,7 +542,7 @@ extern "C" int kpf_repack_features(const void* f_d, const void* f_rgb, const voi
 extern "C" int kpf_point_embed(const void* feat_hi, const void* feat_lo, const int32_t* idx, const float* clos, const float* pcl,
                                const float* joint, const int32_t* order, const void* wmat, const float* wvec, int B, int N, int J, int HW,
                                float kernel_size, int fmt, void* e_out, long long e_batch_stride, float* part_acc, float* part_ms,
-                               void* stage_out, const void* stage_in, int num_sms, long long* dbg, cudaStream_t stream) {
+                               void* stage_out, const void* stage_in, int num_sms, cudaStream_t stream) {
     using namespace kpf;
     KPF_REQUIRE(((uintptr_t)stage_out % 16) == 0 && ((uintptr_t)stage_in % 16) == 0 && !(stage_out && stage_in));
     KPF_REQUIRE(B >= 0 && N >= PE_TP && N % PE_TP == 0 && J >= 1 && J <= 21 && HW >= 1 && num_sms >= 1);
@@ -570,11 +556,6 @@ extern "C" int kpf_point_embed(const void* feat_hi, const void* feat_lo, const i
     KPF_REQUIRE(e_batch_stride >= (long long)N * 256 && e_batch_stride % 8 == 0);
     p.e_out = (uint16_t*)e_out; p.e_bs = e_batch_stride; p.part_acc = part_acc; p.part_ms = part_ms; p.B = B; p.N = N; p.J = J; p.HW = HW;
     p.kernel_size = kernel_size; p.fmt = fmt;
-    {
-        static const int probe = [] { const char* e = getenv("KPF_PE_PROBE"); return e ? atoi(e) : 0; }();
-        p.probe = probe;
-    }
-    p.dbg = dbg;
     p.stage_out = (unsigned char*)stage_out; p.stage_in = (const unsigned char*)stage_in;
     const int st = stage_out ? 1 : stage_in ? 2 : 0;
     auto kern = fmt == FMT_F16 ? (st == 0 ? point_embed_kernel<FMT_F16, 0> : st == 1 ? point_embed_kernel<FMT_F16, 1> : point_embed_kernel<FMT_F16, 2>)

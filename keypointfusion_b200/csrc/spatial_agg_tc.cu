@@ -29,7 +29,6 @@ struct SpatialParams {
     float *sw_out, *feat_j_out;
     int B, J, fs;
     float img_size, flip, hm_std, hm_sigma, gamma;
-    long long* dbg;
     float* scratch;   // [B][split][128][32] partial out[c][j]
     int* counters;    // [B], zero on entry, zero again on exit
     int split, fmt;
@@ -67,12 +66,6 @@ __global__ void __launch_bounds__(K5_NT, 1) spatial_aggregate_tc_kernel(const Sp
     const int t_begin = sp * (T / p.split), t_end = t_begin + T / p.split;
     __shared__ int s_last;
     const uint32_t ACC1 = 0, ACC2 = 32;
-    int n_stamp = 0;
-    auto stamp = [&]() {
-        if (p.dbg && blockIdx.x == 0 && tid == 0 && n_stamp < 64) p.dbg[n_stamp] = clock64();
-        ++n_stamp;
-    };
-    stamp();
     pdl_launch_dependents();
 
     if (warp == 0) tmem_alloc(&tmem_slot, 64);
@@ -135,7 +128,6 @@ __global__ void __launch_bounds__(K5_NT, 1) spatial_aggregate_tc_kernel(const Sp
     };
     float d_next = cell_depth(t_begin);
     bool gemm_b_pending = false;   // GEMM B of the previous tile: waited for only where its operands are rewritten
-    stamp();
     for (int t = t_begin; t < t_end; ++t) {
         uint4* cur = sF + ((t - t_begin) & (NBUF - 1)) * NP * 2048;
         if (NBUF == 1 && t > t_begin) load_tile(t, sF);   // single buffer: its readers (tile t-1's MMAs) were waited for
@@ -144,7 +136,6 @@ __global__ void __launch_bounds__(K5_NT, 1) spatial_aggregate_tc_kernel(const Sp
         const bool prefetch = NBUF == 2 && t + 1 < t_end;   // overlaps the whole iteration
         uint4* nxt = sF + ((t + 1 - t_begin) & 1) * NP * 2048;
         if (prefetch) load_tile(t + 1, nxt, 0, 1);
-        if (t == t_begin + 1) stamp();
         // ---- per-cell geometry (thread = cell `row`, joints [8cg, 8cg + 8)): heat-map chunk (A operand) and GAM (registers)
         const int m = t * 128 + row, r = m / fs, col = m - r * fs;
         const float d = d_next;
@@ -175,7 +166,6 @@ __global__ void __launch_bounds__(K5_NT, 1) spatial_aggregate_tc_kernel(const Sp
             sHm[cg * 128 + row] = oh;
             sHm[512 + cg * 128 + row] = ol;
         }
-        if (t == t_begin + 1) stamp();
         if (prefetch) load_tile(t + 1, nxt, 1, 2);
         // relu copy for GEMM B (same layout)
 #pragma unroll
@@ -198,7 +188,6 @@ __global__ void __launch_bounds__(K5_NT, 1) spatial_aggregate_tc_kernel(const Sp
                 sFr[2048 + tid + i * K5_NT] = l;
             }
         }
-        if (t == t_begin + 1) stamp();
         fence_proxy_async();
         tc_fence_before();
         __syncthreads();
@@ -223,7 +212,6 @@ __global__ void __launch_bounds__(K5_NT, 1) spatial_aggregate_tc_kernel(const Sp
         mbar_wait(&mma_bar, phase);
         phase ^= 1;
         tc_fence_after();
-        if (t == t_begin + 1) stamp();
         {
             float s1[8];
             tmem_ld<8>(tmem + ACC1 + 8 * cg, s1);
@@ -245,7 +233,6 @@ __global__ void __launch_bounds__(K5_NT, 1) spatial_aggregate_tc_kernel(const Sp
             sG[1024 + (row >> 3) * 32 + cg * 8 + (row & 7)] = ol;
         }
         if (prefetch) load_tile(t + 1, nxt, 3, 4);
-        if (t == t_begin + 1) stamp();
         fence_proxy_async();
         tc_fence_before();
         __syncthreads();
@@ -261,12 +248,10 @@ __global__ void __launch_bounds__(K5_NT, 1) spatial_aggregate_tc_kernel(const Sp
             __syncwarp();
         }
         gemm_b_pending = true;
-        if (t == t_begin + 1) stamp();
     }
     mbar_wait(&mma_bar, phase);   // the last tile's GEMM B
     phase ^= 1;
     tc_fence_after();
-    stamp();
     {
         float o[8];
         tmem_ld<8>(tmem + ACC2 + 8 * cg, o);  // thread = (channel `row`, joints [8cg, 8cg + 8)): this CTA's partial out[c][j]
@@ -346,7 +331,7 @@ extern "C" int kpf_spatial_aggregate_tc(const void* feat_rgb, const void* feat_r
                                         const void* wa_packed, const float* ba, const float* weight_dis, const float* fc_w,
                                         const float* fc_b, const float* prev, int B, int C, int J, int fs, float img_size, float flip,
                                         float hm_std, float hm_sigma, float gamma, int fmt, float* sw_out, float* feat_j_out, float* scratch,
-                                        int* counters, int split, long long* dbg, cudaStream_t stream) {
+                                        int* counters, int split, cudaStream_t stream) {
     using namespace kpf;
     KPF_REQUIRE(B >= 0 && C == 128 && J >= 1 && J <= 32 && fs >= 1 && (fs * fs) % 128 == 0);
     KPF_REQUIRE(((uintptr_t)feat_rgb % 16) == 0 && ((uintptr_t)feat_rgb_lo % 16) == 0 && ((uintptr_t)wa_packed % 16) == 0);
@@ -357,7 +342,7 @@ extern "C" int kpf_spatial_aggregate_tc(const void* feat_rgb, const void* feat_r
     p.feat = (const __nv_bfloat16*)feat_rgb; p.feat_lo = (const __nv_bfloat16*)feat_rgb_lo; p.fmt = fmt; p.joints = joints; p.depth = depth; p.depth_bs = depth_bs; p.depth_rs = depth_rs;
     p.depth_cs = depth_cs; p.center = center; p.M = M; p.cube = cube; p.cam = cam; p.wa = (const uint4*)wa_packed; p.ba = ba;
     p.weight_dis = weight_dis; p.fc_w = fc_w; p.fc_b = fc_b; p.prev = prev; p.sw_out = sw_out; p.feat_j_out = feat_j_out;
-    p.dbg = dbg; p.scratch = scratch; p.counters = counters; p.split = split;
+    p.scratch = scratch; p.counters = counters; p.split = split;
     p.B = B; p.J = J; p.fs = fs; p.img_size = img_size; p.flip = flip; p.hm_std = hm_std; p.hm_sigma = hm_sigma; p.gamma = gamma;
     const int NP = feat_rgb_lo ? 2 : 1, NBUF = feat_rgb_lo ? 1 : 2;
     const size_t smem = (size_t)(1024 + 1536 + 1792 + (NBUF + 1) * NP * 2048) * 16 + 32 * 8 * 4 + 32 * 4 + (size_t)2 * 32 * fs * 4;

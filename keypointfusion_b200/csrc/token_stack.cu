@@ -54,7 +54,6 @@ struct TokParams {
     float* out_jc;         // cross only: element (b,t,c) at out_jc[(b*J+t)*stride + c0 + c] or null
     int out_jc_stride, out_jc_c0;
     int B, J, D, L, F, pre, cross, Fc, G, fmt;
-    long long* dbg;        // optional: clock64 stamps of CTA 0 (profiling aid)
     // fused exchange step (SURVEY.md 2b row C1): pred is ALSO stored straight into every rank's gathered-joints buffer over NVLink
     const unsigned long long* peer_bases;   // null, or [world] base addresses of the ranks' symmetric exchange buffers
     const int* xstep;                       // device step counter (its parity selects the half of the double-buffered result)
@@ -254,18 +253,6 @@ __global__ void __launch_bounds__(TS_NT, 1) token_stack_kernel(const TokParams p
         sHead[((part * 4 + q) * 4 + c) * 32 + lane] = hx[0];
     };
 
-    int n_stamp = 0;
-    auto stamp = [&]() {
-        if (p.dbg && blockIdx.x == 0 && tid == 0 && n_stamp < 64) p.dbg[n_stamp] = clock64();
-        ++n_stamp;
-    };
-    stamp();
-    int n_fine = 0;
-    bool fine_on = false;   // fine stamps (dbg[32..63]) inside the first encoder layer
-    auto fine = [&]() {
-        if (fine_on && p.dbg && blockIdx.x == 0 && tid == 0 && n_fine < 32) p.dbg[32 + n_fine] = clock64();
-        ++n_fine;
-    };
     if (tid < 128) sLead[tid] = 0.f;
     wsync();      // sLead is rewritten by warp 0 in the input stage
     pdl_wait();   // everything above touched only weights; the activations below come from the previous kernel
@@ -397,7 +384,6 @@ __global__ void __launch_bounds__(TS_NT, 1) token_stack_kernel(const TokParams p
 #pragma unroll
             for (int i = 0; i < 8; ++i) resid[i] = a[i] = tokv[i] ? a[i] + bb + e[i] : 0.f;
             write_act(bufX, a);
-            stamp();
         }
 
         const float* sv = sVec + (it & 1) * TS_VEC;
@@ -408,9 +394,6 @@ __global__ void __launch_bounds__(TS_NT, 1) token_stack_kernel(const TokParams p
 
         // ---- K and Q projections back to back (ring order K, Q, V, O: V's weights take the slots K frees, the earliest possible);
         //      V follows S
-        fine_on = (it == (p.cross ? 1 : 0));
-        n_fine = 0;
-        fine();
         sync_for_mma();
         if (warp_u == 0) {
             tc_fence_after();
@@ -430,7 +413,6 @@ __global__ void __launch_bounds__(TS_NT, 1) token_stack_kernel(const TokParams p
         // chunk of the head-major attention operands: K index d = lane, row 32q + token
         const uint32_t qidx = (uint32_t)((lane >> 3) * 128 + (4 * q + c) * 8 + (lane & 7));
         wait_bar(1);
-        fine();
         {   // K^T -> MN-major B operand of S
             float a[8];
             tmem_ld<8>(tmem + ACC_K + 8 * c, a);
@@ -441,9 +423,7 @@ __global__ void __launch_bounds__(TS_NT, 1) token_stack_kernel(const TokParams p
             bufK[qidx] = hi;
             bufK[TS_PLANE + qidx] = lo;
         }
-        fine();
         wait_bar(0);
-        fine();
         {   // Q^T -> MN-major A operand of S
             float a[8];
             tmem_ld<8>(tmem + ACC_Q + 8 * c, a);
@@ -454,7 +434,6 @@ __global__ void __launch_bounds__(TS_NT, 1) token_stack_kernel(const TokParams p
             bufQ[qidx] = hi;
             bufQ[TS_PLANE + qidx] = lo;
         }
-        stamp();
         // ---- S for all four heads: D[32h+t][32h'+k] = Q_h[t] . K_h'[k] (diagonal blocks h = h' are the scores); then V^T
         sync_for_mma();
         if (warp_u == 0) {
@@ -470,9 +449,7 @@ __global__ void __launch_bounds__(TS_NT, 1) token_stack_kernel(const TokParams p
             }
             __syncwarp();
         }
-        fine();
         wait_bar(0);
-        fine();
         {   // softmax of row t = lane of head q: every key group takes the row maximum over all keys and exponentiates its 8 keys;
             // P stays un-normalised, the partial sums meet when O is read out
             float sa[32], own[8];
@@ -495,9 +472,7 @@ __global__ void __launch_bounds__(TS_NT, 1) token_stack_kernel(const TokParams p
             bufQ[c * 128 + f] = hi;
             bufQ[TS_PLANE + c * 128 + f] = lo;
         }
-        fine();
         wait_bar(1);
-        fine();
         {   // V^T (lane = 32h + d, K = keys) -> A operand planes in tensor memory
             float a[8];
             tmem_ld<8>(tmem + ACC_V + 8 * c, a);
@@ -536,10 +511,7 @@ __global__ void __launch_bounds__(TS_NT, 1) token_stack_kernel(const TokParams p
 #pragma unroll
             for (int i = 0; i < 8; ++i) inv[i] = tokv[i] ? 1.f / s8[i] : 0.f;
         }
-        fine();
         wait_bar(0);
-        fine();
-        stamp();
         {   // O^T -> activation operand of the output projection
             float a[8];
             tmem_ld<8>(tmem + ACC_O + 32 * q + 8 * c, a);
@@ -591,12 +563,8 @@ __global__ void __launch_bounds__(TS_NT, 1) token_stack_kernel(const TokParams p
             }
             __syncwarp();
         }
-        fine();
         wait_bar(0);
-        fine();
         resid_ln(bo_, g1, be1);
-        fine();
-        stamp();
         // ---- FFN-1, token-major: D[token][F] = X^T W1^T.  A = bufX read as an MN-major A operand (rows >= 32 alias other data
         //      and only produce unused accumulator lanes), B = W1 [N = F][K = 128] K-major
         const int nffn = F == 16 ? 1 : 4;   // ring entries of the FFN weights
@@ -627,9 +595,7 @@ __global__ void __launch_bounds__(TS_NT, 1) token_stack_kernel(const TokParams p
             }
             __syncwarp();
         }
-        fine();
         wait_bar(0);
-        fine();
         if (q == 0) {   // lanes 0..31 of the accumulator = tokens: the four quarter-0 warps take F/4 hidden units each
             const bool tv = lane < J;
             if (F == 16) {
@@ -691,13 +657,9 @@ __global__ void __launch_bounds__(TS_NT, 1) token_stack_kernel(const TokParams p
             }
             __syncwarp();
         }
-        fine();
         wait_bar(0);
-        fine();
         resid_ln(b2, g2, be2);
-        fine();
         g += 8 + nffn;
-        stamp();
     }
 
     if (p.cross && p.L == 0) {
@@ -744,7 +706,6 @@ __global__ void __launch_bounds__(TS_NT, 1) token_stack_kernel(const TokParams p
             if (tid < p.world) asm volatile("red.relaxed.sys.global.add.u32 [%0], 1;" ::"l"(p.peer_bases[tid]) : "memory");
         }
     }
-    stamp();
     tc_fence_before();
     wsync();
     if (warp_u == 0) tmem_dealloc(tmem0, 512);
@@ -786,7 +747,7 @@ extern "C" int kpf_token_stack(const float* x, const float* y, const float* r3d,
                                const void* wseq, const float* wvec, int n_weights, int cross, int pre, int B, int J, int D, int L, int F,
                                int Fc, int fmt, float* tokens_out, float* pred_out, float* out_cj, float* out_jc, int out_jc_stride,
                                int out_jc_c0, const void* peer_bases, const int* xstep, int world, int row0, int rows_total,
-                               long long* dbg, cudaStream_t stream) {
+                               cudaStream_t stream) {
     using namespace kpf;
     KPF_REQUIRE(B >= 0 && J >= 1 && J <= 32 && L >= 0 && (cross || pre || L > 0));
     KPF_REQUIRE(fmt == FMT_F16 || fmt == FMT_BF16);
@@ -804,7 +765,6 @@ extern "C" int kpf_token_stack(const float* x, const float* y, const float* r3d,
     p.x = x; p.y = y; p.r3d = r3d; p.desa = desa; p.jf = jf; p.wmat = (const uint4*)wmat; p.wseq = (const int4*)wseq; p.wvec = wvec;
     p.tokens_out = tokens_out; p.pred_out = pred_out; p.out_cj = out_cj; p.out_jc = out_jc; p.out_jc_stride = out_jc_stride;
     p.out_jc_c0 = out_jc_c0; p.B = B; p.J = J; p.D = D; p.L = L; p.F = F; p.pre = pre; p.cross = cross; p.Fc = Fc; p.G = n_weights; p.fmt = fmt;
-    p.dbg = dbg;
     KPF_REQUIRE(peer_bases == nullptr || (xstep != nullptr && world >= 1 && row0 >= 0 && row0 + B <= rows_total && L > 0));
     p.peer_bases = (const unsigned long long*)peer_bases; p.xstep = xstep; p.world = world; p.row0 = row0; p.rows_total = rows_total;
     auto kern = fmt == FMT_F16 ? token_stack_kernel<FMT_F16> : token_stack_kernel<FMT_BF16>;

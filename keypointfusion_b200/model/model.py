@@ -7,8 +7,6 @@ running statistics (folded into the preceding 1x1 conv), dropout is identity, no
 """
 import math
 
-import os
-
 import torch
 import torch.nn as nn
 import torch.nn.functional as F
@@ -483,8 +481,8 @@ class KPFusion(nn.Module):
         rgb_planes = _rgb_planes(img_feat_rgb)
         # ... and the gathered point-stage operands: both blocks gather the same taps (model.py:297-306 per block); block 1 stores
         # its tiles, the later blocks load them with the TMA engine
-        # (KPF_PE_STAGE=0: every block gathers for itself -- 175 MB less DRAM traffic per 64-sample step for ~6 us more kernel time)
-        staged = self.num_stages > 1 and pcl.shape[1] % 64 == 0 and os.environ.get("KPF_PE_STAGE", "1") != "0"
+        # (unstaged, every block gathers for itself -- 175 MB less DRAM traffic per 64-sample step for ~6 us more kernel time)
+        staged = self.num_stages > 1 and pcl.shape[1] % 64 == 0
         pe_stage = ops.point_embed_stage(pcl.shape[0], pcl.shape[1], pcl.device) if staged else None
         for i in range(self.num_stages):                                                                 # :417-424
             block = getattr(self, f"block{i + 1}")

@@ -621,7 +621,7 @@ def pack_token_program(J, enc=None, cross=None, fusion=None, C=128, fmt=None):
                         fmt)
 
 
-def token_stack(pk, x=None, y=None, r3d=None, desa=None, jf=None, want_tokens=True, out_jc=None, out_jc_c0=0, want_cj=False, dbg=None,
+def token_stack(pk, x=None, y=None, r3d=None, desa=None, jf=None, want_tokens=True, out_jc=None, out_jc_c0=0, want_cj=False,
                 exchange=None):
     """Run one packed token program.  Returns (tokens [B,J,128] | None, pred [B,J,3] | None, out_cj [B,128,J] | None).
     exchange = (peer_ptrs [world] i64 device, xstep [1] i32 device, row0, rows_total): pred is also stored into every rank's gathered
@@ -642,7 +642,7 @@ def token_stack(pk, x=None, y=None, r3d=None, desa=None, jf=None, want_tokens=Tr
     _call("kpf_token_stack", _p(x), _p(y), _p(r3d), _p(desa), _p(jf), _p(pk.wmat), _p(pk.wseq), _p(pk.wvec), pk.n_weights, pk.cross, pk.pre,
           B, J, pk.D, pk.L, pk.F, pk.Fc, pk.fmt, _p(tokens), _p(pred), _p(out_cj), _p(out_jc), stride, out_jc_c0,
           _p(exchange[0]) if exchange else None, _p(exchange[1]) if exchange else None, exchange[0].numel() if exchange else 0,
-          int(exchange[2]) if exchange else 0, int(exchange[3]) if exchange else 0, _p(dbg))
+          int(exchange[2]) if exchange else 0, int(exchange[3]) if exchange else 0)
     return tokens, pred, out_cj
 
 
@@ -728,7 +728,7 @@ def point_embed_stage(B, N, device):
     return torch.empty(int(B) * (int(N) // 64) * PE_STAGE_BYTES_PER_TILE, device=device, dtype=torch.uint8)
 
 
-def point_embed(featT, idx32, clos, pcl, joint, wmat, wvec, kernel_size=0.8, dbg=None, order=None, fmt=None, stage_out=None, stage_in=None):
+def point_embed(featT, idx32, clos, pcl, joint, wmat, wvec, kernel_size=0.8, order=None, fmt=None, stage_out=None, stage_in=None):
     """featT = (hi, lo | None) from repack_features.
     -> e [B,N,256] int16 (rows [hi 128 | lo 128] in the split format), part_acc [B,T,128,32] f32, part_ms [B,T,2,32] f32  (T = N/64).
     stage_out: also store the gathered (joint-independent) operand image of every tile into this point_embed_stage buffer;
@@ -752,7 +752,7 @@ def point_embed(featT, idx32, clos, pcl, joint, wmat, wvec, kernel_size=0.8, dbg
     acc = torch.empty(B, T, 128, 32, device=dev, dtype=torch.float32)
     ms = torch.empty(B, T, 2, 32, device=dev, dtype=torch.float32)
     _call("kpf_point_embed", _p(feat_hi), _p(feat_lo), _p(idx32), _p(clos), _p(pcl), _p(joint), _p(order), _p(wmat), _p(wvec), B, N, J, HW,
-          float(kernel_size), fmt, _p(e), e.stride(0), _p(acc), _p(ms), _p(stage_out), _p(stage_in), sm_count(dev), _p(dbg))
+          float(kernel_size), fmt, _p(e), e.stride(0), _p(acc), _p(ms), _p(stage_out), _p(stage_in), sm_count(dev))
     return e, acc, ms
 
 
@@ -798,7 +798,7 @@ def pack_desa(Wj, bj, Wjx, bjx, scales, fmt=None):
     return torch.cat(mats).contiguous(), torch.cat(vecs).contiguous()
 
 
-def desa_fused(e, part_acc, part_ms, pcl, joint, wmat, wvec, radius, nsample, dbg=None, fmt=None, jf_in=None, keep_scratch=None):
+def desa_fused(e, part_acc, part_ms, pcl, joint, wmat, wvec, radius, nsample, fmt=None, jf_in=None, keep_scratch=None):
     """e: [B,N,256] int16 rows from point_embed (or e_from_float).  jf_in [B,J,128]: the joints' features are given (no embedding)."""
     fmt = SPLIT_FMT if fmt is None else fmt
     pcl, joint = _f32(pcl), _f32(joint)
@@ -818,7 +818,7 @@ def desa_fused(e, part_acc, part_ms, pcl, joint, wmat, wvec, radius, nsample, db
     scratch = torch.empty(B * S * J * 128 * 4 + B * (N + 32) * 16 + B * S * J * nsample * 2 + B * S * 4, device=pcl.device, dtype=torch.uint8)
     _call("kpf_desa_fused", _p(e), e.stride(0), _p(part_acc), _p(part_ms), _p(pcl), _p(joint), _p(wmat), _p(wvec), B, N, J, S, nsample, float(r[0]),
           float(r[1]), float(r[2]), float(r[3]), fmt, _p(_f32(jf_in) if jf_in is not None else None), _p(part), _p(jf), _p(scratch),
-          sm_count(pcl.device), _p(dbg))
+          sm_count(pcl.device))
     if keep_scratch is not None:   # tests read the ball-query indices back out of the hand-over workspace
         keep_scratch["buf"] = scratch
     return part, jf
@@ -873,7 +873,7 @@ def split_map(x):
 
 
 def spatial_aggregate_tc(feat_rgb, joints, img, center, M, cube, cam, wa_packed, ba, weight_dis, fc_w, fc_b, prev=None, img_size=128,
-                         flip=1.0, hm_std=0.8, hm_sigma=1.0, gamma=10.0, dbg=None, fmt=None):
+                         flip=1.0, hm_std=0.8, hm_sigma=1.0, gamma=10.0, fmt=None):
     """feat_rgb: bf16 [B,128,fs,fs], or a (hi, lo) pair of bf16 planes (split_map of an fp32 map)."""
     fmt = SPLIT_FMT if fmt is None else fmt
     feat_rgb, feat_lo = feat_rgb if isinstance(feat_rgb, (tuple, list)) else (feat_rgb, None)
@@ -899,16 +899,15 @@ def spatial_aggregate_tc(feat_rgb, joints, img, center, M, cube, cam, wa_packed,
     split = next((s_ for s_ in (8, 4, 2) if T % s_ == 0 and B * s_ <= sm_count(feat_rgb.device)), 1)
     # ... which is the LATENCY optimum of a launch that has the GPU to itself.  With several steps in flight what counts is the launch's
     # SM-time, and the per-CTA prologue (weights, tables, first tile) is paid `split` times: one CTA per sample is 60 us x 64 SMs against
-    # 35 us x 128.  K5_SPLIT (set by the caller that overlaps steps, before it captures its graphs; env KPF_K5_SPLIT for A/B runs)
-    # overrides the policy: bench.py at batch 64, six steps in flight, split 2 -> 1: 0.479 -> 0.464 ms per step (profiles/ab_overlap_r2.txt)
-    forced = int(os.environ["KPF_K5_SPLIT"]) if os.environ.get("KPF_K5_SPLIT") else K5_SPLIT
-    if forced and T % forced == 0:
-        split = forced
+    # 35 us x 128.  K5_SPLIT (set by the caller that overlaps steps, before it captures its graphs) overrides the policy: bench.py
+    # at batch 64, six steps in flight, split 2 -> 1: 0.479 -> 0.464 ms per step (profiles/ab_overlap_r2.txt)
+    if K5_SPLIT and T % K5_SPLIT == 0:
+        split = K5_SPLIT
     scratch = torch.empty(B, split, 128, 32, device=feat_rgb.device, dtype=torch.float32) if split > 1 else None
     counters = _zero_counters(B, feat_rgb.device) if split > 1 else None
     _call("kpf_spatial_aggregate_tc", _p(feat_rgb), _p(feat_lo), _p(joints), _p(d), bs, rs, cs, _p(center), _p(M), _p(cube), _p(cam),
           _p(wa_packed), _p(ba), _p(weight_dis), _p(fc_w), _p(fc_b), _p(prev), B, C, J, fs, float(img_size), float(flip), float(hm_std),
-          float(hm_sigma), float(gamma), fmt, _p(sw), _p(fj), _p(scratch), _p(counters), split, _p(dbg))
+          float(hm_sigma), float(gamma), fmt, _p(sw), _p(fj), _p(scratch), _p(counters), split)
     return sw, fj
 
 

@@ -20,7 +20,6 @@ class GraphedFusionPath:
         self.net, self.loader, self.sample_num, self.kernel, self.seed = net, loader, sample_num, kernel, seed
         self.exchange = exchange    # a PeerExchange: the fused all-gather of the joints is part of the captured graph
         self.chains = max(1, min(chains, example["img"].shape[0]))
-        self.sm_share = float(__import__("os").environ.get("KPF_SM_SHARE", "1.0"))   # x SMs / chains per chain's persistent kernels
         dev = next(net.parameters()).device
         self.side = [torch.cuda.Stream(device=dev) for _ in range(self.chains - 1)]
         if bind:
@@ -75,7 +74,7 @@ class GraphedFusionPath:
                 st.wait_stream(main)              # fork
             # SM partitioning: each concurrent chain's persistent kernels take their share of the SMs, so that e.g. one chain's
             # (one CTA per sample) token stack and another chain's point stage / DESA tiles are co-resident
-            with torch.cuda.stream(st), ops.sm_budget(max(1, int(ops.sm_count(self.static["img"].device) * self.sm_share / self.chains))):
+            with torch.cuda.stream(st), ops.sm_budget(max(1, ops.sm_count(self.static["img"].device) // self.chains)):
                 res, sw, pcl = self._chain(sub)
                 self.joints_all[lo:hi].copy_(res[-1])
             outs.append((res, sw, pcl))

@@ -1,5 +1,5 @@
 """Tuning aid (not a test): K4a (offset2joint_weight, bf16 fast path) alone, graph-timed over rotating input sets, at batch 64 and 512.
-KPF_K4A_VARIANT=1 forces 3 joints per CTA, =2 forces 7 (default: by grid size, see geometry.cu)"""
+The launcher picks 3 or 7 joints per CTA by grid size (geometry.cu): batch 64 runs the 3-joint kernel, batch 512 the 7-joint one."""
 import os, sys, torch
 sys.path.insert(0, os.getcwd())
 from keypointfusion_b200 import ops
@@ -22,4 +22,4 @@ def t(B, nsets):
     us = e0.elapsed_time(e1) * 1e3 / (5 * 4 * nsets)
     alg = B * (5 * J * H * H * 2 + H * H * 4)
     return us, alg / us / 1e3
-print("variant", os.environ.get("KPF_K4A_VARIANT", "0"), "B=64: %.2f us %.0f GB/s | B=512: %.2f us %.0f GB/s" % (*t(64, 12), *t(512, 3)))
+print("B=64: %.2f us %.0f GB/s | B=512: %.2f us %.0f GB/s" % (*t(64, 12), *t(512, 3)))

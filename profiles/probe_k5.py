@@ -1,4 +1,4 @@
-"""Profiling aid: K5 (spatial_aggregate_tc) alone at the benchmark shape; stamps + graph timing.
+"""Profiling aid: K5 (spatial_aggregate_tc) alone at the benchmark shape, graph-timed.
 profiles/srcstalls.sh spatial_aggregate r2_k5 profiles/probe_k5.py"""
 import os, sys, torch
 sys.path.insert(0, os.getcwd())
@@ -13,8 +13,8 @@ inp = synth.make_inputs(B, 128, 21, 128, seed=5)
 c = {kk: v.to(dev) for kk, v in inp.items()}
 rgb = c["img_feat_rgb"].bfloat16()
 r3d = (torch.rand(B, 21, 3, device=dev) - 0.5)
-fn = lambda dbg=None: ops.spatial_aggregate_tc(rgb, r3d, c["img"][:, :, ::4, ::4], c["center"], c["M"], c["cube"], c["cam"], k["wa_packed"], b.atten_spatial.bias,
-                                               b.weight_dis, b.fc_spatial2joint_feature.weight, b.fc_spatial2joint_feature.bias, dbg=dbg)
+fn = lambda: ops.spatial_aggregate_tc(rgb, r3d, c["img"][:, :, ::4, ::4], c["center"], c["M"], c["cube"], c["cam"], k["wa_packed"], b.atten_spatial.bias,
+                                      b.weight_dis, b.fc_spatial2joint_feature.weight, b.fc_spatial2joint_feature.bias)
 for _ in range(10): fn()
 torch.cuda.synchronize()
 g = torch.cuda.CUDAGraph()
@@ -26,7 +26,3 @@ e0.record()
 for _ in range(5): g.replay()
 e1.record(); torch.cuda.synchronize()
 print("K5 us per launch: %.1f" % (e0.elapsed_time(e1) * 1e3 / 50))
-dbg = torch.zeros(64, dtype=torch.int64, device=dev)
-fn(dbg); torch.cuda.synchronize()
-d = [v for v in dbg.cpu().tolist() if v]
-print("stamps (cycles):", [d[i + 1] - d[i] for i in range(len(d) - 1)], "total", d[-1] - d[0] if d else 0)

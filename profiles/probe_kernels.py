@@ -1,5 +1,5 @@
-"""Profiling aid (not a test): graph-timed point stage / DESA with the KPF_PE_PROBE / KPF_DESA_PROBE switches (gather and MMAs
-off) to see which part of a tile bounds it.  Run on the GPU box: KPF_DESA_PROBE=1 python profiles/probe_kernels.py"""
+"""Profiling aid (not a test): graph-timed point stage (plain, storing and loading staged tiles) and DESA at batch 64.
+Run on a B200: python profiles/probe_kernels.py"""
 import os, sys, torch, numpy as np
 sys.path.insert(0, os.getcwd())
 from keypointfusion_b200 import ops
@@ -35,11 +35,3 @@ stage = ops.point_embed_stage(B, pcl.shape[1], dev)
 print("point_embed + stage_out us", t(lambda: ops.point_embed(featT, idx, close, pcl, joint, k["pe_wmat"], k["pe_wvec"], 0.8, order=order, stage_out=stage)))
 print("point_embed from stage_in us", t(lambda: ops.point_embed(featT, idx, close, pcl, joint, k["pe_wmat"], k["pe_wvec"], 0.8, order=order, stage_in=stage)))
 print("desa us", t(lambda: ops.desa_fused(e, acc, ms, pcl, joint, k["ds_wmat"], k["ds_wvec"], blk.FA.radius, 64)))
-# clock stamps of the DESA kernels (CTA 0 / thread 0; prep: the joint-embedding role dbg[0..7] and the ball-query role dbg[8..15]; tile: dbg[16..])
-dbg = torch.zeros(128, dtype=torch.int64, device=dev)
-ops.desa_fused(e, acc, ms, pcl, joint, k["ds_wmat"], k["ds_wvec"], blk.FA.radius, 64, dbg=dbg)
-torch.cuda.synchronize()
-d = dbg.cpu().tolist()
-pr = [v for v in d[0:8] if v]; bq = [v for v in d[8:16] if v]; co = [v for v in d[16:64] if v]
-print("desa prep, joint embedding role (cycles between stamps):", [pr[i + 1] - pr[i] for i in range(len(pr) - 1)], " ball query role:", [bq[i + 1] - bq[i] for i in range(len(bq) - 1)])
-print("desa tile (cycles between stamps):", [co[i + 1] - co[i] for i in range(len(co) - 1)], "total", co[-1] - co[0] if co else 0)

@@ -4,9 +4,6 @@ sys.path.insert(0, os.getcwd())
 exec(open("profiles/probe_kernels.py").read().split("def t(fn")[0])
 stage = ops.point_embed_stage(B, pcl.shape[1], dev)
 ops.point_embed(featT, idx, close, pcl, joint, k["pe_wmat"], k["pe_wvec"], 0.8, order=order, stage_out=stage)
-dbg = torch.zeros(64, dtype=torch.int64, device=dev)
 for _ in range(12):
-    ops.point_embed(featT, idx, close, pcl, joint, k["pe_wmat"], k["pe_wvec"], 0.8, order=order, stage_in=stage, dbg=dbg)
+    ops.point_embed(featT, idx, close, pcl, joint, k["pe_wmat"], k["pe_wvec"], 0.8, order=order, stage_in=stage)
 torch.cuda.synchronize()
-d = [v for v in dbg.cpu().tolist() if v]
-print("stamps:", [d[i + 1] - d[i] for i in range(len(d) - 1)][:24])

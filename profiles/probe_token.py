@@ -1,5 +1,5 @@
-"""Profiling aid (not a test): clock64 stamps of CTA 0 inside token_stack_kernel (coarse: per stage; fine: inside the first encoder
-layer) for the two token programs of a block, plus their graph-timed duration.  Run on the GPU box: python profiles/probe_token.py"""
+"""Profiling aid (not a test): graph-timed duration of token_stack_kernel for the two token programs of a block, at batch 64 and
+at 1 / 16 / 148 samples.  Run on a B200: python profiles/probe_token.py"""
 import os, sys, torch
 sys.path.insert(0, os.getcwd())
 from keypointfusion_b200 import ops
@@ -26,15 +26,7 @@ def t(fn, n=10):
     return e0.elapsed_time(e1) * 1e3 / (5 * n)
 for name, kw in (("tok_init", dict(desa=desa, jf=jf)), ("tok_final", dict(x=x, y=y, r3d=r3d, want_tokens=False))):
     pk = k[name]
-    dbg = torch.zeros(64, dtype=torch.int64, device=dev)
-    ops.token_stack(pk, dbg=dbg, **kw)
-    torch.cuda.synchronize()
-    d = dbg.cpu().tolist()
-    coarse = [v for v in d[:32] if v]
-    fine = [v for v in d[32:] if v]
     print(name, "L", pk.L, "F", pk.F, "cross", pk.cross, "pre", pk.pre, "ring entries", pk.n_weights)
-    print("  coarse (cycles between stamps):", [coarse[i + 1] - coarse[i] for i in range(len(coarse) - 1)], "total", coarse[-1] - coarse[0])
-    print("  fine, first encoder layer      :", [fine[i + 1] - fine[i] for i in range(len(fine) - 1)])
     print("  us per launch (graph of 10)    : %.1f" % t(lambda: ops.token_stack(pk, **kw)))
     for Bs in (1, 16, 148):
         kw2 = {kk: (v[:Bs] if Bs <= B else v.repeat((Bs + B - 1) // B, *[1] * (v.dim() - 1))[:Bs]) if torch.is_tensor(v) else v for kk, v in kw.items()}

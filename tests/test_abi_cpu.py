@@ -47,3 +47,15 @@ def test_product_never_touches_the_oracle():
             assert not any(n.split(".")[0] == "oracle" for n in names), f"{path} imports the oracle"
     for path in glob.glob(os.path.join(root, "csrc", "*")):
         assert "oracle/" not in open(path, errors="ignore").read().replace("oracle/kpf_oracle.py", ""), path
+
+
+def test_kernels_read_no_environment():
+    """A kernel's code path is chosen by its arguments and inputs alone, never by an environment variable read inside the library."""
+    import glob
+    import os
+    import re
+    root = os.path.join(os.path.dirname(__file__), "..", "keypointfusion_b200", "csrc")
+    srcs = glob.glob(os.path.join(root, "*"))
+    assert srcs
+    for path in srcs:
+        assert not re.search(r"\bgetenv\s*\(", open(path, errors="ignore").read()), f"{path} calls getenv"

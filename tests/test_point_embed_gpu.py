@@ -174,15 +174,20 @@ def test_desa_fused(path_params, B, which, radii):
     featT = ops.repack_features(c["img_feat"].bfloat16(), c["img_feat_rgb"].bfloat16(), c["img_offset"][:, 84:].bfloat16())
     e, acc, ms = ops.point_embed(featT, idx, close, pcl, joint, k["pe_wmat"], k["pe_wvec"], 0.8)
     part, jf = ops.desa_fused(e, acc, ms, pcl, joint, k["ds_wmat"], k["ds_wvec"], blk.FA.radius, blk.FA.S[0])
-    # narrow groups (a scale whose widest ball holds <= 16 / 32 points is tiled 16 / 32 rows per joint) leave every bit unchanged:
-    # KPF_DESA_PROBE=8 forces nsample rows per joint
-    import os
-    os.environ["KPF_DESA_PROBE"] = "8"
-    try:
-        part_w, jf_w = ops.desa_fused(e, acc, ms, pcl, joint, k["ds_wmat"], k["ds_wvec"], blk.FA.radius, blk.FA.S[0])
-    finally:
-        del os.environ["KPF_DESA_PROBE"]
-    assert torch.equal(part, part_w) and torch.equal(jf, jf_w)
+    # narrow groups (a scale whose widest ball holds <= 16 / 32 points is tiled 16 / 32 rows per joint) leave every bit unchanged.
+    # The group width is chosen per launch, from the widest ball of any sample: a launch with one extra sample whose points and
+    # joints all sit inside one 0.01 cube (every ball of every scale saturated) groups nsample rows per joint for every sample.
+    N, NS, S = pcl.shape[1], blk.FA.S[0], len(blk.FA.radius)
+    gen = torch.Generator(device=DEV).manual_seed(B)
+    tight = lambda n: pcl[:1, :1] + 0.01 * torch.rand(1, n, 3, device=DEV, generator=gen)
+    scratch = {}
+    part_w, jf_w = ops.desa_fused(torch.cat([e, e[:1]]), torch.cat([acc, acc[:1]]), torch.cat([ms, ms[:1]]), torch.cat([pcl, tight(N)]),
+                                  torch.cat([joint, tight(21)]), k["ds_wmat"], k["ds_wvec"], blk.FA.radius, NS, keep_scratch=scratch)
+    torch.cuda.synchronize()
+    off_gw = (B + 1) * (S * 21 * 128 * 4 + (N + 32) * 16 + S * 21 * NS * 2)
+    gw = scratch["buf"][off_gw:off_gw + (B + 1) * S * 4].view(torch.int32).cpu().reshape(B + 1, S)
+    assert (gw[B] > 32).all(), gw     # the extra sample widens every scale to nsample rows per joint
+    assert torch.equal(part, part_w[:B]) and torch.equal(jf, jf_w[:B])
     fu = blk.FA.kc()["fusion"]
     out = F.relu(F.linear(torch.cat([part.permute(0, 2, 1, 3).reshape(B, 21, -1), jf], -1), *fu))
     # oracle

@@ -50,29 +50,3 @@ def test_umma_split_gemm(N, K, fmt, a_tmem, capsys):
     ref = (A16.double() @ B.double().t())
     assert float((D.double() - ref).norm() / ref.norm()) < (3e-5 if fmt else 2e-6)
 
-
-@pytest.mark.parametrize("a_tmem", [0, 1])
-@pytest.mark.parametrize("N", [16, 64, 128])
-def test_tma_row_gather_swizzled_operand(N, a_tmem, capsys):
-    """csrc/tma_gather.cuh: rows of a [R][hi 128 | lo 128] fp16-plane table gathered by the TMA engine (tile::gather4, four rows per
-    instruction, 128-byte swizzle applied on the way) are directly a SWIZZLE_128B K-major tcgen05.mma operand:
-    D = A X[idx]^T at split precision.  Random rows incl. repeats, first and last row of the table."""
-    from keypointfusion_b200 import ops
-    torch.manual_seed(N)
-    R = 1056
-    X = torch.randn(R, 128, device="cuda")
-    hi = X.half()
-    lo = (X - hi.float()).half()
-    table = torch.cat([hi, lo], 1).contiguous().view(torch.int16)
-    idx = torch.randint(0, R, (N,), device="cuda", dtype=torch.int32)
-    idx[0], idx[1], idx[-1] = 0, R - 1, idx[2]
-    A = torch.randn(128, 128, device="cuda")
-    D = torch.zeros(128, N, device="cuda")
-    cyc = torch.zeros(4, dtype=torch.int64, device="cuda")
-    ops._call("kpf_tma_gather_selftest", ops._p(table), R, ops._p(A), ops._p(idx), ops._p(D), N, a_tmem, ops._p(cyc))
-    torch.cuda.synchronize()
-    ref = A.double() @ X[idx.long()].double().t()
-    rel = float((D.double() - ref).norm() / ref.norm())
-    with capsys.disabled():
-        print(f"\n[tma gather4] N={N}: rel err {rel:.2e}, gather cold {int(cyc[0])} cycles, L2-hot {int(cyc[2])} cycles ({N * 512 / max(int(cyc[2]), 1):.1f} B/clk); A from {'tmem' if a_tmem else 'smem'}: 24 MMAs {int(cyc[1])} cycles, steady {(int(cyc[3]) - int(cyc[1])) / (7 * 24):.1f} cycles/MMA")
-    assert rel < 2e-6, rel
