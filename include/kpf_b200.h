@@ -185,7 +185,7 @@ int kpf_ball_query(const float* xyz, const float* centers, int B, int Np, int J,
  * Outputs: L > 0 -> tokens_out [B,J,128] (may be NULL), pred_out [B,J,3];  cross only -> out_cj [B,128,J] and/or out_jc.
  * wmat (16-bit canonical half-K weight tiles, hi and lo planes), wseq ((offset, count, vector layer, 0) int32 quadruples, n_weights
  * of them), wvec (f32): ops.pack_token_program.  F, Fc (FFN widths) in {16, 128}.
- * Split-precision tensor-core operands (fmt: 0 = fp16 planes, 1 = bf16 planes; csrc/umma_split.cuh): fp32-class results;
+ * Split-precision tensor-core operands (fmt: 0 = fp16 planes, 1 = bf16 planes; csrc/tcgen05.cuh): fp32-class results;
  * fp32 accumulation, residual stream, LayerNorm, softmax and regression heads.  J <= 32. */
 int kpf_token_stack(const float* x, const float* y, const float* r3d, const float* desa, const float* jf, const void* wmat,
                     const void* wseq, const float* wvec, int n_weights, int cross, int pre, int B, int J, int D, int L, int F, int Fc,
@@ -218,7 +218,7 @@ int kpf_exchange_wait(const void* exchange_buffer, int* xstep, int samples_per_s
  *   folded Conv1d+BN embeddings and both relus as a row [hi 128 | lo 128] of two planes in format fmt (0 = fp16, 1 = bf16);
  *   part_acc [B,N/64,128,32] f32 and part_ms [B,N/64,2,32] f32: per 64-point tile the softmax-aggregation numerators
  *   sum_n e[n][c]*exp(w[n][j]-max_tile) and (max_tile, sum_tile).  N % 64 == 0.  Split-precision tensor-core GEMMs
- *   (csrc/umma_split.cuh), weights resident in tensor memory: fp32-class results.
+ *   (csrc/tcgen05.cuh), weights resident in tensor memory: fp32-class results.
  *   stage_out / stage_in (either or both NULL, never both set): the gathered inputs do not depend on the joints, and the two
  *   blocks of KPFusion gather the same taps (model.py:297-306 per block).  With stage_out the launch also stores every tile's
  *   gathered operand image ([B*N/64] x KPF_POINT_EMBED_STAGE_BYTES_PER_TILE bytes, 16-byte aligned); a later launch on the
@@ -252,7 +252,7 @@ int kpf_desa_fused(void* e, long long e_batch_stride, const float* part_acc, con
 /* ---- a12 on tensor cores (csrc/spatial_agg_tc.cu): same contract as kpf_spatial_aggregate for feat_rgb [B,128,fs,fs] with
  * fs*fs % 128 == 0, given as bf16 (feat_rgb_lo = NULL: exact in one plane) or as the two bf16 planes of an fp32 map
  * (kpf_split_planes); wa_packed from ops.pack_spatial_wa (atten_spatial.weight as canonical 16-bit planes, format fmt).
- * Split-precision GEMMs (csrc/umma_split.cuh; fmt 0 = fp16 planes, 1 = bf16 planes for the computed operands): fp32-class results.
+ * Split-precision GEMMs (csrc/tcgen05.cuh; fmt 0 = fp16 planes, 1 = bf16 planes for the computed operands): fp32-class results.
  * split > 1: each sample's cell tiles are spread over `split` CTAs; caller workspace scratch [B,split,128,32] f32 and
  * counters [B] i32 (ZERO on entry; the kernel leaves them zero again), reduction order fixed (deterministic). */
 int kpf_spatial_aggregate_tc(const void* feat_rgb, const void* feat_rgb_lo, const float* joints, const float* depth, long long depth_bs,
@@ -283,13 +283,14 @@ int kpf_crop_rgb(const void* rgb_u8, const double* center, const float* cube, co
  * after GFM.rigid_align (similarity Procrustes, 3x3 SVD per sample in fp64 on the device). */
 int kpf_eval_errors(const float* pred, const float* gt, const float* cube, int B, int J, float* err, float* pa_err, cudaStream_t stream);
 
-/* ---- bring-up self-test of the tcgen05 primitives (csrc/umma.cuh): D[128,N] f32 = A * B^T with bf16 operands.
+/* ---- bring-up self-test of the tcgen05 primitives (csrc/tcgen05.cuh): D[128,N] f32 = A * B^T with bf16 operands.
  * a_mn == 0: A is [128,K] row-major (K-major operand), else A is given transposed [K,128] (MN-major operand);
  * b_mn == 0: B is [N,K] row-major, else B is given as [K,N]. */
 int kpf_umma_selftest(const void* A, const void* B, float* D, int N, int K, int a_mn, int b_mn, cudaStream_t stream);
 
-/* split-precision forms (csrc/umma_split.cuh): D[128,N] f32 = A[128,K] * B[N,K]^T with fp32 A, B carried as (hi, lo) 16-bit planes
- * (fmt 0 = fp16, 1 = bf16), A read from shared memory (a_tmem = 0) or from tensor memory (1); a_exact = 1 drops A's lo plane.
+/* split-precision forms (csrc/tcgen05.cuh): D[128,N] f32 = A[128,K] * B[N,K]^T with fp32 A, B carried as (hi, lo) 16-bit planes
+ * (fmt 0 = fp16, 1 = bf16), K in {16, 32, 64, 128, 256} (anything else is KPF_ERR_BAD_ARGUMENT), A read from shared memory
+ * (a_tmem = 0) or from tensor memory (1); a_exact = 1 drops A's lo plane.
  * cycles (2 x int64 device, may be NULL): one GEMM issue -> completion, eight GEMMs back to back. */
 int kpf_umma_split_selftest(const float* A, const float* B, float* D, int N, int K, int fmt, int a_tmem, int a_exact, long long* cycles,
                             cudaStream_t stream);

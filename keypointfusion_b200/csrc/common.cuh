@@ -225,5 +225,34 @@ __device__ __forceinline__ void tma_bulk_g2s(void* smem_dst, const void* gmem_sr
                  "l"(gmem_src), "r"(bytes), "r"(smem_u32(bar))
                  : "memory");
 }
+// 1-D bulk copy shared -> global through the TMA engine (SASS: UBLKCP), tracked per thread in bulk groups; bytes % 16 == 0, 16 B aligned
+__device__ __forceinline__ void tma_bulk_s2g(void* gmem_dst, const void* smem_src, uint32_t bytes) {
+    asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(gmem_dst), "r"(smem_u32(smem_src)), "r"(bytes) : "memory");
+}
+__device__ __forceinline__ void bulk_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
+// at most N bulk groups still reading their shared-memory sources / still pending
+template <int N>
+__device__ __forceinline__ void bulk_wait_read() { asm volatile("cp.async.bulk.wait_group.read %0;" ::"n"(N) : "memory"); }
+template <int N>
+__device__ __forceinline__ void bulk_wait() { asm volatile("cp.async.bulk.wait_group %0;" ::"n"(N) : "memory"); }
+
+// ---- cp.async (SASS: LDGSTS): 16-byte copies global -> shared, waited for per thread ------------------------------------
+__device__ __forceinline__ void cp_async16(void* smem_dst, const void* gmem_src) {
+    asm volatile("cp.async.ca.shared.global [%0], [%1], 16;" ::"r"(smem_u32(smem_dst)), "l"(gmem_src) : "memory");
+}
+// .cg: through L2 only; the bytes of the chunk past src_bytes (0..16) are zero filled
+__device__ __forceinline__ void cp_async16_cg(void* smem_dst, const void* gmem_src, uint32_t src_bytes) {
+    asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;" ::"r"(smem_u32(smem_dst)), "l"(gmem_src), "r"(src_bytes) : "memory");
+}
+__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
+__device__ __forceinline__ void cp_async_wait_all() { asm volatile("cp.async.wait_all;" ::: "memory"); }
+// at most N committed groups of this thread still pending
+template <int N>
+__device__ __forceinline__ void cp_async_wait_group() { asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory"); }
+
+// named barrier `id` (1..15; 0 is __syncthreads) over `nthreads` threads, a multiple of 32
+__device__ __forceinline__ void named_bar_sync(uint32_t id, uint32_t nthreads) {
+    asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(nthreads) : "memory");
+}
 
 }  // namespace kpf

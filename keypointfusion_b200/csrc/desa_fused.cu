@@ -1,5 +1,5 @@
 // DESA on tensor cores (model/model.py:129-204 + the joint embeddings :323-325), SURVEY.md 8f-1.  Split precision throughout
-// (csrc/umma_split.cuh): every operand is two 16-bit planes, three MMAs per product, so the results are fp32-class.  The point
+// (csrc/tcgen05.cuh): every operand is two 16-bit planes, three MMAs per product, so the results are fp32-class.  The point
 // features e arrive as rows [hi 128 | lo 128] (kpf_point_embed); the tile kernel keeps each scale's W1 / W2 planes in TENSOR
 // MEMORY as the A operands (256 of the 512 columns), which frees their shared memory for the second plane of the activations.
 // Two kernels:
@@ -24,7 +24,7 @@
 //             are issued together; while they run the rows of tile s+2 are copied (indices fetched one iteration earlier);
 //             then epilogue 2 of s and epilogue 1 of s+1.  One __syncthreads per tile.
 //   output    desa_part[b][scale][j][:], jf[b][j][:]; the 512->128 fusion conv follows in kpf_token_stack.
-#include "umma_split.cuh"
+#include "tcgen05.cuh"
 
 namespace kpf {
 
@@ -225,8 +225,8 @@ __global__ void __launch_bounds__(DS_NT, 1) desa_prep_kernel(const DesaParams p)
 #pragma unroll
             for (int j = 0; j < 4; ++j) agg[j] = (4 * jq + j) < J ? agg[j] / sMS[T * 64 + 4 * jq + j] : 0.f;
             uint2 oh, ol;
-            split2(fmt, agg[0], agg[1], oh.x, ol.x);
-            split2(fmt, agg[2], agg[3], oh.y, ol.y);
+            split2<FMT>(agg[0], agg[1], oh.x, ol.x);
+            split2<FMT>(agg[2], agg[3], oh.y, ol.y);
             // (k = channel, n = joint), n contiguous: chunk jq / 2 of the row, half jq & 1
             reinterpret_cast<uint2*>(sAgg + (ch >> 3) * 32 + (jq >> 1) * 8 + (ch & 7))[jq & 1] = oh;
             reinterpret_cast<uint2*>(sAgg + 512 + (ch >> 3) * 32 + (jq >> 1) * 8 + (ch & 7))[jq & 1] = ol;
@@ -240,7 +240,7 @@ __global__ void __launch_bounds__(DS_NT, 1) desa_prep_kernel(const DesaParams p)
         mbar_wait(&wbar, 0);   // (also when the embedding is skipped: the buffer is refilled below)
         if (!given) {
             if (elect_one()) {
-                umma_gemm3_ss(tmem0, opW, opA, id_jf, 128, false);
+                umma_gemm3_ss<128>(tmem0, opW, opA, id_jf, false);
                 umma_commit(&mma_bar);
             }
             __syncwarp();
@@ -272,7 +272,7 @@ __global__ void __launch_bounds__(DS_NT, 1) desa_prep_kernel(const DesaParams p)
                 v = given ? __ldg(p.jf_in + ((size_t)b * J + j) * 128 + ch) : fmaxf(d[i] + bj + wx.x * c.x + wx.y * c.y + wx.z * c.z, 0.f);
                 if (p.jf_out) p.jf_out[((size_t)b * J + j) * 128 + ch] = v;
                 uint32_t h2, l2;   // the joints are points N .. N+J-1 of the grouped set (model.py:168-169)
-                split2(fmt, v, 0.f, h2, l2);
+                split2<FMT>(v, 0.f, h2, l2);
                 erow[(size_t)j * 256] = (uint16_t)h2;
                 erow[(size_t)j * 256 + 128] = (uint16_t)l2;
             }
@@ -280,7 +280,7 @@ __global__ void __launch_bounds__(DS_NT, 1) desa_prep_kernel(const DesaParams p)
         }
         // jf as the B operand [K = channel][N = joint] of the W1 jf GEMMs (same layout as sAgg, whose reader has completed)
         uint4 oh, ol;
-        split8(fmt, d, oh, ol);
+        split8<FMT>(d, oh, ol);
         sAgg[(ch >> 3) * 32 + cg * 8 + (ch & 7)] = oh;
         sAgg[512 + (ch >> 3) * 32 + cg * 8 + (ch & 7)] = ol;
     }
@@ -303,7 +303,7 @@ __global__ void __launch_bounds__(DS_NT, 1) desa_prep_kernel(const DesaParams p)
                     w.hi = smem_u32(sW1 + sc * 4096);
                     w.lo = w.hi + 2048 * 16;
                 }
-                umma_gemm3_ss(tmem0 + 32 * (sc + 1), w, opA, id_jf, 128, false);
+                umma_gemm3_ss<128>(tmem0 + 32 * (sc + 1), w, opA, id_jf, false);
             }
             __syncwarp();
         }
@@ -337,7 +337,7 @@ __global__ void __launch_bounds__(DS_NT, 1) desa_prep_kernel(const DesaParams p)
                 SmemOp w = opW;
                 w.hi = smem_u32(sW1);
                 w.lo = w.hi + 2048 * 16;
-                umma_gemm3_ss(tmem0 + 32, w, opA, id_jf, 128, false);
+                umma_gemm3_ss<128>(tmem0 + 32, w, opA, id_jf, false);
                 umma_commit(&mma_bar);
             }
             __syncwarp();
@@ -498,15 +498,15 @@ __global__ void __launch_bounds__(DS_TILE_NT, 1) desa_tile_kernel(const DesaPara
         // 16-byte chunk 8k + g8 of the 512-byte row [hi 128 | lo 128]: k-chunk (8k + g8) & 15 of plane k >> 1; the eight g8 lanes of a row
         // read 128 contiguous bytes = ONE request.  (.cg: the rows stream through L2 only -- measured 9 % faster than .ca, whose L1 is
         // ~30 KB next to 225 KB of shared memory.)  Rows beyond the last joint are zero filled (src-size 0).
-        asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;" ::"r"(smem_u32(X + (k >> 1) * 2048 + (k & 1) * 64)), "l"(src + 64 * k), "r"(nbytes) : "memory");
+        cp_async16_cg(X + (k >> 1) * 2048 + (k & 1) * 64, src + 64 * k, nbytes);
         if (k == 0 && g8 == 0) {   // xyz of the row's point and of its centre -> staging; the tail is built from it one iteration later
             const float4* tab = p.xyz4 + (size_t)it_copy.b * (N + 32);
             float4* st = sXyz + ((item & 1) * 128 + row) * 2;
-            asm volatile("cp.async.ca.shared.global [%0], [%1], 16;" ::"r"(smem_u32(st)), "l"(tab + ii[h]) : "memory");
-            asm volatile("cp.async.ca.shared.global [%0], [%1], 16;" ::"r"(smem_u32(st + 1)), "l"(tab + N + (ok ? jj : 0)) : "memory");
+            cp_async16(st, tab + ii[h]);
+            cp_async16(st + 1, tab + N + (ok ? jj : 0));
             tail_ok[h] = ok;
         }
-        if (part == 7) asm volatile("cp.async.commit_group;" ::: "memory");
+        if (part == 7) cp_async_commit();
     };
     auto store_tail = [&](int item) {   // group_xyz_norm = (xyz[idx] - centre) / radius   model.py:177
         if (g8 != 0) return;
@@ -523,7 +523,7 @@ __global__ void __launch_bounds__(DS_TILE_NT, 1) desa_tile_kernel(const DesaPara
             }
             uint4* X = sX + (item % 3) * DS_XBUF + 4096 + (row >> 3) * 8 + (row & 7);
             uint4 th, tl;
-            split8(fmt, t8, th, tl);
+            split8<FMT>(t8, th, tl);
             X[0] = th;
             X[128] = tl;
         }
@@ -578,7 +578,7 @@ __global__ void __launch_bounds__(DS_TILE_NT, 1) desa_tile_kernel(const DesaPara
         if (!issuer) fetch_idx();   // fill: indices of i0
         for (int s = i0 - 2; s < i1; ++s) {
             if (s >= i0 - 1) {
-                asm volatile("cp.async.wait_group 0;" ::: "memory");   // this thread's rows of tile s + 1 have landed
+                cp_async_wait_group<0>();   // this thread's rows of tile s + 1 have landed
                 if (!issuer && s + 1 < i1) store_tail(s + 1);          // ... and their xyz: the operand's K tail
                 fence_proxy_async();
                 tc_fence_before();
@@ -598,10 +598,10 @@ __global__ void __launch_bounds__(DS_TILE_NT, 1) desa_tile_kernel(const DesaPara
                             a.hi = tmem0 + TW1_HI; a.lo = tmem0 + TW1_LO;
                             SmemOp xb, ta, tb;
                             xb.hi = X; xb.lo = X + 2048 * 16; xb.lbo = 128; xb.sbo = 2048;
-                            umma_gemm3_ts(tmem0 + ACC1, a, xb, id128, 128, false);
+                            umma_gemm3_ts<128>(tmem0 + ACC1, a, xb, id128, false);
                             ta.hi = smem_u32(sW1t); ta.lo = ta.hi + 256 * 16; ta.lbo = 2048; ta.sbo = 128;
                             tb.hi = X + 4096 * 16; tb.lo = tb.hi + 128 * 16; tb.lbo = 0; tb.sbo = 128;   // lbo 0: k-chunk 1 (zero weights) re-reads chunk 0
-                            umma_gemm3_ss(tmem0 + ACC1, ta, tb, id128, 16, true);
+                            umma_gemm3_ss<16>(tmem0 + ACC1, ta, tb, id128, true);
                             umma_commit(&g1_bar);
                         }
                         if (s >= i0) {   // layer 2 of tile s: D2[c][row] = W2 h
@@ -609,7 +609,7 @@ __global__ void __launch_bounds__(DS_TILE_NT, 1) desa_tile_kernel(const DesaPara
                             a.hi = tmem0 + TW2_HI; a.lo = tmem0 + TW2_LO;
                             SmemOp hb;
                             hb.hi = smem_u32(sX + (s % 3) * DS_XBUF); hb.lo = hb.hi + 2048 * 16; hb.lbo = 2048; hb.sbo = 128;
-                            umma_gemm3_ts(tmem0 + ACC2, a, hb, umma_idesc_f16(128, 128, false, true, fmt, fmt), 128, false);
+                            umma_gemm3_ts<128>(tmem0 + ACC2, a, hb, umma_idesc_f16(128, 128, false, true, fmt, fmt), false);
                             umma_commit(&g2_bar);
                         }
                     }
@@ -651,7 +651,7 @@ __global__ void __launch_bounds__(DS_TILE_NT, 1) desa_tile_kernel(const DesaPara
 #pragma unroll
                         for (int c = 0; c < 2; ++c) {
                             uint4 hh, hl;
-                            split8(fmt, a + 8 * c, hh, hl);
+                            split8<FMT>(a + 8 * c, hh, hl);
                             H[(ch >> 3) * 128 + (4 * cg + 2 * hf + c) * 8 + (ch & 7)] = hh;
                             H[2048 + (ch >> 3) * 128 + (4 * cg + 2 * hf + c) * 8 + (ch & 7)] = hl;
                         }

@@ -13,7 +13,7 @@
 //       D[c][j] = sum_n e[n][c] p[n][j]                                    tcgen05 with MN-major operands
 //     outputs: e [B,N,128] bf16, and per tile (D, max, sum) partials that the DESA kernel combines flash-style.
 //   Weights (96 KB bf16) stay resident in shared memory; CTAs are persistent over tiles.
-#include "umma_split.cuh"
+#include "tcgen05.cuh"
 
 namespace kpf {
 
@@ -135,11 +135,6 @@ constexpr int PE_ST_X1 = 20 * 8 * 16;                      // bytes per (plane, 
 constexpr int PE_ST_T = (21 * 65 + 3) * 4;                 // bytes of sT
 constexpr int PE_STAGE_BYTES = 16 * PE_ST_X1 + 2 * 1024 * 16 + PE_ST_T;
 
-// bulk copy shared -> global through the TMA engine (SASS: UBLKCP); bytes % 16 == 0, 16 B aligned
-__device__ __forceinline__ void tma_bulk_s2g(void* gmem_dst, const void* smem_src, uint32_t bytes) {
-    asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(gmem_dst), "r"(smem_u32(smem_src)), "r"(bytes) : "memory");
-}
-
 // The whole point stage, computed TRANSPOSED: D^T[channel][point] = W[channel][k] X[point][k].  The folded weights (K = 384, two
 // 16-bit planes) stay in TENSOR MEMORY for the life of the persistent CTA as the A operands; a tile is 64 points whose gathered
 // inputs are written as K-major B operand planes; a thread of the epilogue owns one output channel (its TMEM lane) and 16 points.
@@ -161,7 +156,7 @@ __global__ void __launch_bounds__(PE_NT, 1) point_embed_kernel(const PointParams
     __shared__ __align__(8) uint64_t mma_bar, in_bar;
     __shared__ uint32_t tmem_slot;
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-    const int warp_u = warp_index_uniform();  // MMA issue: one elected lane of warp 0 from warp-uniform code (umma.cuh)
+    const int warp_u = warp_index_uniform();  // MMA issue: one elected lane of warp 0 from warp-uniform code (tcgen05.cuh)
     // gather: warp = 8 points x 4 chunk lanes (64 contiguous bytes of a tap row per point per load; the 8 points fill the 8 rows x
     // 16 B core matrices of the operand, so the stores are conflict free).  Warps 0-7 (grp 0) take the depth-branch and weight-map
     // chunks and the joint offsets, warps 8-15 (grp 1) the rgb-branch chunks of the same 64 points.
@@ -301,7 +296,7 @@ __global__ void __launch_bounds__(PE_NT, 1) point_embed_kernel(const PointParams
             for (int u = 0; u < 5; ++u) {
                 if (u < nload) {
                     uint4 oh, ol;
-                    split8(fmt, acc[u], oh, ol);
+                    split8<FMT>(acc[u], oh, ol);
                     if (grp == 1) {
                         x2r[(4 * u + sub) * 8] = oh;
                         x2r[1024 + (4 * u + sub) * 8] = ol;
@@ -335,7 +330,7 @@ __global__ void __launch_bounds__(PE_NT, 1) point_embed_kernel(const PointParams
             if (lane < 16) tma_bulk_s2g(dst + (size_t)lane * PE_ST_X1, sX1 + (lane >> 3) * 2048 + (lane & 7) * 256, PE_ST_X1);
             else if (lane == 16) tma_bulk_s2g(dst + 16 * PE_ST_X1, sX2, 2 * 1024 * 16);
             else tma_bulk_s2g(dst + 16 * PE_ST_X1 + 2 * 1024 * 16, sT, PE_ST_T);
-            asm volatile("cp.async.bulk.commit_group;" ::: "memory");
+            bulk_commit();
         }
         // ---- K4b: items 0..J-1 = [unit offset xyz, closeness] of a joint, item J = the point's xyz; item i fills half (i & 1) of
         //      k-chunk 20 + i / 2 of A1 (ops.pack_point_embed orders W1's columns to match).  The eight threads of a point (four
@@ -363,8 +358,8 @@ __global__ void __launch_bounds__(PE_NT, 1) point_embed_kernel(const PointParams
                     o2 = pz;
                 }
                 uint2 oh, ol;
-                split2(fmt, o0, o1, oh.x, ol.x);
-                split2(fmt, o2, o3, oh.y, ol.y);
+                split2<FMT>(o0, o1, oh.x, ol.x);
+                split2<FMT>(o2, o3, oh.y, ol.y);
                 reinterpret_cast<uint2*>(x1r + (20 + (j >> 1)) * 8)[j & 1] = oh;
                 reinterpret_cast<uint2*>(x1r + 2048 + (20 + (j >> 1)) * 8)[j & 1] = ol;
             }
@@ -382,7 +377,7 @@ __global__ void __launch_bounds__(PE_NT, 1) point_embed_kernel(const PointParams
             if (rs == 0) sRed[rj] = rj < J ? m : -INFINITY;
         }
         // the bulk stores have read their sources: sT is rewritten after the barrier below, the operands by the next tile
-        if (ST_OUT && warp == 0 && lane < 18) asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
+        if (ST_OUT && warp == 0 && lane < 18) bulk_wait_read<0>();
         fence_proxy_async();
         tc_fence_before();
         __syncthreads();
@@ -395,10 +390,10 @@ __global__ void __launch_bounds__(PE_NT, 1) point_embed_kernel(const PointParams
                 // B operands: 128 B between k-chunks, 4096 / 2048 B between 8-point groups
                 a.hi = tmem0 + PE_W1H; a.lo = tmem0 + PE_W1L;
                 xb.hi = smem_u32(sX1); xb.lo = xb.hi + 2048 * 16; xb.lbo = 128; xb.sbo = 4096;
-                umma_gemm3_ts(tmem0 + PE_ACC1, a, xb, id64, 256, false);
+                umma_gemm3_ts<256>(tmem0 + PE_ACC1, a, xb, id64, false);
                 a.hi = tmem0 + PE_W2H; a.lo = tmem0 + PE_W2L;
                 xb.hi = smem_u32(sX2); xb.lo = xb.hi + 1024 * 16; xb.lbo = 128; xb.sbo = 2048;
-                umma_gemm3_ts(tmem0 + PE_ACC2, a, xb, id64, 128, false);
+                umma_gemm3_ts<128>(tmem0 + PE_ACC2, a, xb, id64, false);
                 umma_commit(&mma_bar);
             }
             __syncwarp();
@@ -416,13 +411,13 @@ __global__ void __launch_bounds__(PE_NT, 1) point_embed_kernel(const PointParams
                 if (j < J) sT[j * 65 + r] = pj[k];
             }
             uint4 oh, ol;
-            split8(fmt, pj, oh, ol);
+            split8<FMT>(pj, oh, ol);
             sP[(r >> 3) * 32 + sub * 8 + (r & 7)] = oh;
             sP[256 + (r >> 3) * 32 + sub * 8 + (r & 7)] = ol;
         }
         if (tid < 32) ms[tid] = sRed[tid];
         if (grp == 0) {   // the numerators and their sums involve only warps 0-7: their own barrier, so nobody waits for the MMA issuer here
-            asm volatile("bar.sync 1, 256;" ::: "memory");
+            named_bar_sync(1, 256);
             const int rj = tid >> 3, rs = tid & 7;
             float sm_ = 0.f;
             if (rj < J) {
@@ -449,7 +444,7 @@ __global__ void __launch_bounds__(PE_NT, 1) point_embed_kernel(const PointParams
             for (int i = 0; i < 8; ++i) {
                 const float e0 = fmaxf(fmaxf(a[2 * i] + b1, 0.f) + rr[2 * i] + b2, 0.f);
                 const float e1 = fmaxf(fmaxf(a[2 * i + 1] + b1, 0.f) + rr[2 * i + 1] + b2, 0.f);
-                split2(fmt, e0, e1, eh[i], el[i]);
+                split2<FMT>(e0, e1, eh[i], el[i]);
                 // staged rows [point][hi 128 | lo 128]: a warp's 32 channels are 64 contiguous bytes of each
                 se[(16 * cg + 2 * i) * 256] = (uint16_t)eh[i];
                 se[(16 * cg + 2 * i) * 256 + 128] = (uint16_t)el[i];
@@ -479,7 +474,7 @@ __global__ void __launch_bounds__(PE_NT, 1) point_embed_kernel(const PointParams
                 a.hi = tmem0 + PE_EH; a.lo = tmem0 + PE_EL;
                 SmemOp pb;
                 pb.hi = smem_u32(sP); pb.lo = pb.hi + 256 * 16; pb.lbo = 512; pb.sbo = 128;
-                umma_gemm3_ts(tmem0 + PE_ACC3, a, pb, umma_idesc_f16(128, 32, false, true, fmt, fmt), PE_TP, false);
+                umma_gemm3_ts<PE_TP>(tmem0 + PE_ACC3, a, pb, umma_idesc_f16(128, 32, false, true, fmt, fmt), false);
                 umma_commit(&mma_bar);
             }
             __syncwarp();
@@ -503,7 +498,7 @@ __global__ void __launch_bounds__(PE_NT, 1) point_embed_kernel(const PointParams
         tc_fence_before();
         tile_par ^= 1;
     }
-    if (ST_OUT && warp == 0 && lane < 18) asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");   // the staged images are written
+    if (ST_OUT && warp == 0 && lane < 18) bulk_wait<0>();   // the staged images are written
     __syncthreads();
     if (warp == 0) tmem_dealloc(tmem0, 512);
 }

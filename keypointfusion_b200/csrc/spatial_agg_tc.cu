@@ -5,14 +5,14 @@
 //   epilogue sw = sigmoid(S1 + ba) -> global ; G[hw][j] = fc_w[hw] (sg GAM + (1-sg) sw)    (thread = cell)
 //   GEMM B   out[c][j] += sum_hw relu(F[c][hw]) G[hw][j]                                   M = 128 channels, N = 32, K = 128 cells
 //
-// Split precision (csrc/umma_split.cuh): the bf16 feature map is exact in one plane (fp32 maps arrive as two bf16 planes from
+// Split precision (csrc/tcgen05.cuh): the bf16 feature map is exact in one plane (fp32 maps arrive as two bf16 planes from
 // kpf_split_planes); its GEMM partners (Wa's feature part, G) are THREE bf16 planes (both operands of an MMA must share a format);
 // the heat map and Wa's heat-map part are two planes in format fmt.  fp32-class results.
 // The NCHW feature tile [128 c x 128 hw] is staged ONCE per tile with 16-byte cp.async into the SWIZZLE_NONE canonical
 // layout and read by GEMM A as an MN-major A operand (M = hw contiguous) and -- same bytes, LBO/SBO swapped, after an
 // in-place relu pass -- by GEMM B as a K-major A operand (K = hw contiguous).  One CTA per sample sweeps its HW/128
 // tiles, accumulating out[c][j] in TMEM; the next tile's features are prefetched while the current one is consumed.
-#include "umma_split.cuh"
+#include "tcgen05.cuh"
 
 namespace kpf {
 
@@ -33,11 +33,6 @@ struct SpatialParams {
     int* counters;    // [B], zero on entry, zero again on exit
     int split, fmt;
 };
-
-__device__ __forceinline__ void cp_async16(void* smem, const void* gmem) {
-    asm volatile("cp.async.ca.shared.global [%0], [%1], 16;" ::"r"(smem_u32(smem)), "l"(gmem) : "memory");
-}
-__device__ __forceinline__ void cp_async_wait_all() { asm volatile("cp.async.wait_all;" ::: "memory"); }
 
 constexpr int K5_NT = 512;   // thread = (cell or channel row = 32 * (warp % 4) + lane, joint group warp / 4 of 8 joints)
 
@@ -60,7 +55,7 @@ __global__ void __launch_bounds__(K5_NT, 1) spatial_aggregate_tc_kernel(const Sp
     __shared__ uint32_t tmem_slot;
     __shared__ CamF cam;
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-    const int warp_u = warp_index_uniform();  // MMA issue: one elected lane of warp 0 from warp-uniform code (umma.cuh)
+    const int warp_u = warp_index_uniform();  // MMA issue: one elected lane of warp 0 from warp-uniform code (tcgen05.cuh)
     const int q = warp & 3, cg = warp >> 2, row = 32 * q + lane;   // TMEM lane `row` (cell / channel), joints [8cg, 8cg + 8)
     const int b = blockIdx.x / p.split, sp = blockIdx.x - b * p.split, J = p.J, fs = p.fs, HW = fs * fs, T = HW / 128;
     const int t_begin = sp * (T / p.split), t_end = t_begin + T / p.split;
@@ -162,7 +157,7 @@ __global__ void __launch_bounds__(K5_NT, 1) spatial_aggregate_tc_kernel(const Sp
         }
         {
             uint4 oh, ol;
-            split8(fmt, hm, oh, ol);
+            split8<FMT>(hm, oh, ol);
             sHm[cg * 128 + row] = oh;
             sHm[512 + cg * 128 + row] = ol;
         }
@@ -202,7 +197,7 @@ __global__ void __launch_bounds__(K5_NT, 1) spatial_aggregate_tc_kernel(const Sp
                 SmemOp a, bo;
                 a.hi = smem_u32(sHm); a.lo = a.hi + 512 * 16; a.lbo = 2048; a.sbo = 128;
                 bo.hi = smem_u32(sWa + 1536); bo.lo = bo.hi + 128 * 16; bo.lbo = 512; bo.sbo = 128;
-                umma_gemm3_ss(tmem0 + ACC1, a, bo, umma_idesc_f16(128, 32, false, false, fmt, fmt), 32, true);
+                umma_gemm3_ss<32>(tmem0 + ACC1, a, bo, umma_idesc_f16(128, 32, false, false, fmt, fmt), true);
                 umma_commit(&mma_bar);
             }
             __syncwarp();

@@ -1,5 +1,5 @@
 // Keypoint-token transformer stacks on tcgen05 tensor cores, split precision (fp32 operands as two 16-bit planes, three MMAs
-// per product, fp32 accumulation in TMEM: csrc/umma_split.cuh) -- results are fp32-class, which the 0.05 mm joint bar needs.
+// per product, fp32 accumulation in TMEM: csrc/tcgen05.cuh) -- results are fp32-class, which the 0.05 mm joint bar needs.
 //
 //   encoder : KP_Interaction_TR.forward, model/model.py:45-126 (transformers 4.25.1 BertLayer x L):
 //             h = pos_emb + x W_emb^T + b ; L x { self-attention, +res, LN, FFN(gelu), +res, LN } ; pred = cls_head(h) + residual(x)
@@ -23,7 +23,7 @@
 //   * Weights stream through a ring of four 32 KB slots (a 128x128 matrix with both planes = two half-K tiles) filled by a
 //     dedicated producer warp with cp.async.bulk; tcgen05.commit on a slot's "empty" barrier hands it back.  Per-layer vectors
 //     are double-buffered the same way.  The fp32 residual stream stays in registers.
-#include "umma_split.cuh"
+#include "tcgen05.cuh"
 
 namespace kpf {
 
@@ -192,7 +192,7 @@ __global__ void __launch_bounds__(TS_NT, 1) token_stack_kernel(const TokParams p
 
     // =========================== workers ===========================
     // all worker-only synchronisation goes through named barrier 1 (512 threads): the producer warp has left
-    auto wsync = [&]() { asm volatile("bar.sync 1, 512;" ::: "memory"); };
+    auto wsync = [&]() { named_bar_sync(1, 512); };
     uint32_t bar_phase[4] = {0, 0, 0, 0};
     auto wait_bar = [&](int i) {
         mbar_wait(&bars[i], bar_phase[i]);
@@ -219,14 +219,14 @@ __global__ void __launch_bounds__(TS_NT, 1) token_stack_kernel(const TokParams p
             SmemOp a, bo;
             a.hi = slot_addr(e + h); a.lo = a.hi + 16384; a.lbo = 2048; a.sbo = 128;
             bo.hi = smem_u32(act) + h * 4096; bo.lo = bo.hi + TS_PLANE * 16; bo.lbo = 512; bo.sbo = 128;
-            umma_gemm3_ss(tmem0 + acc, a, bo, id, 64, accumulate || h > 0);
+            umma_gemm3_ss<64>(tmem0 + acc, a, bo, id, accumulate || h > 0);
             umma_commit(&empty[(e + h) & (TS_RING - 1)]);
         }
     };
     const uint32_t xidx = (uint32_t)((f >> 3) * 32 + c * 8 + (f & 7));   // this thread's chunk of an MN-major [128][32] operand plane
     auto write_act = [&](uint4* buf, const float* v) {   // 8 tokens of feature f -> both planes
         uint4 hi, lo;
-        split8(fmt, v, hi, lo);
+        split8<FMT>(v, hi, lo);
         buf[xidx] = hi;
         buf[TS_PLANE + xidx] = lo;
     };
@@ -348,10 +348,10 @@ __global__ void __launch_bounds__(TS_NT, 1) token_stack_kernel(const TokParams p
                     sLead[4 * t + k] = s;
                 }
                 uint4 hi, lo;
-                split8(fmt, tl, hi, lo);
+                split8<FMT>(tl, hi, lo);
                 bufAt[t] = hi;
                 bufAt[64 + t] = lo;
-                split8(fmt, tl + 8, hi, lo);
+                split8<FMT>(tl + 8, hi, lo);
                 bufAt[32 + t] = hi;
                 bufAt[96 + t] = lo;
             }
@@ -367,7 +367,7 @@ __global__ void __launch_bounds__(TS_NT, 1) token_stack_kernel(const TokParams p
                         SmemOp a, bo;
                         a.hi = slot_addr(g + 2); a.lo = a.hi + 256 * 16; a.lbo = 2048; a.sbo = 128;
                         bo.hi = smem_u32(bufAt); bo.lo = bo.hi + 64 * 16; bo.lbo = 512; bo.sbo = 128;
-                        umma_gemm3_ss(tmem0 + ACC_X, a, bo, umma_idesc_f16(128, 32, false, false, fmt, fmt), 16, true);
+                        umma_gemm3_ss<16>(tmem0 + ACC_X, a, bo, umma_idesc_f16(128, 32, false, false, fmt, fmt), true);
                         umma_commit(&empty[(g + 2) & (TS_RING - 1)]);
                     }
                     umma_commit(&bars[0]);
@@ -419,7 +419,7 @@ __global__ void __launch_bounds__(TS_NT, 1) token_stack_kernel(const TokParams p
 #pragma unroll
             for (int i = 0; i < 8; ++i) a[i] = tokv[i] ? a[i] + bk : 0.f;
             uint4 hi, lo;
-            split8(fmt, a, hi, lo);
+            split8<FMT>(a, hi, lo);
             bufK[qidx] = hi;
             bufK[TS_PLANE + qidx] = lo;
         }
@@ -430,7 +430,7 @@ __global__ void __launch_bounds__(TS_NT, 1) token_stack_kernel(const TokParams p
 #pragma unroll
             for (int i = 0; i < 8; ++i) a[i] = tokv[i] ? (a[i] + bq) * qscale : 0.f;
             uint4 hi, lo;
-            split8(fmt, a, hi, lo);
+            split8<FMT>(a, hi, lo);
             bufQ[qidx] = hi;
             bufQ[TS_PLANE + qidx] = lo;
         }
@@ -442,7 +442,7 @@ __global__ void __launch_bounds__(TS_NT, 1) token_stack_kernel(const TokParams p
                 SmemOp a, bo;
                 a.hi = smem_u32(bufQ); a.lo = a.hi + TS_PLANE * 16; a.lbo = 2048; a.sbo = 128;
                 bo.hi = smem_u32(bufK); bo.lo = bo.hi + TS_PLANE * 16; bo.lbo = 2048; bo.sbo = 128;
-                umma_gemm3_ss(tmem0 + ACC_S, a, bo, umma_idesc_f16(128, 128, true, true, fmt, fmt), 32, false);
+                umma_gemm3_ss<32>(tmem0 + ACC_S, a, bo, umma_idesc_f16(128, 128, true, true, fmt, fmt), false);
                 umma_commit(&bars[0]);
                 issue_proj(ACC_V, kv_src, g + 4, false);
                 umma_commit(&bars[1]);
@@ -468,7 +468,7 @@ __global__ void __launch_bounds__(TS_NT, 1) token_stack_kernel(const TokParams p
             }
             sSum[c * 128 + f] = psum;
             uint4 hi, lo;   // P: K-major B operand [N = 32h + t][K = 32 keys], over the (dead) Q
-            split8(fmt, own, hi, lo);
+            split8<FMT>(own, hi, lo);
             bufQ[c * 128 + f] = hi;
             bufQ[TS_PLANE + c * 128 + f] = lo;
         }
@@ -479,7 +479,7 @@ __global__ void __launch_bounds__(TS_NT, 1) token_stack_kernel(const TokParams p
 #pragma unroll
             for (int i = 0; i < 8; ++i) a[i] = tokv[i] ? a[i] + bv : 0.f;
             uint4 hi, lo;
-            split8(fmt, a, hi, lo);
+            split8<FMT>(a, hi, lo);
             tmem_st_nw<4>(tmem + VT_HI + 4 * c, reinterpret_cast<const float*>(&hi));
             tmem_st_nw<4>(tmem + VT_LO + 4 * c, reinterpret_cast<const float*>(&lo));
             tmem_wait_st();
@@ -493,7 +493,7 @@ __global__ void __launch_bounds__(TS_NT, 1) token_stack_kernel(const TokParams p
                 a.hi = tmem0 + VT_HI; a.lo = tmem0 + VT_LO;
                 SmemOp bo;
                 bo.hi = smem_u32(bufQ); bo.lo = bo.hi + TS_PLANE * 16; bo.lbo = 2048; bo.sbo = 128;
-                umma_gemm3_ts(tmem0 + ACC_O, a, bo, umma_idesc_f16(128, 128, false, false, fmt, fmt), 32, false);
+                umma_gemm3_ts<32>(tmem0 + ACC_O, a, bo, umma_idesc_f16(128, 128, false, false, fmt, fmt), false);
                 umma_commit(&bars[0]);
             }
             __syncwarp();
@@ -578,7 +578,7 @@ __global__ void __launch_bounds__(TS_NT, 1) token_stack_kernel(const TokParams p
                     wait_full(g + 8);
                     tc_fence_after();
                     bo.hi = slot_addr(g + 8); bo.lo = bo.hi + 256 * 16; bo.lbo = 256; bo.sbo = 128;
-                    umma_gemm3_ss(tmem0 + ACC_F, a, bo, umma_idesc_f16(128, 16, true, false, fmt, fmt), 128, false);
+                    umma_gemm3_ss<128>(tmem0 + ACC_F, a, bo, umma_idesc_f16(128, 16, true, false, fmt, fmt), false);
                 } else {
 #pragma unroll 1
                     for (int h = 0; h < 2; ++h) {
@@ -587,7 +587,7 @@ __global__ void __launch_bounds__(TS_NT, 1) token_stack_kernel(const TokParams p
                         SmemOp ah = a;
                         ah.hi += h * 4096; ah.lo += h * 4096;
                         bo.hi = slot_addr(g + 8 + h); bo.lo = bo.hi + 16384; bo.lbo = 2048; bo.sbo = 128;
-                        umma_gemm3_ss(tmem0 + ACC_F, ah, bo, umma_idesc_f16(128, 128, true, false, fmt, fmt), 64, h > 0);
+                        umma_gemm3_ss<64>(tmem0 + ACC_F, ah, bo, umma_idesc_f16(128, 128, true, false, fmt, fmt), h > 0);
                         umma_commit(&empty[(g + 8 + h) & (TS_RING - 1)]);
                     }
                 }
@@ -607,8 +607,8 @@ __global__ void __launch_bounds__(TS_NT, 1) token_stack_kernel(const TokParams p
                     a[i] = tv ? (act == 1 ? gelu_erf(u) : fmaxf(u, 0.f)) : 0.f;
                 }
                 uint2 hi, lo;
-                split2(fmt, a[0], a[1], hi.x, lo.x);
-                split2(fmt, a[2], a[3], hi.y, lo.y);
+                split2<FMT>(a[0], a[1], hi.x, lo.x);
+                split2<FMT>(a[2], a[3], hi.y, lo.y);
                 // hidden operand: K-major B [N = 32 tokens][K = 16]: chunk (k >> 3) * 32 + token
                 reinterpret_cast<uint2*>(bufY + (c >> 1) * 32 + lane)[c & 1] = hi;
                 reinterpret_cast<uint2*>(bufY + TS_PLANE + (c >> 1) * 32 + lane)[c & 1] = lo;
@@ -623,7 +623,7 @@ __global__ void __launch_bounds__(TS_NT, 1) token_stack_kernel(const TokParams p
                         a[i] = tv ? (act == 1 ? gelu_erf(u) : fmaxf(u, 0.f)) : 0.f;
                     }
                     uint4 hi, lo;
-                    split8(fmt, a, hi, lo);
+                    split8<FMT>(a, hi, lo);
                     bufY[(4 * c + j4) * 32 + lane] = hi;
                     bufY[TS_PLANE + (4 * c + j4) * 32 + lane] = lo;
                 }
@@ -639,7 +639,7 @@ __global__ void __launch_bounds__(TS_NT, 1) token_stack_kernel(const TokParams p
                 const uint32_t id = umma_idesc_f16(128, 32, false, false, fmt, fmt);
                 if (F == 16) {
                     a.hi = slot_addr(g + 8) + 512 * 16; a.lo = a.hi + 256 * 16; a.lbo = 2048; a.sbo = 128;
-                    umma_gemm3_ss(tmem0 + ACC_X, a, bo, id, 16, false);
+                    umma_gemm3_ss<16>(tmem0 + ACC_X, a, bo, id, false);
                     umma_commit(&empty[(g + 8) & (TS_RING - 1)]);
                 } else {
 #pragma unroll 1
@@ -649,7 +649,7 @@ __global__ void __launch_bounds__(TS_NT, 1) token_stack_kernel(const TokParams p
                         a.hi = slot_addr(g + 10 + h); a.lo = a.hi + 16384; a.lbo = 2048; a.sbo = 128;
                         SmemOp bh = bo;
                         bh.hi += h * 4096; bh.lo += h * 4096;
-                        umma_gemm3_ss(tmem0 + ACC_X, a, bh, id, 64, h > 0);
+                        umma_gemm3_ss<64>(tmem0 + ACC_X, a, bh, id, h > 0);
                         umma_commit(&empty[(g + 10 + h) & (TS_RING - 1)]);
                     }
                 }
@@ -702,7 +702,7 @@ __global__ void __launch_bounds__(TS_NT, 1) token_stack_kernel(const TokParams p
             // barrier, so relaxed additions suffice and all ranks' counters are updated at once (eight serial release-reductions and a
             // 512-thread system fence cost 22 us per step at 8 GPUs: KPF_EXCHANGE=off vs peer, DESIGN.md section 7).
             __threadfence_system();
-            asm volatile("bar.sync 2, 96;" ::: "memory");
+            named_bar_sync(2, 96);
             if (tid < p.world) asm volatile("red.relaxed.sys.global.add.u32 [%0], 1;" ::"l"(p.peer_bases[tid]) : "memory");
         }
     }

@@ -1,6 +1,6 @@
-// Self-test of the tcgen05 building blocks in umma.cuh: one 128 x N x K bf16 GEMM through shared-memory descriptors
+// Self-test of the tcgen05 building blocks in tcgen05.cuh: one 128 x N x K bf16 GEMM through shared-memory descriptors
 // (K-major and MN-major operands), TMEM accumulation and tcgen05.ld read-back.  Used by tests/test_umma_gpu.py.
-#include "umma.cuh"
+#include "tcgen05.cuh"
 
 namespace kpf {
 
@@ -49,7 +49,7 @@ umma_selftest_kernel(const __nv_bfloat16* __restrict__ A, const __nv_bfloat16* _
     const uint32_t tmem = tmem_slot;
     if (tid == 0) {
         const uint32_t a_lbo = a_mn ? 16 * 128 : 128 * 16, b_lbo = b_mn ? (N / 8) * 128 : N * 16;
-        umma_gemm(tmem, smem_u32(sA), a_lbo, 128, smem_u32(sB), b_lbo, 128, umma_idesc_bf16(128, N, a_mn != 0, b_mn != 0), K, false);
+        umma_gemm(tmem, smem_u32(sA), a_lbo, 128, smem_u32(sB), b_lbo, 128, umma_idesc_f16(128, N, a_mn != 0, b_mn != 0, FMT_BF16, FMT_BF16), K, false);
         umma_commit(&bar);
     }
     mbar_wait(&bar, 0);
@@ -57,7 +57,7 @@ umma_selftest_kernel(const __nv_bfloat16* __restrict__ A, const __nv_bfloat16* _
     const int row = tid;  // lane == row of D
     for (int c0 = 0; c0 < N; c0 += 32) {
         float v[32];
-        tmem_ld32(tmem + ((uint32_t)(warp * 32) << 16) + c0, v);
+        tmem_ld<32>(tmem + ((uint32_t)(warp * 32) << 16) + c0, v);
         for (int i = 0; i < 32 && c0 + i < N; ++i) D[(size_t)row * N + c0 + i] = v[i];
     }
     tc_fence_before();

@@ -475,7 +475,7 @@ def ball_query(xyz, centers, radius, nsample):
 
 # ------------------------------------------------------------------------------------------------ split-precision operands
 # fp32 weights / activations reach the tensor cores as two 16-bit planes (hi = rn16(x), lo = rn16(x - hi)), three MMAs per product
-# (csrc/umma_split.cuh).  fp16 planes carry 22 mantissa bits (results indistinguishable from an fp32 GEMM), bf16 planes 16 bits
+# (csrc/tcgen05.cuh).  fp16 planes carry 22 mantissa bits (results indistinguishable from an fp32 GEMM), bf16 planes 16 bits
 # with the full fp32 exponent range.  KPF_SPLIT_FMT=bf16 selects the latter, e.g. for a checkpoint with |w| or |activation| > 65504.
 FMT_F16, FMT_BF16 = 0, 1
 SPLIT_FMT = FMT_BF16 if os.environ.get("KPF_SPLIT_FMT", "fp16").lower() in ("bf16", "1") else FMT_F16
@@ -498,7 +498,7 @@ def split_planes(W, fmt=None):
 
 
 def _canon16(W16):
-    """[N,K] 16-bit -> SWIZZLE_NONE canonical K-major operand [K/8][N][8] (csrc/umma.cuh), flattened, as raw int16 bits."""
+    """[N,K] 16-bit -> SWIZZLE_NONE canonical K-major operand [K/8][N][8] (csrc/tcgen05.cuh), flattened, as raw int16 bits."""
     N, K = W16.shape
     assert K % 8 == 0
     return W16.reshape(N, K // 8, 8).permute(1, 0, 2).contiguous().reshape(-1).view(torch.int16)
@@ -840,7 +840,7 @@ def _zero_counters(n, device):
 
 def split_planes3_bf16(W):
     """fp32 -> three bf16 planes (hi + mid + lo = W to 2^-24): the GEMM partner of a bf16 feature-map operand (both operands of an
-    MMA share one format, csrc/umma_split.cuh)."""
+    MMA share one format, csrc/tcgen05.cuh)."""
     W = W.detach().float()
     hi = W.bfloat16()
     r = W - hi.float()

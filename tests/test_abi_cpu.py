@@ -23,6 +23,14 @@ def test_library_exports_every_declared_symbol():
     assert _lib.lib().kpf_abi_version() >= 1
 
 
+def test_split_selftest_refuses_unsupported_k():
+    """The split-precision self-test has kernels for K in {16, 32, 64, 128, 256} only: any other K is refused before a launch,
+    never run as a 256-deep GEMM over whatever memory follows the operands."""
+    L = _lib.lib()
+    for K in (48, 80, 240, 512):
+        assert L.kpf_umma_split_selftest(None, None, None, 128, K, 0, 0, 0, None, None) == -1   # KPF_ERR_BAD_ARGUMENT
+
+
 def test_no_fallback_on_cpu_tensors():
     import torch
     from keypointfusion_b200 import ops
