@@ -187,6 +187,23 @@ def full_model(dev, world, rank, steps, warmup, total_batch=512, barrier=None):
             "backbones_ms": ms_bb, "path_ms_by_difference": ms / steps - ms_bb}
 
 
+def demo_frames(rs, F, hands=1):
+    """F synthetic 640x480 frames with `hands` hands each, drawn from RandomState rs -> (rgb [F,480,640,3] uint8 (random BGR),
+    depth [F,480,640] uint16 (900 mm background), bbox [F*hands,4] f64 (x,y,w,h); box f*hands+h is hand h of frame f).
+    A "hand" is a disc 120-170 px wide at 450-650 mm with +-20 mm relief, inside its bounding box (discs of one frame may overlap)."""
+    depth = np.full((F, 480, 640), 900, np.uint16)
+    yy, xx = np.mgrid[0:480, 0:640]
+    bbox = np.zeros((F * hands, 4), np.float64)
+    for f in range(F):
+        for h in range(hands):
+            cx, cy, r = rs.uniform(200, 440), rs.uniform(150, 330), rs.uniform(60, 85)
+            disc = (xx - cx) ** 2 + (yy - cy) ** 2 <= r * r
+            depth[f][disc] = (rs.uniform(450, 650) + 20 * np.sin(xx[disc] / 9.0) * np.cos(yy[disc] / 7.0)).astype(np.uint16)
+            bbox[f * hands + h] = (cx - r - 10, cy - r - 10, 2 * r + 20, 2 * r + 20)
+    rgb = rs.randint(0, 256, (F, 480, 640, 3)).astype(np.uint8)
+    return rgb, depth, bbox
+
+
 def demo(dev, world, rank, steps, warmup, total_batch=128, barrier=None):
     """config 5: 640x480 frames (uint16 depth + uint8 BGR) -> crop (K0) -> back-projection (K1) -> backbones -> fusion path."""
     from keypointfusion_b200.demo_RGBD import Model_RGBD
@@ -196,15 +213,7 @@ def demo(dev, world, rank, steps, warmup, total_batch=128, barrier=None):
     rs = np.random.RandomState(40 + rank)
     frames = []
     for s in range(3):
-        depth = np.full((B, 480, 640), 900, np.uint16)
-        yy, xx = np.mgrid[0:480, 0:640]
-        bbox = np.zeros((B, 4), np.float64)
-        for b in range(B):   # a "hand": a disc 120-170 px wide at 450-650 mm with +-20 mm relief, inside its bounding box
-            cx, cy, r = rs.uniform(200, 440), rs.uniform(150, 330), rs.uniform(60, 85)
-            disc = (xx - cx) ** 2 + (yy - cy) ** 2 <= r * r
-            depth[b][disc] = (rs.uniform(450, 650) + 20 * np.sin(xx[disc] / 9.0) * np.cos(yy[disc] / 7.0)).astype(np.uint16)
-            bbox[b] = (cx - r - 10, cy - r - 10, 2 * r + 20, 2 * r + 20)
-        rgb = rs.randint(0, 256, (B, 480, 640, 3)).astype(np.uint8)
+        rgb, depth, bbox = demo_frames(rs, B)
         frames.append((torch.from_numpy(rgb).pin_memory(), torch.from_numpy(depth.view(np.int16)).pin_memory(), torch.from_numpy(bbox).pin_memory()))
     dev_frames = [tuple(t.to(dev) for t in f) for f in frames]
 

@@ -266,17 +266,28 @@ int kpf_spatial_aggregate_tc(const void* feat_rgb, const void* feat_rgb_lo, cons
 int kpf_split_planes(const float* x, long long n, void* hi, void* lo, cudaStream_t stream);
 
 /* ---- 8f-3 crop + normalise front end for in-the-wild frames (demo_RGBD.py:253-276, :378-385, :410-569) ------------------
- * depth_u16 [B,Hf,Wf] uint16 (mm), rgb_u8 [B,Hf,Wf,3] uint8 (BGR as cv2 reads it); bbox [B,4] f64 (x,y,w,h);
+ * depth_u16 [F,Hf,Wf] uint16 (mm), rgb_u8 [F,Hf,Wf,3] uint8 (BGR as cv2 reads it); bbox [B,4] f64 (x,y,w,h), one box per hand;
  * center [B,3] f64 (u,v,d_mm); cube [B,3] f32 (mm); cam [B,4] f64 (fx,fy,fu,fv) -- f64 because the reference computes its
  * integer crop bounds from Python floats.  Integer work is bit-exact vs the reference (cv2 INTER_NEAREST rule included).
+ * frame_index [B] i32: box b reads frame frame_index[b], so a frame with several hands is uploaded and stored once;
+ *   NULL: box b reads frame b (requires F == B).  An index outside [0,F) is never dereferenced: every output of that box
+ *   (center_out, img_out, M_out, com3d_out, the rgb crop) is NaN; the other boxes are unaffected.
  * kpf_center_from_bbox -> center_out [B,3] f64;  kpf_crop_depth -> img_out [B,1,dsize,dsize] f32 (normalised, background 1),
  * M_out [B,3,3] f32 (frame px -> crop px), com3d_out [B,3] f32;  kpf_crop_rgb -> out [B,3,dsize,dsize] f32 in [0,1]. */
-int kpf_center_from_bbox(const void* depth_u16, const double* bbox, int B, int Hf, int Wf, int upper, int lower, double* center_out,
-                         cudaStream_t stream);
-int kpf_crop_depth(const void* depth_u16, const double* center, const float* cube, const double* cam, int B, int Hf, int Wf, int dsize,
-                   float* img_out, float* M_out, float* com3d_out, cudaStream_t stream);
-int kpf_crop_rgb(const void* rgb_u8, const double* center, const float* cube, const double* cam, int B, int Hf, int Wf, int dsize,
-                 float* out, cudaStream_t stream);
+int kpf_center_from_bbox(const void* depth_u16, const double* bbox, const int32_t* frame_index, int F, int B, int Hf, int Wf, int upper,
+                         int lower, double* center_out, cudaStream_t stream);
+int kpf_crop_depth(const void* depth_u16, const double* center, const float* cube, const double* cam, const int32_t* frame_index, int F,
+                   int B, int Hf, int Wf, int dsize, float* img_out, float* M_out, float* com3d_out, cudaStream_t stream);
+int kpf_crop_rgb(const void* rgb_u8, const double* center, const float* cube, const double* cam, const int32_t* frame_index, int F, int B,
+                 int Hf, int Wf, int dsize, float* out, cudaStream_t stream);
+
+/* ---- a5 (frame half)  dataloader/loader.py:821-834 xyz_nl2uvdnl_tensor up to points3DToImg (:277-288) -----------------------
+ * joints [B,P,3] f32 normalised xyz, center [B,3] f32 (mm, the com3d of the crop), cube [B,3] f32, cam [B,4] f32 ->
+ * xyz_cam_out [B,P,3] f32 = joints * cube / 2 + center (camera space, mm);
+ * uvd_frame_out [B,P,3] f32 = (X*fx/(Z+1e-8) + fu, flip*Y*fy/Z + fv, Z): frame pixels and depth in mm.
+ * Same fp32 operations in the same order as kpf_xyz2uvd (one shared device function), which goes on through M into the crop. */
+int kpf_joints_to_frame(const float* joints, const float* center, const float* cube, const float* cam, int B, int P, float flip,
+                        float* uvd_frame_out, float* xyz_cam_out, cudaStream_t stream);
 
 /* ---- 8f-4 evaluation tail (train.py:330-386, :470-488; util/generateFeature.py:681-703) -----------------------------------
  * pred, gt [B,J,3] f32 normalised xyz, cube [B,3] -> err [B,J] f32 (mm) and, if pa_err != NULL, pa_err [B,J] f32: the error

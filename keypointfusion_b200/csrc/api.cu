@@ -1,4 +1,4 @@
 // Library-level entry points of libkpf_b200.so.
 #include "common.cuh"
 
-extern "C" int kpf_abi_version(void) { return 3; }
+extern "C" int kpf_abi_version(void) { return 4; }

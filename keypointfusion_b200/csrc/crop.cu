@@ -1,7 +1,8 @@
 // SURVEY 8f-3: crop + normalise front end for in-the-wild RGB-D frames (BASELINE config 5), demo_RGBD.py:
 //   get_center_from_bbx :253-276, comToBounds :519-529, getCrop :531-569, Crop_Image_deep_pp :410-462,
 //   Crop_Image_deep_pp_RGB :464-517, normalize_img :378-385, jointImgTo3D :387-.
-// One CTA per frame.  All integer work (bounds, cv2 INTER_NEAREST source indices, paste offsets, uint16 z-threshold casts)
+// One CTA per box; box b reads frame frame_index[b] (frame b when frame_index is NULL), so several hands of one frame share
+// one upload.  An index outside [0,F) is never dereferenced: that box's outputs are NaN.  All integer work (bounds, cv2 INTER_NEAREST source indices, paste offsets, uint16 z-threshold casts)
 // is reproduced bit-exactly in fp64 / integer arithmetic; the frame is read once (only the pixels the crop samples).
 // HBM-bound and tiny: a 128 x 128 crop touches <= 16384 source pixels of the uint16 frame.
 #include "common.cuh"
@@ -12,6 +13,11 @@ struct CropGeom {
     int xs, xe, ys, ye, szw, szh, px, py;
     double zs, ze, sc, ifx, ify;
 };
+
+__device__ __forceinline__ int box_frame(const int32_t* frame_index, int b, int F) {
+    const int f = frame_index ? frame_index[b] : b;
+    return (f >= 0 && f < F) ? f : -1;
+}
 
 // comToBounds + resize size + paste offset (fp64, reference operation order)
 __device__ __forceinline__ void crop_geometry(const double* com, const float* size, const double* cam, int dsize, CropGeom& g) {
@@ -39,16 +45,21 @@ __device__ __forceinline__ void crop_geometry(const double* com, const float* si
 }
 
 __global__ void __launch_bounds__(256)
-center_from_bbox_kernel(const uint16_t* __restrict__ depth, const double* __restrict__ bbox, int Hf, int Wf, int upper, int lower,
-                        double* __restrict__ center) {
+center_from_bbox_kernel(const uint16_t* __restrict__ depth, const double* __restrict__ bbox, const int32_t* __restrict__ frame_index,
+                        int F, int Hf, int Wf, int upper, int lower, double* __restrict__ center) {
     __shared__ unsigned long long sh[4][8];
     const int b = blockIdx.x, tid = threadIdx.x;
+    const int fr = box_frame(frame_index, b, F);
+    if (fr < 0) {   // uniform over the CTA
+        if (tid < 3) center[3 * b + tid] = __longlong_as_double(0x7ff8000000000000ll);
+        return;
+    }
     const double* bb = bbox + 4 * b;
     const int x0 = (int)bb[0], x1 = (int)(bb[0] + bb[2]), y0 = (int)bb[1], y1 = (int)(bb[1] + bb[3]);
     const int cx0 = max(x0, 0), cx1 = min(x1, Wf), cy0 = max(y0, 0), cy1 = min(y1, Hf);   // numpy slicing clips at the frame
     const int w = max(cx1 - cx0, 0), h = max(cy1 - cy0, 0);
     unsigned long long sc = 0, sr = 0, sd = 0, cnt = 0;
-    const uint16_t* f = depth + (size_t)b * Hf * Wf;
+    const uint16_t* f = depth + (size_t)fr * Hf * Wf;
     for (int i = tid; i < w * h; i += blockDim.x) {
         const int r = i / w, c = i - r * w;
         const int v = f[(size_t)(cy0 + r) * Wf + cx0 + c];
@@ -88,12 +99,20 @@ center_from_bbox_kernel(const uint16_t* __restrict__ depth, const double* __rest
 
 __global__ void __launch_bounds__(256)
 crop_depth_kernel(const uint16_t* __restrict__ depth, const double* __restrict__ center, const float* __restrict__ cube,
-                  const double* __restrict__ cam, int Hf, int Wf, int dsize, float* __restrict__ img_out, float* __restrict__ M_out,
-                  float* __restrict__ com3d_out) {
+                  const double* __restrict__ cam, const int32_t* __restrict__ frame_index, int F, int Hf, int Wf, int dsize,
+                  float* __restrict__ img_out, float* __restrict__ M_out, float* __restrict__ com3d_out) {
     extern __shared__ float crop[];   // [dsize*dsize]
     __shared__ CropGeom g;
     __shared__ float red[8];
     const int b = blockIdx.x, tid = threadIdx.x;
+    const int fr = box_frame(frame_index, b, F);
+    if (fr < 0) {   // uniform over the CTA
+        const float nan = __int_as_float(0x7fc00000);
+        if (tid < 9) M_out[9 * b + tid] = nan;
+        if (tid < 3) com3d_out[3 * b + tid] = nan;
+        for (int i = tid; i < dsize * dsize; i += blockDim.x) img_out[(size_t)b * dsize * dsize + i] = nan;
+        return;
+    }
     const double* com = center + 3 * b;
     if (tid == 0) {
         crop_geometry(com, cube + 3 * b, cam + 4 * b, dsize, g);
@@ -108,7 +127,7 @@ crop_depth_kernel(const uint16_t* __restrict__ depth, const double* __restrict__
         com3d_out[3 * b + 2] = (float)com[2];
     }
     __syncthreads();
-    const uint16_t* f = depth + (size_t)b * Hf * Wf;
+    const uint16_t* f = depth + (size_t)fr * Hf * Wf;
     const int wb = g.xe - g.xs, hb = g.ye - g.ys;
     const uint16_t zs_cast = (uint16_t)g.zs;   // cropped[msk1] = zstart on a uint16 array
     float mx = 0.f;
@@ -154,12 +173,19 @@ crop_depth_kernel(const uint16_t* __restrict__ depth, const double* __restrict__
 
 __global__ void __launch_bounds__(256)
 crop_rgb_kernel(const uint8_t* __restrict__ rgb, const double* __restrict__ center, const float* __restrict__ cube,
-                const double* __restrict__ cam, int Hf, int Wf, int dsize, float* __restrict__ out) {
+                const double* __restrict__ cam, const int32_t* __restrict__ frame_index, int F, int Hf, int Wf, int dsize,
+                float* __restrict__ out) {
     __shared__ CropGeom g;
     const int b = blockIdx.x, tid = threadIdx.x;
+    const int fr = box_frame(frame_index, b, F);
+    if (fr < 0) {   // uniform over the CTA
+        const float nan = __int_as_float(0x7fc00000);
+        for (int i = tid; i < 3 * dsize * dsize; i += blockDim.x) out[(size_t)b * 3 * dsize * dsize + i] = nan;
+        return;
+    }
     if (tid == 0) crop_geometry(center + 3 * b, cube + 3 * b, cam + 4 * b, dsize, g);
     __syncthreads();
-    const uint8_t* f = rgb + (size_t)b * Hf * Wf * 3;
+    const uint8_t* f = rgb + (size_t)fr * Hf * Wf * 3;
     const int wb = g.xe - g.xs, hb = g.ye - g.ys;
     for (int i = tid; i < dsize * dsize; i += blockDim.x) {
         const int oy = i / dsize, ox = i - oy * dsize;
@@ -186,35 +212,36 @@ crop_rgb_kernel(const uint8_t* __restrict__ rgb, const double* __restrict__ cent
 
 }  // namespace kpf
 
-extern "C" int kpf_center_from_bbox(const void* depth_u16, const double* bbox, int B, int Hf, int Wf, int upper, int lower,
-                                    double* center_out, cudaStream_t stream) {
+extern "C" int kpf_center_from_bbox(const void* depth_u16, const double* bbox, const int32_t* frame_index, int F, int B, int Hf, int Wf,
+                                    int upper, int lower, double* center_out, cudaStream_t stream) {
     using namespace kpf;
-    KPF_REQUIRE(B >= 0 && Hf >= 1 && Wf >= 1);
+    KPF_REQUIRE(B >= 0 && F >= 0 && Hf >= 1 && Wf >= 1 && (frame_index != nullptr || F == B));
     if (B == 0) return 0;
-    center_from_bbox_kernel<<<B, 256, 0, stream>>>((const uint16_t*)depth_u16, bbox, Hf, Wf, upper, lower, center_out);
+    center_from_bbox_kernel<<<B, 256, 0, stream>>>((const uint16_t*)depth_u16, bbox, frame_index, F, Hf, Wf, upper, lower, center_out);
     KPF_CHECK_LAUNCH();
     return 0;
 }
 
-extern "C" int kpf_crop_depth(const void* depth_u16, const double* center, const float* cube, const double* cam, int B, int Hf, int Wf,
-                              int dsize, float* img_out, float* M_out, float* com3d_out, cudaStream_t stream) {
+extern "C" int kpf_crop_depth(const void* depth_u16, const double* center, const float* cube, const double* cam, const int32_t* frame_index,
+                              int F, int B, int Hf, int Wf, int dsize, float* img_out, float* M_out, float* com3d_out, cudaStream_t stream) {
     using namespace kpf;
-    KPF_REQUIRE(B >= 0 && Hf >= 1 && Wf >= 1 && dsize >= 8 && dsize <= 224);
+    KPF_REQUIRE(B >= 0 && F >= 0 && Hf >= 1 && Wf >= 1 && dsize >= 8 && dsize <= 224 && (frame_index != nullptr || F == B));
     if (B == 0) return 0;
     const size_t smem = (size_t)dsize * dsize * sizeof(float);
     cudaError_t e = kpf::set_smem(crop_depth_kernel, smem);
     if (e != cudaSuccess) return (int)e;
-    crop_depth_kernel<<<B, 256, smem, stream>>>((const uint16_t*)depth_u16, center, cube, cam, Hf, Wf, dsize, img_out, M_out, com3d_out);
+    crop_depth_kernel<<<B, 256, smem, stream>>>((const uint16_t*)depth_u16, center, cube, cam, frame_index, F, Hf, Wf, dsize, img_out,
+                                                  M_out, com3d_out);
     KPF_CHECK_LAUNCH();
     return 0;
 }
 
-extern "C" int kpf_crop_rgb(const void* rgb_u8, const double* center, const float* cube, const double* cam, int B, int Hf, int Wf,
-                            int dsize, float* out, cudaStream_t stream) {
+extern "C" int kpf_crop_rgb(const void* rgb_u8, const double* center, const float* cube, const double* cam, const int32_t* frame_index, int F,
+                            int B, int Hf, int Wf, int dsize, float* out, cudaStream_t stream) {
     using namespace kpf;
-    KPF_REQUIRE(B >= 0 && Hf >= 1 && Wf >= 1 && dsize >= 8);
+    KPF_REQUIRE(B >= 0 && F >= 0 && Hf >= 1 && Wf >= 1 && dsize >= 8 && (frame_index != nullptr || F == B));
     if (B == 0) return 0;
-    crop_rgb_kernel<<<B, 256, 0, stream>>>((const uint8_t*)rgb_u8, center, cube, cam, Hf, Wf, dsize, out);
+    crop_rgb_kernel<<<B, 256, 0, stream>>>((const uint8_t*)rgb_u8, center, cube, cam, frame_index, F, Hf, Wf, dsize, out);
     KPF_CHECK_LAUNCH();
     return 0;
 }

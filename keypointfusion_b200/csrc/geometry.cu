@@ -26,6 +26,23 @@ __global__ void uvd2xyz_kernel(const float* __restrict__ uvd, const float* __res
     }
 }
 
+// The points3DToImg half of xyz_nl2uvdnl_tensor: normalised xyz s -> camera-space point (X, Y, Z) in mm (loader.py:828) and its
+// frame pixel (pu, pv) (loader.py:277-288).  Shared by xyz2uvd_kernel (which goes on into the crop) and joints_to_frame_kernel.
+struct FramePoint {
+    float X, Y, Z, pu, pv;
+};
+
+__device__ __forceinline__ FramePoint xyznl_to_frame(const float* s, float cx, float cy, float cz, float sx, float sy, float sz, float fx,
+                                                     float fy, float fu, float fv, float flip) {
+    FramePoint q;
+    q.X = xadd(xdiv(xmul(s[0], sx), 2.0f), cx);  // loader.py:828
+    q.Y = xadd(xdiv(xmul(s[1], sy), 2.0f), cy);
+    q.Z = xadd(xdiv(xmul(s[2], sz), 2.0f), cz);
+    q.pu = xadd(xdiv(xmul(q.X, fx), xadd(q.Z, 1e-8f)), fu);  // loader.py:281-283
+    q.pv = xadd(xdiv(xmul(xmul(flip, q.Y), fy), q.Z), fv);   // loader.py:284-286
+    return q;
+}
+
 __global__ void xyz2uvd_kernel(const float* __restrict__ xyz, const float* __restrict__ center, const float* __restrict__ M,
                                const float* __restrict__ cube, const float* __restrict__ cam, int P, float img_size, float flip,
                                float* __restrict__ out) {
@@ -35,19 +52,34 @@ __global__ void xyz2uvd_kernel(const float* __restrict__ xyz, const float* __res
     const float sx = cube[3 * b], sy = cube[3 * b + 1], sz = cube[3 * b + 2];
     const float fx = cam[4 * b], fy = cam[4 * b + 1], fu = cam[4 * b + 2], fv = cam[4 * b + 3];
     for (int p = blockIdx.x * blockDim.x + threadIdx.x; p < P; p += gridDim.x * blockDim.x) {
-        const float* s = xyz + ((size_t)b * P + p) * 3;
-        const float X = xadd(xdiv(xmul(s[0], sx), 2.0f), cx);  // loader.py:828
-        const float Y = xadd(xdiv(xmul(s[1], sy), 2.0f), cy);
-        const float Z = xadd(xdiv(xmul(s[2], sz), 2.0f), cz);
-        const float pu = xadd(xdiv(xmul(X, fx), xadd(Z, 1e-8f)), fu);  // loader.py:281-283
-        const float pv = xadd(xdiv(xmul(xmul(flip, Y), fy), Z), fv);   // loader.py:284-286
-        const float tu = xadd(xadd(xmul(m[0], pu), xmul(m[1], pv)), m[2]);
-        const float tv = xadd(xadd(xmul(m[3], pu), xmul(m[4], pv)), m[5]);
+        const FramePoint q = xyznl_to_frame(xyz + ((size_t)b * P + p) * 3, cx, cy, cz, sx, sy, sz, fx, fy, fu, fv, flip);
+        const float tu = xadd(xadd(xmul(m[0], q.pu), xmul(m[1], q.pv)), m[2]);
+        const float tv = xadd(xadd(xmul(m[3], q.pu), xmul(m[4], q.pv)), m[5]);
         float* d = out + ((size_t)b * P + p) * 3;
         d[0] = xsub(xmul(xdiv(tu, img_size), 2.0f), 1.0f);  // loader.py:831
         d[1] = xsub(xmul(xdiv(tv, img_size), 2.0f), 1.0f);
-        d[2] = xdiv(xsub(Z, cz), xdiv(sz, 2.0f));           // loader.py:832
+        d[2] = xdiv(xsub(q.Z, cz), xdiv(sz, 2.0f));         // loader.py:832
     }
+}
+
+// Joints back into the frame they were cropped from: uvd_frame (frame pixels u, v and depth in mm) and xyz_cam (camera mm).
+// One thread per joint over the flat [B*P] range (P is a hand's 21 joints: a per-sample grid row would idle most of its threads).
+__global__ void joints_to_frame_kernel(const float* __restrict__ joints, const float* __restrict__ center, const float* __restrict__ cube,
+                                       const float* __restrict__ cam, int B, int P, float flip, float* __restrict__ uvd_frame,
+                                       float* __restrict__ xyz_cam) {
+    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= (long long)B * P) return;
+    const int b = (int)(i / P);
+    const FramePoint q = xyznl_to_frame(joints + i * 3, center[3 * b], center[3 * b + 1], center[3 * b + 2], cube[3 * b], cube[3 * b + 1],
+                                        cube[3 * b + 2], cam[4 * b], cam[4 * b + 1], cam[4 * b + 2], cam[4 * b + 3], flip);
+    float* u = uvd_frame + i * 3;
+    u[0] = q.pu;
+    u[1] = q.pv;
+    u[2] = q.Z;
+    float* x = xyz_cam + i * 3;
+    x[0] = q.X;
+    x[1] = q.Y;
+    x[2] = q.Z;
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -604,6 +636,16 @@ extern "C" int kpf_xyz2uvd(const float* xyz, const float* center, const float* M
     if (B == 0 || P == 0) return 0;
     dim3 grid((P + 255) / 256 > 64 ? 64 : (P + 255) / 256, B);
     xyz2uvd_kernel<<<grid, 256, 0, stream>>>(xyz, center, M, cube, cam, P, img_size, flip, out);
+    KPF_CHECK_LAUNCH();
+    return 0;
+}
+
+extern "C" int kpf_joints_to_frame(const float* joints, const float* center, const float* cube, const float* cam, int B, int P, float flip,
+                                   float* uvd_frame_out, float* xyz_cam_out, cudaStream_t stream) {
+    KPF_REQUIRE(B >= 0 && P >= 0);
+    const long long n = (long long)B * P;
+    if (n == 0) return 0;
+    joints_to_frame_kernel<<<(unsigned)((n + 255) / 256), 256, 0, stream>>>(joints, center, cube, cam, B, P, flip, uvd_frame_out, xyz_cam_out);
     KPF_CHECK_LAUNCH();
     return 0;
 }

@@ -385,6 +385,53 @@ def _(pred, gt, cube):
     return pred.new_empty(B, J, dtype=torch.float32), pred.new_empty(B, J, dtype=torch.float32)
 
 
+# ------------------------------------------------------------------------------------------------ 8f-3 frame front end
+# frame_index: None (box b reads frame b) or a [B] int32 tensor on the device (out-of-range boxes give NaN, include/kpf_b200.h)
+@_op("center_from_bbox")
+def center_from_bbox(depth: Tensor, bbox: Tensor, upper: int, lower: int, frame_index: Optional[Tensor] = None) -> Tensor:
+    return ops.center_from_bbox(depth, bbox, upper, lower, frame_index=frame_index)
+
+
+@center_from_bbox.register_fake
+def _(depth, bbox, upper, lower, frame_index=None):
+    return depth.new_empty(bbox.shape[0], 3, dtype=torch.float64)
+
+
+@_op("crop_depth")
+def crop_depth(depth: Tensor, center: Tensor, cube: Tensor, cam: Tensor, dsize: int, frame_index: Optional[Tensor] = None) -> Tuple[Tensor, Tensor, Tensor]:
+    """-> (img [B,1,dsize,dsize], M [B,3,3], com3d [B,3]) for center [B,3], cube [B,3] f32, cam [B,4] or [4] f64."""
+    img, M, com3d, _ = ops.crop_depth(depth, center, cube, cam, dsize, frame_index=frame_index)
+    return img, M, com3d
+
+
+@crop_depth.register_fake
+def _(depth, center, cube, cam, dsize, frame_index=None):
+    B = center.shape[0]
+    f = lambda *shape: depth.new_empty(shape, dtype=torch.float32)
+    return f(B, 1, dsize, dsize), f(B, 3, 3), f(B, 3)
+
+
+@_op("crop_rgb")
+def crop_rgb(rgb: Tensor, center: Tensor, cube: Tensor, cam: Tensor, dsize: int, frame_index: Optional[Tensor] = None) -> Tensor:
+    return ops.crop_rgb(rgb, center, cube, cam, dsize, frame_index=frame_index)
+
+
+@crop_rgb.register_fake
+def _(rgb, center, cube, cam, dsize, frame_index=None):
+    return rgb.new_empty(center.shape[0], 3, dsize, dsize, dtype=torch.float32)
+
+
+@_op("joints_to_frame")
+def joints_to_frame(joints: Tensor, center: Tensor, cube: Tensor, cam: Tensor, flip: float) -> Tuple[Tensor, Tensor]:
+    """-> (uvd_frame [B,P,3]: frame pixels and depth mm, xyz_cam [B,P,3]: camera-space mm)."""
+    return ops.joints_to_frame(joints, center, cube, cam, flip)
+
+
+@joints_to_frame.register_fake
+def _(joints, center, cube, cam, flip):
+    return joints.new_empty(joints.shape, dtype=torch.float32), joints.new_empty(joints.shape, dtype=torch.float32)
+
+
 def run_token_program(pk, x=None, y=None, r3d=None, desa=None, jf=None, want_tokens=True, exchange=None):
     """TokenProgram (plain Python holder of three tensors + ints) -> the custom op.  Returns (tokens | None, pred | None).
     exchange: a runtime.PeerExchange (the fused exchange step) or None."""

@@ -927,36 +927,84 @@ def _f64(t, device):
     return t.to(device=device, dtype=torch.float64).contiguous()
 
 
-def center_from_bbox(depth_u16, bbox, upper=1500, lower=171):
+def frame_index_arg(frame_index, B, F, device):
+    """frame_index of the front-end ops -> None or a [B] int32 tensor on `device`.
+    None: box b reads frame b, which needs F == B.  Indices given on the host (list, numpy array, CPU tensor) are checked
+    against [0, F) here, before any launch (ValueError).  A CUDA int32 tensor is passed through unchecked, so the calls can be
+    captured in a CUDA graph; a box whose device index is out of range gets NaN outputs and reads no frame."""
+    if frame_index is None:
+        if F != B:
+            raise ValueError(f"frame_index=None reads frame b for box b, but there are {F} frames and {B} boxes")
+        return None
+    if torch.is_tensor(frame_index) and frame_index.is_cuda:
+        if frame_index.dtype != torch.int32 or tuple(frame_index.shape) != (B,):
+            raise ValueError(f"a device frame_index must be an int32 tensor of shape ({B},), got {frame_index.dtype} {tuple(frame_index.shape)}")
+        return frame_index.contiguous()
+    fi = torch.as_tensor(frame_index)
+    if fi.dtype.is_floating_point or fi.dtype.is_complex or fi.dtype == torch.bool:
+        raise ValueError(f"frame_index must hold integers, got {fi.dtype}")
+    fi = fi.reshape(-1)
+    if fi.numel() != B:
+        raise ValueError(f"frame_index has {fi.numel()} entries for {B} boxes")
+    bad = (fi < 0) | (fi >= F)
+    if bool(bad.any()):
+        raise ValueError(f"frame_index {fi[bad].tolist()} outside [0, {F}) (F = number of frames)")
+    return fi.to(device=device, dtype=torch.int32)
+
+
+def center_from_bbox(depth_u16, bbox, upper=1500, lower=171, frame_index=None):
+    """depth [F,Hf,Wf] uint16, bbox [B,4] (x,y,w,h) -> centre [B,3] f64 (u, v, d_mm); box b reads frame frame_index[b]."""
+    F, Hf, Wf = depth_u16.shape
+    B = torch.as_tensor(bbox).numel() // 4
+    fi = frame_index_arg(frame_index, B, F, depth_u16.device)
     d = _u16(depth_u16)
-    B, Hf, Wf = d.shape
     bbox = _f64(bbox, d.device).reshape(B, 4)
     out = torch.empty(B, 3, device=d.device, dtype=torch.float64)
-    _call("kpf_center_from_bbox", _p(d), _p(bbox), B, Hf, Wf, int(upper), int(lower), _p(out))
+    _call("kpf_center_from_bbox", _p(d), _p(bbox), _p(fi), F, B, Hf, Wf, int(upper), int(lower), _p(out))
     return out
 
 
-def crop_depth(depth_u16, center, cube, cam, dsize=128):
+def crop_depth(depth_u16, center, cube, cam, dsize=128, frame_index=None):
+    """depth [F,Hf,Wf] uint16, center [B,3] -> (img [B,1,dsize,dsize], M [B,3,3], com3d [B,3], cube [B,3]); box b reads frame
+    frame_index[b]."""
+    F, Hf, Wf = depth_u16.shape
+    B = torch.as_tensor(center).numel() // 3
+    fi = frame_index_arg(frame_index, B, F, depth_u16.device)
     d = _u16(depth_u16)
-    B, Hf, Wf = d.shape
     center, cam = _f64(center, d.device).reshape(B, 3), _f64(cam, d.device).reshape(-1, 4).expand(B, 4).contiguous()
     cube = torch.as_tensor(cube, dtype=torch.float32).to(d.device).reshape(-1, 3).expand(B, 3).contiguous()
     img = torch.empty(B, 1, dsize, dsize, device=d.device, dtype=torch.float32)
     M = torch.empty(B, 3, 3, device=d.device, dtype=torch.float32)
     com3d = torch.empty(B, 3, device=d.device, dtype=torch.float32)
-    _call("kpf_crop_depth", _p(d), _p(center), _p(cube), _p(cam), B, Hf, Wf, dsize, _p(img), _p(M), _p(com3d))
+    _call("kpf_crop_depth", _p(d), _p(center), _p(cube), _p(cam), _p(fi), F, B, Hf, Wf, dsize, _p(img), _p(M), _p(com3d))
     return img, M, com3d, cube
 
 
-def crop_rgb(rgb_u8, center, cube, cam, dsize=128):
+def crop_rgb(rgb_u8, center, cube, cam, dsize=128, frame_index=None):
+    """rgb [F,Hf,Wf,3] uint8, center [B,3] -> [B,3,dsize,dsize] f32 in [0,1]; box b reads frame frame_index[b]."""
+    F, Hf, Wf, _ = rgb_u8.shape
+    B = torch.as_tensor(center).numel() // 3
+    fi = frame_index_arg(frame_index, B, F, rgb_u8.device)
     _need_cuda(rgb_u8)
     r = rgb_u8.to(torch.uint8).contiguous()
-    B, Hf, Wf, _ = r.shape
     center, cam = _f64(center, r.device).reshape(B, 3), _f64(cam, r.device).reshape(-1, 4).expand(B, 4).contiguous()
     cube = torch.as_tensor(cube, dtype=torch.float32).to(r.device).reshape(-1, 3).expand(B, 3).contiguous()
     out = torch.empty(B, 3, dsize, dsize, device=r.device, dtype=torch.float32)
-    _call("kpf_crop_rgb", _p(r), _p(center), _p(cube), _p(cam), B, Hf, Wf, dsize, _p(out))
+    _call("kpf_crop_rgb", _p(r), _p(center), _p(cube), _p(cam), _p(fi), F, B, Hf, Wf, dsize, _p(out))
     return out
+
+
+def joints_to_frame(joints, center, cube, cam, flip=1.0):
+    """Normalised joints [B,P,3] of crops with com3d `center` [B,3] (mm), `cube` [B,3], `cam` [B,4] (fx,fy,fu,fv) ->
+    (uvd_frame [B,P,3]: frame pixels u, v and depth mm;  xyz_cam [B,P,3]: camera-space mm).  The points3DToImg half of
+    xyz_nl2uvdnl_tensor (loader.py:821-834, :277-288): the same fp32 operations as xyz2uvd before it applies M."""
+    joints, center, cube, cam = _f32(joints), _f32(center), _f32(cube), _f32(cam)
+    B, P, _ = joints.shape
+    uvd = torch.empty_like(joints)
+    xyz = torch.empty_like(joints)
+    _call("kpf_joints_to_frame", _p(joints), _p(center.reshape(B, 3)), _p(cube.reshape(B, 3)), _p(cam.reshape(B, 4)), B, P, float(flip),
+          _p(uvd), _p(xyz))
+    return uvd, xyz
 
 
 # ------------------------------------------------------------------------------------------------ 8f-4 evaluation tail

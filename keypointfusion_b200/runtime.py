@@ -11,6 +11,7 @@ class GraphedFusionPath:
     device, or pinned host to device) and replays.  Inputs: dict with img [B,1,S,S] f32, img_feat / img_feat_rgb [B,128,H,H],
     img_offset [B,5J,H,H] (bf16 or f32), center [B,3], M [B,3,3], cube [B,3], cam [B,4]."""
     KEYS = ("img", "img_feat", "img_feat_rgb", "img_offset", "center", "M", "cube", "cam")
+    FETCH = ("joints",)   # the outputs PipelinedRunner copies back to the host
 
     def __init__(self, net, loader, example, sample_num=1024, kernel=0.8, seed=0, warmup=2, chains=1, bind=False, exchange=None):
         """chains > 1: the batch is split into `chains` contiguous sub-batches whose (latency-bound, small-grid) kernel chains
@@ -82,6 +83,60 @@ class GraphedFusionPath:
             main.wait_stream(st)                  # join
         self._count = ops.launch_count() - n0
         return dict(joints=self.joints_all, chains=outs)
+
+    def __call__(self, inputs=None):
+        if inputs is not None:
+            for k in self.KEYS:
+                self.static[k].copy_(inputs[k], non_blocking=True)
+        self.graph.replay()
+        return self.out
+
+
+class GraphedFramePath:
+    """Frames to keypoints as one captured graph: the crop front end (demo_RGBD.Model_RGBD.prepare_batch), the two stock-PyTorch
+    backbones, KPFusion.forward_path and joints_to_frame, over static buffers rgb [F,Hf,Wf,3] uint8, depth [F,Hf,Wf] uint16 (or
+    int16 with the same bits), bbox [B,4] f64 and frame_index [B] int32 (box b is in frame frame_index[b]).  `out` holds joints
+    (normalised), joints_uvd_frame (frame pixels, depth mm), joints_xyz_cam (camera mm) and the full result list.
+
+    A step has a fixed (F, B) shape.  A caller with fewer hands in a step repeats a box (any valid frame / box pair) and ignores
+    the extra rows.  frame_index lives on the device, so it is not range-checked per step: an index outside [0,F) gives NaN
+    keypoints for that hand only (include/kpf_b200.h)."""
+    KEYS = ("rgb", "depth", "bbox", "frame_index")
+    FETCH = ("joints_uvd_frame", "joints_xyz_cam")
+
+    def __init__(self, net, loader, example, cam_para=(617.0, 617.0, 312.0, 241.0), cube=(250, 250, 250), img_size=128, sample_num=1024,
+                 seed=0, warmup=2, bind=False):
+        """net: KPFusion with backbones; loader: the geometry helper passed to the network (None: a loader(img_size)).
+        bind=True: capture over the caller's device tensors `example` (as GraphedFusionPath)."""
+        from .demo_RGBD import Model_RGBD
+        self.model = Model_RGBD(net, cam_para=cam_para, cube=cube, img_size=img_size, sample_num=sample_num, seed=seed)
+        if loader is not None:
+            self.model.depthloader = loader
+        dev = next(net.parameters()).device
+        if bind:
+            assert all(example[k].is_cuda and example[k].is_contiguous() for k in self.KEYS), "bind=True needs contiguous device tensors"
+            self.static = {k: example[k] for k in self.KEYS}
+        else:
+            self.static = {k: torch.empty_like(example[k], device=dev).copy_(example[k]) for k in self.KEYS}
+        assert self.static["frame_index"].dtype == torch.int32, "frame_index must be int32"
+        self.stream = torch.cuda.Stream(device=dev)
+        self.stream.wait_stream(torch.cuda.current_stream(dev))
+        with torch.cuda.stream(self.stream), torch.no_grad():
+            for _ in range(warmup):  # packed weight caches, device constants and backbone algorithm choices before capture
+                self._run()
+        torch.cuda.current_stream(dev).wait_stream(self.stream)
+        torch.cuda.synchronize(dev)
+        self.graph = torch.cuda.CUDAGraph()
+        with torch.no_grad(), torch.cuda.graph(self.graph, stream=self.stream):
+            self.out = self._run()
+        self.launches_per_replay = self._count
+
+    def _run(self):
+        n0 = ops.launch_count()
+        s = self.static
+        res, b = self.model.estimate_pose_RGBD(s["rgb"], s["depth"], s["bbox"], s["frame_index"])
+        self._count = ops.launch_count() - n0
+        return dict(joints=res[-1], joints_uvd_frame=b["joints_uvd_frame"], joints_xyz_cam=b["joints_xyz_cam"], result=res)
 
     def __call__(self, inputs=None):
         if inputs is not None:
@@ -216,32 +271,36 @@ class InputArena:
 class PipelinedRunner:
     """Host-fed serving loop: two captured graphs, each bound to its own device input arena; while graph[i % 2] computes step i
     on the compute stream, a copy stream uploads step i+1's pinned host inputs into the other arena, and the host reads step
-    i-1's joints from pinned memory.  Every step still does its own H2D of all inputs and its own D2H of the result.
+    i-1's results from pinned memory.  Every step still does its own H2D of all inputs and its own D2H of the result.
     `new_host_inputs()` hands the caller a dict of pinned views (one arena): filling those and passing the dict to `submit`
-    uploads a step with a single copy; any other dict of host tensors is uploaded tensor by tensor."""
+    uploads a step with a single copy; any other dict of host tensors is uploaded tensor by tensor.
 
-    def __init__(self, net, loader, example, **kw):
+    path_cls: GraphedFusionPath (crops + backbone maps in, normalised joints out) or GraphedFramePath (frames, boxes and
+    frame_index in, keypoints in frame pixels and camera mm out); `example` holds that class's KEYS and `kw` go to it."""
+
+    def __init__(self, net, loader, example, path_cls=GraphedFusionPath, **kw):
         dev = next(net.parameters()).device
         self.dev = dev
-        keys = GraphedFusionPath.KEYS
+        self.keys = keys = path_cls.KEYS
         self.arenas = [InputArena(example, keys, device=dev) for _ in range(2)]
         for a in self.arenas:
             for k in keys:
                 a.views[k].copy_(example[k])
-        self.paths = [GraphedFusionPath(net, loader, a.views, bind=True, **kw) for a in self.arenas]
+        self.paths = [path_cls(net, loader, a.views, bind=True, **kw) for a in self.arenas]
         self._example = {k: example[k] for k in keys}
         self.copy_stream = torch.cuda.Stream(device=dev)
         self.copied = [torch.cuda.Event() for _ in range(2)]
         self.done = [torch.cuda.Event() for _ in range(2)]
-        j = self.paths[0].out["joints"]
-        self.host_out = [torch.empty(j.shape, dtype=j.dtype).pin_memory() for _ in range(2)]
+        self.fetch_keys = path_cls.FETCH
+        outs = self.paths[0].out
+        self.host_out = [[torch.empty(outs[k].shape, dtype=outs[k].dtype).pin_memory() for k in self.fetch_keys] for _ in range(2)]
         self.step = 0
         for e in self.done:
             e.record(torch.cuda.current_stream(dev))
 
     def new_host_inputs(self):
         """A dict of pinned host tensors (views of one arena laid out like the device arenas) for the caller to fill."""
-        a = InputArena(self._example, GraphedFusionPath.KEYS, pinned=True)
+        a = InputArena(self._example, self.keys, pinned=True)
         d = dict(a.views)
         d["_arena"] = a.buf
         return d
@@ -262,12 +321,15 @@ class PipelinedRunner:
             self.copied[s].record(self.copy_stream)
         main.wait_event(self.copied[s])
         path.graph.replay()
-        self.host_out[s].copy_(path.out["joints"], non_blocking=True)
+        for h, k in zip(self.host_out[s], self.fetch_keys):
+            h.copy_(path.out[k], non_blocking=True)
         self.done[s].record(main)
         self.step += 1
         return s
 
     def fetch(self, slot):
-        """Block until the step submitted into `slot` is complete; returns its joints (pinned host tensor)."""
+        """Block until the step submitted into `slot` is complete; returns its result (pinned host memory): the joints for
+        GraphedFusionPath, the tuple (joints_uvd_frame, joints_xyz_cam) for GraphedFramePath."""
         self.done[slot].synchronize()
-        return self.host_out[slot]
+        h = self.host_out[slot]
+        return h[0] if len(h) == 1 else tuple(h)
