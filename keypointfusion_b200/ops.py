@@ -656,29 +656,12 @@ def exchange_wait(buf, xstep, samples_per_step, inflight, flush=False):
 _sm_count = {}
 
 
-_sm_budget = [None]   # CTAs a persistent kernel may take (None: every SM); runtime.GraphedFusionPath lowers it per concurrent chain
-
-
 def sm_count(device):
+    """Multiprocessors of `device` (cached): the persistent kernels' grid size, and one wave for K5's split."""
     i = torch.device(device).index or 0
     if i not in _sm_count:
         _sm_count[i] = torch.cuda.get_device_properties(i).multi_processor_count
-    n = _sm_count[i]
-    return n if _sm_budget[0] is None else max(1, min(n, _sm_budget[0]))
-
-
-class sm_budget:
-    """with ops.sm_budget(n): persistent kernels launched inside take at most n CTAs (SM partitioning between concurrent chains)."""
-
-    def __init__(self, n):
-        self.n = n
-
-    def __enter__(self):
-        self.prev = _sm_budget[0]
-        _sm_budget[0] = self.n
-
-    def __exit__(self, *a):
-        _sm_budget[0] = self.prev
+    return _sm_count[i]
 
 
 def repack_features(img_feat, img_feat_rgb, weight_map):

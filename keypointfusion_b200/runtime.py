@@ -6,23 +6,17 @@ import torch
 from . import ops
 
 
-class GraphedFusionPath:
-    """Capture `getpcl + KPFusion.forward_path` once; `__call__` copies a step's inputs into the static buffers (device to
-    device, or pinned host to device) and replays.  Inputs: dict with img [B,1,S,S] f32, img_feat / img_feat_rgb [B,128,H,H],
-    img_offset [B,5J,H,H] (bf16 or f32), center [B,3], M [B,3,3], cube [B,3], cam [B,4]."""
-    KEYS = ("img", "img_feat", "img_feat_rgb", "img_offset", "center", "M", "cube", "cam")
-    FETCH = ("joints",)   # the outputs PipelinedRunner copies back to the host
+class _GraphedPath:
+    """What the graphed paths share: the step's inputs (KEYS) in static device buffers, a warm-up of `_run` on a private stream,
+    one `_run` captured on that same stream into `graph` (its outputs in `out`, the kernels of ours it launches counted in
+    `launches_per_replay`), and `__call__`, which stages a step's inputs and replays."""
+    KEYS = ()
+    FETCH = ()   # the outputs PipelinedRunner copies back to the host
 
-    def __init__(self, net, loader, example, sample_num=1024, kernel=0.8, seed=0, warmup=2, chains=1, bind=False, exchange=None):
-        """chains > 1: the batch is split into `chains` contiguous sub-batches whose (latency-bound, small-grid) kernel chains
-        are captured on parallel streams inside the one graph, so they overlap on the 148 SMs; results are identical.
-        bind=True: capture directly over the caller's (device-resident) `example` tensors instead of private static buffers;
-        `__call__()` then replays with no staging copy and reads whatever those tensors hold at replay time."""
-        self.net, self.loader, self.sample_num, self.kernel, self.seed = net, loader, sample_num, kernel, seed
-        self.exchange = exchange    # a PeerExchange: the fused all-gather of the joints is part of the captured graph
-        self.chains = max(1, min(chains, example["img"].shape[0]))
+    def _warm_up(self, net, example, warmup, bind):
+        """bind=True: the static buffers are the caller's own (device-resident, contiguous) `example` tensors, so a replay reads
+        whatever they hold at that time; otherwise they are private copies of `example` on the network's device."""
         dev = next(net.parameters()).device
-        self.side = [torch.cuda.Stream(device=dev) for _ in range(self.chains - 1)]
         if bind:
             assert all(example[k].is_cuda and example[k].is_contiguous() for k in self.KEYS), "bind=True needs contiguous device tensors"
             self.static = {k: example[k] for k in self.KEYS}
@@ -31,58 +25,19 @@ class GraphedFusionPath:
         self.stream = torch.cuda.Stream(device=dev)
         self.stream.wait_stream(torch.cuda.current_stream(dev))
         with torch.cuda.stream(self.stream), torch.no_grad():
-            for _ in range(warmup):  # builds every lazily packed weight cache before capture
+            for _ in range(warmup):  # packed weight caches, device constants and backbone algorithm choices are built before capture
                 self._run()
         torch.cuda.current_stream(dev).wait_stream(self.stream)
         torch.cuda.synchronize(dev)
-        if exchange is not None:
-            with torch.cuda.stream(self.stream):
-                exchange.flush()    # complete the last warm-up step's gather
-            exchange.sync_ranks()   # every rank has finished the same number of (exchanging) warm-up steps before anyone captures
+
+    def _capture(self):
         self.graph = torch.cuda.CUDAGraph()
+        n0 = ops.launch_count()
         # captured on the warm-up stream: per-stream persistent workspaces (ops._zero_counters) already exist, so no fill node
         # lands inside the graph (it would also cut the programmatic-launch chain between two kernels)
         with torch.no_grad(), torch.cuda.graph(self.graph, stream=self.stream):
             self.out = self._run()
-        self.launches_per_replay = self._count
-
-    def _chain(self, s):
-        if self.exchange is not None:
-            self.exchange.begin_step()   # completes the PREVIOUS step's gather (normally already there) and opens this one
-        pcl, count = ops.getpcl(s["img"], s["center"], s["cube"], s["M"], s["cam"], self.sample_num, seed=self.seed)
-        res, sw, _ = self.net.forward_path(s["img_offset"], s["img_feat"], None, s["img_feat_rgb"], s["img"], pcl, self.loader, s["center"],
-                                           s["M"], s["cube"], s["cam"], self.kernel, exchange=self.exchange)
-        return res, sw, pcl
-
-    def _run(self):
-        n0 = ops.launch_count()
-        if self.chains == 1:
-            res, sw, pcl = self._chain(self.static)
-            self._count = ops.launch_count() - n0
-            return dict(joints=res[-1], result=res, spatial_weight=sw, pcl=pcl)
-        from .runtime import shard_batch
-        B = self.static["img"].shape[0]
-        main = torch.cuda.current_stream()
-        if not hasattr(self, "joints_all"):
-            J = self.net.joint_num
-            self.joints_all = torch.empty(B, J, 3, device=self.static["img"].device)
-        outs = []
-        for c in range(self.chains):
-            lo, hi = shard_batch(B, c, self.chains)
-            sub = {k: v[lo:hi] for k, v in self.static.items()}
-            st = main if c == 0 else self.side[c - 1]
-            if c > 0:
-                st.wait_stream(main)              # fork
-            # SM partitioning: each concurrent chain's persistent kernels take their share of the SMs, so that e.g. one chain's
-            # (one CTA per sample) token stack and another chain's point stage / DESA tiles are co-resident
-            with torch.cuda.stream(st), ops.sm_budget(max(1, ops.sm_count(self.static["img"].device) // self.chains)):
-                res, sw, pcl = self._chain(sub)
-                self.joints_all[lo:hi].copy_(res[-1])
-            outs.append((res, sw, pcl))
-        for st in self.side:
-            main.wait_stream(st)                  # join
-        self._count = ops.launch_count() - n0
-        return dict(joints=self.joints_all, chains=outs)
+        self.launches_per_replay = ops.launch_count() - n0
 
     def __call__(self, inputs=None):
         if inputs is not None:
@@ -92,7 +47,40 @@ class GraphedFusionPath:
         return self.out
 
 
-class GraphedFramePath:
+class GraphedFusionPath(_GraphedPath):
+    """Capture `getpcl + KPFusion.forward_path` once; `__call__` copies a step's inputs into the static buffers (device to
+    device, or pinned host to device) and replays.  Inputs: dict with img [B,1,S,S] f32, img_feat / img_feat_rgb [B,128,H,H],
+    img_offset [B,5J,H,H] (bf16 or f32), center [B,3], M [B,3,3], cube [B,3], cam [B,4].  `out` holds joints (the final joints),
+    result and spatial_weight (forward_path's lists) and pcl (the sampled point cloud)."""
+    KEYS = ("img", "img_feat", "img_feat_rgb", "img_offset", "center", "M", "cube", "cam")
+    FETCH = ("joints",)
+
+    def __init__(self, net, loader, example, sample_num=1024, kernel=0.8, seed=0, warmup=2, chains=1, bind=False, exchange=None):
+        """chains must be 1: a step is one chain of kernels on one stream.  Batches share the GPU by keeping several steps in
+        flight (OverlappedSteps).  bind=True: capture directly over the caller's (device-resident) `example` tensors instead of
+        private static buffers; `__call__()` then replays with no staging copy and reads whatever those tensors hold at replay time."""
+        if chains != 1:
+            raise ValueError(f"chains={chains}: a step is one kernel chain; keep several steps in flight with OverlappedSteps instead")
+        self.net, self.loader, self.sample_num, self.kernel, self.seed = net, loader, sample_num, kernel, seed
+        self.exchange = exchange    # a PeerExchange: the fused all-gather of the joints is part of the captured graph
+        self._warm_up(net, example, warmup, bind)
+        if exchange is not None:
+            with torch.cuda.stream(self.stream):
+                exchange.flush()    # complete the last warm-up step's gather
+            exchange.sync_ranks()   # every rank has finished the same number of (exchanging) warm-up steps before anyone captures
+        self._capture()
+
+    def _run(self):
+        s = self.static
+        if self.exchange is not None:
+            self.exchange.begin_step()   # completes the PREVIOUS step's gather (normally already there) and opens this one
+        pcl, _ = ops.getpcl(s["img"], s["center"], s["cube"], s["M"], s["cam"], self.sample_num, seed=self.seed)
+        res, sw, _ = self.net.forward_path(s["img_offset"], s["img_feat"], None, s["img_feat_rgb"], s["img"], pcl, self.loader, s["center"],
+                                           s["M"], s["cube"], s["cam"], self.kernel, exchange=self.exchange)
+        return dict(joints=res[-1], result=res, spatial_weight=sw, pcl=pcl)
+
+
+class GraphedFramePath(_GraphedPath):
     """Frames to keypoints as one captured graph: the crop front end (demo_RGBD.Model_RGBD.prepare_batch), the two stock-PyTorch
     backbones, KPFusion.forward_path and joints_to_frame, over static buffers rgb [F,Hf,Wf,3] uint8, depth [F,Hf,Wf] uint16 (or
     int16 with the same bits), bbox [B,4] f64 and frame_index [B] int32 (box b is in frame frame_index[b]).  `out` holds joints
@@ -109,41 +97,17 @@ class GraphedFramePath:
         """net: KPFusion with backbones; loader: the geometry helper passed to the network (None: a loader(img_size)).
         bind=True: capture over the caller's device tensors `example` (as GraphedFusionPath)."""
         from .demo_RGBD import Model_RGBD
+        assert example["frame_index"].dtype == torch.int32, "frame_index must be int32"
         self.model = Model_RGBD(net, cam_para=cam_para, cube=cube, img_size=img_size, sample_num=sample_num, seed=seed)
         if loader is not None:
             self.model.depthloader = loader
-        dev = next(net.parameters()).device
-        if bind:
-            assert all(example[k].is_cuda and example[k].is_contiguous() for k in self.KEYS), "bind=True needs contiguous device tensors"
-            self.static = {k: example[k] for k in self.KEYS}
-        else:
-            self.static = {k: torch.empty_like(example[k], device=dev).copy_(example[k]) for k in self.KEYS}
-        assert self.static["frame_index"].dtype == torch.int32, "frame_index must be int32"
-        self.stream = torch.cuda.Stream(device=dev)
-        self.stream.wait_stream(torch.cuda.current_stream(dev))
-        with torch.cuda.stream(self.stream), torch.no_grad():
-            for _ in range(warmup):  # packed weight caches, device constants and backbone algorithm choices before capture
-                self._run()
-        torch.cuda.current_stream(dev).wait_stream(self.stream)
-        torch.cuda.synchronize(dev)
-        self.graph = torch.cuda.CUDAGraph()
-        with torch.no_grad(), torch.cuda.graph(self.graph, stream=self.stream):
-            self.out = self._run()
-        self.launches_per_replay = self._count
+        self._warm_up(net, example, warmup, bind)
+        self._capture()
 
     def _run(self):
-        n0 = ops.launch_count()
         s = self.static
         res, b = self.model.estimate_pose_RGBD(s["rgb"], s["depth"], s["bbox"], s["frame_index"])
-        self._count = ops.launch_count() - n0
         return dict(joints=res[-1], joints_uvd_frame=b["joints_uvd_frame"], joints_xyz_cam=b["joints_xyz_cam"], result=res)
-
-    def __call__(self, inputs=None):
-        if inputs is not None:
-            for k in self.KEYS:
-                self.static[k].copy_(inputs[k], non_blocking=True)
-        self.graph.replay()
-        return self.out
 
 
 class OverlappedSteps:

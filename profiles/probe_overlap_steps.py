@@ -1,8 +1,7 @@
-"""Profiling aid: throughput when consecutive STEPS (independent batches of 64) are kept in flight on two streams, each step's
-persistent kernels limited to a share of the SMs.  Prints us per step for (streams, SM budget per step)."""
+"""Profiling aid: throughput when consecutive STEPS (independent batches of 64) are kept in flight on several streams.
+Prints us per step for 1, 2 and 3 streams."""
 import os, sys, torch
 sys.path.insert(0, os.getcwd())
-from keypointfusion_b200 import ops
 from keypointfusion_b200.dataloader.loader import loader
 from keypointfusion_b200.model.model import KPFusion
 from keypointfusion_b200.runtime import GraphedFusionPath
@@ -16,9 +15,8 @@ for s in range(4):
     for kk in ("img_feat", "img_feat_rgb", "img_offset"): d[kk] = d[kk].bfloat16()
     sets.append(d)
 L = loader(img_size=128)
-for nstream, budget in ((1, 148), (2, 148), (2, 112), (2, 96), (2, 74), (3, 74), (3, 56)):
-    with ops.sm_budget(budget):
-        graphs = [GraphedFusionPath(net, L, d, bind=True) for d in sets]
+graphs = [GraphedFusionPath(net, L, d, bind=True) for d in sets]
+for nstream in (1, 2, 3):
     streams = [torch.cuda.Stream() for _ in range(nstream)]
     def run(n):
         for i in range(n):
@@ -31,4 +29,4 @@ for nstream, budget in ((1, 148), (2, 148), (2, 112), (2, 96), (2, 74), (3, 74),
     run(40)
     for s in streams: torch.cuda.current_stream().wait_stream(s)
     e1.record(); torch.cuda.synchronize()
-    print(f"streams {nstream} budget {budget:3d}: {e0.elapsed_time(e1) * 1e3 / 40:7.1f} us per step", flush=True)
+    print(f"streams {nstream}: {e0.elapsed_time(e1) * 1e3 / 40:7.1f} us per step", flush=True)
