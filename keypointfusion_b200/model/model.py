@@ -297,16 +297,19 @@ class DESA(_KernelCache, nn.Module):
         k = self.kc()
         B, J, C = node_feat.shape
         N = pcl_feat.shape[1]
-        if k["scales"] is None or C != 128 or N % 64 or J > 32 or len(set(self.S)) != 1 or self.scale_num > 4:
-            raise NotImplementedError("DESA kernels: 128 channels, one nsample for all scales, N % 64 == 0, single-conv MLPs (no fallback path)")
+        # the fusion conv runs in the token-stack prologue, which reads exactly three scales
+        if k["scales"] is None or C != 128 or N % 64 or J > 32 or len(set(self.S)) != 1 or self.scale_num != 3:
+            raise NotImplementedError("DESA kernels: 128 channels, three scales sharing one nsample, N % 64 == 0, single-conv MLPs "
+                                      "(no fallback path)")
         dev = node_feat.device
         if "ds" not in k:
             eye, z = torch.eye(128, device=dev), torch.zeros(128, device=dev)
             k["ds"] = ops.pack_desa(eye, z, torch.zeros(128, 3, device=dev), z, k["scales"])
-            k["fu"] = ops.pack_token_program(J, fusion=k["fusion"]).to(dev)
+        if J not in k:  # the fusion program is packed for one token count
+            k[J] = ops.pack_token_program(J, fusion=k["fusion"]).to(dev)
         e = ops.e_from_float(pcl_feat.float())
         part, _ = ops.desa_fused(e, None, None, pcl_xyz, node_xyz, k["ds"][0], k["ds"][1], self.radius, self.S[0], jf_in=node_feat)
-        return cops.run_token_program(k["fu"], desa=part, jf=node_feat)[0]
+        return cops.run_token_program(k[J], desa=part, jf=node_feat)[0]
 
 
 # ----------------------------------------------------------------------------------------------------------------------

@@ -599,6 +599,15 @@ def ball_query(xyz, centers, radius, nsample, return_counts=False):
 
 def desa(p, prefix, pcl_feat, node_feat, pcl_xyz, node_xyz, radius=(0.1, 0.2, 0.4), nsample=(64, 64, 64)):
     """DESA.forward model.py:166-204 with the pointnet2_ops grouping restated."""
+    outs = desa_scales(p, prefix, pcl_feat, node_feat, pcl_xyz, node_xyz, radius, nsample)
+    outs.append(node_feat)
+    cat = torch.cat(outs, -1)
+    y = F.linear(cat, p[prefix + "fusion.0.weight"].squeeze(-1), p[prefix + "fusion.0.bias"])
+    return torch.relu(_bn2d(p, prefix + "fusion.1.", y))
+
+
+def desa_scales(p, prefix, pcl_feat, node_feat, pcl_xyz, node_xyz, radius=(0.1, 0.2, 0.4), nsample=(64, 64, 64)):
+    """DESA's grouping and per-scale MLP, before the fusion conv (model.py:166-200): one max-pooled [B,J,C] tensor per radius."""
     B, J, C = node_feat.shape
     xyz = torch.cat([pcl_xyz, node_xyz], 1)
     feat = torch.cat([pcl_feat, node_feat], 1)
@@ -619,10 +628,7 @@ def desa(p, prefix, pcl_feat, node_feat, pcl_xyz, node_xyz, radius=(0.1, 0.2, 0.
             g = torch.relu(_bn2d(p, f"{prefix}bn_blocks.{i}.{j}.",
                                  F.linear(g, w.view(w.shape[0], -1), p[f"{prefix}conv_blocks.{i}.{j}.bias"])))
         outs.append(g.max(2)[0])  # B J C
-    outs.append(node_feat)
-    cat = torch.cat(outs, -1)
-    y = F.linear(cat, p[prefix + "fusion.0.weight"].squeeze(-1), p[prefix + "fusion.0.bias"])
-    return torch.relu(_bn2d(p, prefix + "fusion.1.", y))
+    return outs
 
 
 def bert_layer(p, prefix, h, num_heads=4, eps=1e-12):
