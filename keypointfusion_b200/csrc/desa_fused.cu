@@ -175,9 +175,8 @@ __global__ void __launch_bounds__(DS_NT, 1) desa_prep_kernel(const DesaParams p)
         }
     }
     constexpr int fmt = FMT;
-    SmemOp opW, opA;   // A = the weight planes in sWj, B = joint_agg / jf planes in sAgg
-    opW.hi = smem_u32(sWj); opW.lo = opW.hi + 2048 * 16; opW.lbo = 2048; opW.sbo = 128;
-    opA.hi = smem_u32(sAgg); opA.lo = opA.hi + 512 * 16; opA.lbo = 512; opA.sbo = 128;
+    // A = the weight planes in sWj, B = joint_agg / jf planes in sAgg
+    const SmemOp opW = smem_op_k_outer(smem_u32(sWj), 128, 128), opA = smem_op_k_outer(smem_u32(sAgg), 32, 128);
     const uint32_t id_jf = umma_idesc_f16(128, 32, false, true, fmt, fmt);
     pdl_wait();   // weights only so far
     if (tid < 32) {
@@ -298,11 +297,7 @@ __global__ void __launch_bounds__(DS_NT, 1) desa_prep_kernel(const DesaParams p)
             if (sc < 2) mbar_wait(&w1bar[sc], 0);
             else mbar_wait(&wbar, 1);
             if (elect_one()) {
-                SmemOp w = opW;
-                if (sc < 2) {
-                    w.hi = smem_u32(sW1 + sc * 4096);
-                    w.lo = w.hi + 2048 * 16;
-                }
+                const SmemOp w = sc < 2 ? smem_op_k_outer(smem_u32(sW1 + sc * 4096), 128, 128) : opW;
                 umma_gemm3_ss<128>(tmem0 + 32 * (sc + 1), w, opA, id_jf, false);
             }
             __syncwarp();
@@ -334,10 +329,7 @@ __global__ void __launch_bounds__(DS_NT, 1) desa_prep_kernel(const DesaParams p)
             tc_fence_after();
             mbar_wait(&w1bar[0], 1);
             if (elect_one()) {
-                SmemOp w = opW;
-                w.hi = smem_u32(sW1);
-                w.lo = w.hi + 2048 * 16;
-                umma_gemm3_ss<128>(tmem0 + 32, w, opA, id_jf, false);
+                umma_gemm3_ss<128>(tmem0 + 32, smem_op_k_outer(smem_u32(sW1), 128, 128), opA, id_jf, false);
                 umma_commit(&mma_bar);
             }
             __syncwarp();
@@ -593,22 +585,18 @@ __global__ void __launch_bounds__(DS_TILE_NT, 1) desa_tile_kernel(const DesaPara
                         if (s + 1 < i1) {   // layer 1 of tile s + 1: D1[c][row] = W1 [feat - jf | xyz]
                             const uint32_t X = smem_u32(sX + ((s + 1) % 3) * DS_XBUF);
                             const uint32_t id128 = umma_idesc_f16(128, 128, false, false, fmt, fmt);
-                            // B operand: 128 B between k-chunks, 2048 B (main) / 256 B (tail) between 8-row groups
                             TmemOp a;
                             a.hi = tmem0 + TW1_HI; a.lo = tmem0 + TW1_LO;
-                            SmemOp xb, ta, tb;
-                            xb.hi = X; xb.lo = X + 2048 * 16; xb.lbo = 128; xb.sbo = 2048;
-                            umma_gemm3_ts<128>(tmem0 + ACC1, a, xb, id128, false);
-                            ta.hi = smem_u32(sW1t); ta.lo = ta.hi + 256 * 16; ta.lbo = 2048; ta.sbo = 128;
-                            tb.hi = X + 4096 * 16; tb.lo = tb.hi + 128 * 16; tb.lbo = 0; tb.sbo = 128;   // lbo 0: k-chunk 1 (zero weights) re-reads chunk 0
-                            umma_gemm3_ss<16>(tmem0 + ACC1, ta, tb, id128, true);
+                            umma_gemm3_ts<128>(tmem0 + ACC1, a, smem_op_mn_outer(X, 128, 128), id128, false);
+                            SmemOp tb = smem_op_k_outer(X + 4096 * 16, 128, 8);   // the tail's one stored k-chunk
+                            tb.lbo = 0;   // k-chunk 1 (zero weights) re-reads chunk 0
+                            umma_gemm3_ss<16>(tmem0 + ACC1, smem_op_k_outer(smem_u32(sW1t), 128, 16), tb, id128, true);
                             umma_commit(&g1_bar);
                         }
                         if (s >= i0) {   // layer 2 of tile s: D2[c][row] = W2 h
                             TmemOp a;
                             a.hi = tmem0 + TW2_HI; a.lo = tmem0 + TW2_LO;
-                            SmemOp hb;
-                            hb.hi = smem_u32(sX + (s % 3) * DS_XBUF); hb.lo = hb.hi + 2048 * 16; hb.lbo = 2048; hb.sbo = 128;
+                            const SmemOp hb = smem_op_k_outer(smem_u32(sX + (s % 3) * DS_XBUF), 128, 128);
                             umma_gemm3_ts<128>(tmem0 + ACC2, a, hb, umma_idesc_f16(128, 128, false, true, fmt, fmt), false);
                             umma_commit(&g2_bar);
                         }

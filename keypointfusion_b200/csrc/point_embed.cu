@@ -386,14 +386,10 @@ __global__ void __launch_bounds__(PE_NT, 1) point_embed_kernel(const PointParams
             if (elect_one()) {
                 const uint32_t id64 = umma_idesc_f16(128, PE_TP, false, false, fmt, fmt);
                 TmemOp a;
-                SmemOp xb;
-                // B operands: 128 B between k-chunks, 4096 / 2048 B between 8-point groups
                 a.hi = tmem0 + PE_W1H; a.lo = tmem0 + PE_W1L;
-                xb.hi = smem_u32(sX1); xb.lo = xb.hi + 2048 * 16; xb.lbo = 128; xb.sbo = 4096;
-                umma_gemm3_ts<256>(tmem0 + PE_ACC1, a, xb, id64, false);
+                umma_gemm3_ts<256>(tmem0 + PE_ACC1, a, smem_op_mn_outer(smem_u32(sX1), PE_TP, 256), id64, false);
                 a.hi = tmem0 + PE_W2H; a.lo = tmem0 + PE_W2L;
-                xb.hi = smem_u32(sX2); xb.lo = xb.hi + 1024 * 16; xb.lbo = 128; xb.sbo = 2048;
-                umma_gemm3_ts<128>(tmem0 + PE_ACC2, a, xb, id64, false);
+                umma_gemm3_ts<128>(tmem0 + PE_ACC2, a, smem_op_mn_outer(smem_u32(sX2), PE_TP, 128), id64, false);
                 umma_commit(&mma_bar);
             }
             __syncwarp();
@@ -472,8 +468,7 @@ __global__ void __launch_bounds__(PE_NT, 1) point_embed_kernel(const PointParams
             if (elect_one()) {   // D[c][j] = sum_n e[n][c] p[n][j]
                 TmemOp a;
                 a.hi = tmem0 + PE_EH; a.lo = tmem0 + PE_EL;
-                SmemOp pb;
-                pb.hi = smem_u32(sP); pb.lo = pb.hi + 256 * 16; pb.lbo = 512; pb.sbo = 128;
+                const SmemOp pb = smem_op_k_outer(smem_u32(sP), 32, PE_TP);
                 umma_gemm3_ts<PE_TP>(tmem0 + PE_ACC3, a, pb, umma_idesc_f16(128, 32, false, true, fmt, fmt), false);
                 umma_commit(&mma_bar);
             }

@@ -189,14 +189,11 @@ __global__ void __launch_bounds__(K5_NT, 1) spatial_aggregate_tc_kernel(const Sp
         if (warp_u == 0) {
             tc_fence_after();
             if (elect_one()) {
-                // GEMM A: A = F tile MN-major (LBO 2048 between channel groups, SBO 128 between cell groups), bf16 plane(s);
-                //         B = Wa's feature part, three bf16 planes
-                const uint32_t fa = smem_u32(cur);
-                umma_gemm_map_x3(tmem0 + ACC1, fa, has_lo ? fa + 2048 * 16 : 0u, 2048, 128, smem_u32(sWa), 512 * 16, 512, 128,
+                // GEMM A: A = F tile MN-major, bf16 plane(s); B = Wa's feature part, three bf16 planes
+                const SmemOp fa = smem_op_k_outer(smem_u32(cur), 128, 128), wa = smem_op_k_outer(smem_u32(sWa), 32, 128);
+                umma_gemm_map_x3(tmem0 + ACC1, fa.hi, has_lo ? fa.lo : 0u, fa.lbo, fa.sbo, wa.hi, 32 * 128 * 2, wa.lbo, wa.sbo,
                                  umma_idesc_f16(128, 32, true, false, FMT_BF16, FMT_BF16), 128, false);
-                SmemOp a, bo;
-                a.hi = smem_u32(sHm); a.lo = a.hi + 512 * 16; a.lbo = 2048; a.sbo = 128;
-                bo.hi = smem_u32(sWa + 1536); bo.lo = bo.hi + 128 * 16; bo.lbo = 512; bo.sbo = 128;
+                const SmemOp a = smem_op_k_outer(smem_u32(sHm), 128, 32), bo = smem_op_k_outer(smem_u32(sWa + 1536), 32, 32);
                 umma_gemm3_ss<32>(tmem0 + ACC1, a, bo, umma_idesc_f16(128, 32, false, false, fmt, fmt), true);
                 umma_commit(&mma_bar);
             }
@@ -234,9 +231,9 @@ __global__ void __launch_bounds__(K5_NT, 1) spatial_aggregate_tc_kernel(const Sp
         if (warp_u == 0) {
             tc_fence_after();
             if (elect_one()) {
-                // GEMM B: A = relu(F) tile read K-major (K = cells): LBO 128 between cell groups, SBO 2048 between channel groups
-                const uint32_t fr = smem_u32(sFr);
-                umma_gemm_map_x3(tmem0 + ACC2, fr, has_lo ? fr + 2048 * 16 : 0u, 128, 2048, smem_u32(sG), 512 * 16, 512, 128,
+                // GEMM B: A = relu(F) tile read K-major (K = cells); B = G, three bf16 planes
+                const SmemOp fr = smem_op_mn_outer(smem_u32(sFr), 128, 128), gb = smem_op_k_outer(smem_u32(sG), 32, 128);
+                umma_gemm_map_x3(tmem0 + ACC2, fr.hi, has_lo ? fr.lo : 0u, fr.lbo, fr.sbo, gb.hi, 32 * 128 * 2, gb.lbo, gb.sbo,
                                  umma_idesc_f16(128, 32, false, true, FMT_BF16, FMT_BF16), 128, t > t_begin);
                 umma_commit(&mma_bar);
             }

@@ -2,12 +2,10 @@
 // synchronisation and TMEM allocation, TMEM <-> register moves, and the split-precision operand planes.
 // Descriptor bit layouts follow the PTX ISA "tcgen05 matrix descriptor" / "instruction descriptor" tables.
 //
-// Shared-memory operand layout used everywhere in this repo: SWIZZLE_NONE ("interleaved") canonical layout with
-// 8x16-byte core matrices stored chunk-major:
-//   K-major  operand X[rows][K] (bf16): element (r,k) at  (k/8)*LBO + (r/8)*SBO + (r%8)*16 + (k%8)*2
-//            with SBO = 128, LBO = rows*16  ==  uint4 smem[K/8][rows]   (one 16-byte chunk = 8 consecutive k)
-//   MN-major operand Y[K][MN]  (bf16): element (k,n) at  (k/8)*LBO + (n/8)*SBO + (k%8)*16 + (n%8)*2
-//            with SBO = 128, LBO = (MN/8)*128 == uint4 smem[K/8][MN/8][8]  (one chunk = 8 consecutive mn)
+// Shared-memory operands use the SWIZZLE_NONE ("interleaved") canonical layout of 8x16-byte core matrices:
+//   K-major  operand X[MN][K] (16-bit): element (r,k) at  (k/8)*LBO + (r/8)*SBO + (r%8)*16 + (k%8)*2   (one chunk = 8 consecutive k)
+//   MN-major operand Y[K][MN] (16-bit): element (k,n) at  (k/8)*LBO + (n/8)*SBO + (k%8)*16 + (n%8)*2   (one chunk = 8 consecutive mn)
+// i.e. LBO is the byte stride between core matrices along K and SBO the one along MN; the SmemOp constructors below set both.
 // One tcgen05.mma consumes K=16 (two 8-k groups); the descriptor start address advances by 2*LBO per step.
 //
 // Split-precision GEMMs: an fp32 operand x is carried as TWO 16-bit planes  x = hi + lo  (hi = rn16(x), lo = rn16(x - hi)),
@@ -45,6 +43,12 @@ struct SmemOp {
     uint32_t hi, lo;      // shared-memory byte addresses of the two planes
     uint32_t lbo, sbo;    // descriptor strides (layout above)
 };
+// An MN x K operand at `hi`, planes of MN*K*2 bytes each, the lo plane right after the hi plane.  The kernels store the core
+// matrices in one of two orders, with the same strides for K-major and MN-major operands:
+//   k_outer : uint4 [K/8][MN/8][8]   LBO = MN*16, SBO = 128
+//   mn_outer: uint4 [MN/8][K/8][8]   LBO = 128,   SBO = K*16
+__device__ __forceinline__ constexpr SmemOp smem_op_k_outer(uint32_t hi, uint32_t mn, uint32_t k) { return {hi, hi + mn * k * 2, mn * 16, 128}; }
+__device__ __forceinline__ constexpr SmemOp smem_op_mn_outer(uint32_t hi, uint32_t mn, uint32_t k) { return {hi, hi + mn * k * 2, 128, k * 16}; }
 // A operand planes in tensor memory: 16-bit elements, K/2 columns per plane
 struct TmemOp {
     uint32_t hi, lo;      // TMEM addresses (lane 0 of the operand, first column); lo == 0xffffffff: no lo plane
@@ -55,6 +59,7 @@ constexpr uint32_t NO_PLANE = 0xffffffffu;
 // along K, by a constant that folds into an immediate once the K loop is unrolled; the 64-bit add-with-carry, the per-iteration
 // R2UR of the accumulator address / instruction descriptor and the loop control of the rolled form cost ~16 uniform-datapath
 // instructions per MMA (~42 cycles per MMA measured, against a 16-cycle tensor-pipe floor at N = 32).
+// 64-bit descriptor: start[0,14) | LBO[16,30) | SBO[32,46) | version=1 [46,48) | swizzle none
 __device__ __forceinline__ uint32_t desc_lo(uint32_t smem_addr, uint32_t lbo_bytes) {
     return ((smem_addr >> 4) & 0x3FFFu) | (((lbo_bytes >> 4) & 0x3FFFu) << 16);
 }
@@ -135,10 +140,8 @@ __device__ __forceinline__ void umma_gemm3_ts(uint32_t tmem_d, const TmemOp a, c
 }
 
 // ---- the rolled single-plane form with a 64-bit descriptor (K5's map GEMMs and the bring-up self-test)
-// 64-bit shared-memory matrix descriptor: start[0,14) | LBO[16,30) | SBO[32,46) | version=1 [46,48) | swizzle none
 __device__ __forceinline__ uint64_t umma_smem_desc(uint32_t smem_addr, uint32_t lbo_bytes, uint32_t sbo_bytes) {
-    return (uint64_t)((smem_addr >> 4) & 0x3FFFu) | ((uint64_t)((lbo_bytes >> 4) & 0x3FFFu) << 16) |
-           ((uint64_t)((sbo_bytes >> 4) & 0x3FFFu) << 32) | (1ull << 46);
+    return ((uint64_t)desc_hi(sbo_bytes) << 32) | desc_lo(smem_addr, lbo_bytes);
 }
 
 __device__ __forceinline__ void umma_bf16(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, bool accumulate) {

@@ -216,9 +216,7 @@ __global__ void __launch_bounds__(TS_NT, 1) token_stack_kernel(const TokParams p
         for (int h = 0; h < 2; ++h) {
             wait_full(e + h);
             tc_fence_after();
-            SmemOp a, bo;
-            a.hi = slot_addr(e + h); a.lo = a.hi + 16384; a.lbo = 2048; a.sbo = 128;
-            bo.hi = smem_u32(act) + h * 4096; bo.lo = bo.hi + TS_PLANE * 16; bo.lbo = 512; bo.sbo = 128;
+            const SmemOp a = smem_op_k_outer(slot_addr(e + h), 128, 64), bo = smem_op_k_outer(smem_u32(act) + h * 4096, 32, 128);
             umma_gemm3_ss<64>(tmem0 + acc, a, bo, id, accumulate || h > 0);
             umma_commit(&empty[(e + h) & (TS_RING - 1)]);
         }
@@ -364,9 +362,7 @@ __global__ void __launch_bounds__(TS_NT, 1) token_stack_kernel(const TokParams p
                     if (shift > 0) {   // K tail: A = W_emb[:, :shift] (zero padded to 16) [2 chunks][128 rows], B = bufAt K-major
                         wait_full(g + 2);
                         tc_fence_after();
-                        SmemOp a, bo;
-                        a.hi = slot_addr(g + 2); a.lo = a.hi + 256 * 16; a.lbo = 2048; a.sbo = 128;
-                        bo.hi = smem_u32(bufAt); bo.lo = bo.hi + 64 * 16; bo.lbo = 512; bo.sbo = 128;
+                        const SmemOp a = smem_op_k_outer(slot_addr(g + 2), 128, 16), bo = smem_op_k_outer(smem_u32(bufAt), 32, 16);
                         umma_gemm3_ss<16>(tmem0 + ACC_X, a, bo, umma_idesc_f16(128, 32, false, false, fmt, fmt), true);
                         umma_commit(&empty[(g + 2) & (TS_RING - 1)]);
                     }
@@ -439,9 +435,7 @@ __global__ void __launch_bounds__(TS_NT, 1) token_stack_kernel(const TokParams p
         if (warp_u == 0) {
             tc_fence_after();
             if (elect_one()) {
-                SmemOp a, bo;
-                a.hi = smem_u32(bufQ); a.lo = a.hi + TS_PLANE * 16; a.lbo = 2048; a.sbo = 128;
-                bo.hi = smem_u32(bufK); bo.lo = bo.hi + TS_PLANE * 16; bo.lbo = 2048; bo.sbo = 128;
+                const SmemOp a = smem_op_k_outer(smem_u32(bufQ), 128, 32), bo = smem_op_k_outer(smem_u32(bufK), 128, 32);
                 umma_gemm3_ss<32>(tmem0 + ACC_S, a, bo, umma_idesc_f16(128, 128, true, true, fmt, fmt), false);
                 umma_commit(&bars[0]);
                 issue_proj(ACC_V, kv_src, g + 4, false);
@@ -491,8 +485,7 @@ __global__ void __launch_bounds__(TS_NT, 1) token_stack_kernel(const TokParams p
             if (elect_one()) {
                 TmemOp a;
                 a.hi = tmem0 + VT_HI; a.lo = tmem0 + VT_LO;
-                SmemOp bo;
-                bo.hi = smem_u32(bufQ); bo.lo = bo.hi + TS_PLANE * 16; bo.lbo = 2048; bo.sbo = 128;
+                const SmemOp bo = smem_op_k_outer(smem_u32(bufQ), 128, 32);
                 umma_gemm3_ts<32>(tmem0 + ACC_O, a, bo, umma_idesc_f16(128, 128, false, false, fmt, fmt), false);
                 umma_commit(&bars[0]);
             }
@@ -572,22 +565,18 @@ __global__ void __launch_bounds__(TS_NT, 1) token_stack_kernel(const TokParams p
         if (warp_u == 0) {
             tc_fence_after();
             if (elect_one()) {
-                SmemOp a, bo;
-                a.hi = smem_u32(bufX); a.lo = a.hi + TS_PLANE * 16; a.lbo = 512; a.sbo = 128;
                 if (F == 16) {
                     wait_full(g + 8);
                     tc_fence_after();
-                    bo.hi = slot_addr(g + 8); bo.lo = bo.hi + 256 * 16; bo.lbo = 256; bo.sbo = 128;
+                    const SmemOp a = smem_op_k_outer(smem_u32(bufX), 32, 128), bo = smem_op_k_outer(slot_addr(g + 8), 16, 128);
                     umma_gemm3_ss<128>(tmem0 + ACC_F, a, bo, umma_idesc_f16(128, 16, true, false, fmt, fmt), false);
                 } else {
 #pragma unroll 1
                     for (int h = 0; h < 2; ++h) {
                         wait_full(g + 8 + h);
                         tc_fence_after();
-                        SmemOp ah = a;
-                        ah.hi += h * 4096; ah.lo += h * 4096;
-                        bo.hi = slot_addr(g + 8 + h); bo.lo = bo.hi + 16384; bo.lbo = 2048; bo.sbo = 128;
-                        umma_gemm3_ss<64>(tmem0 + ACC_F, ah, bo, umma_idesc_f16(128, 128, true, false, fmt, fmt), h > 0);
+                        const SmemOp a = smem_op_k_outer(smem_u32(bufX) + h * 4096, 32, 128), bo = smem_op_k_outer(slot_addr(g + 8 + h), 128, 64);
+                        umma_gemm3_ss<64>(tmem0 + ACC_F, a, bo, umma_idesc_f16(128, 128, true, false, fmt, fmt), h > 0);
                         umma_commit(&empty[(g + 8 + h) & (TS_RING - 1)]);
                     }
                 }
@@ -634,11 +623,9 @@ __global__ void __launch_bounds__(TS_NT, 1) token_stack_kernel(const TokParams p
         if (warp_u == 0) {
             tc_fence_after();
             if (elect_one()) {
-                SmemOp a, bo;
-                bo.hi = smem_u32(bufY); bo.lo = bo.hi + TS_PLANE * 16; bo.lbo = 512; bo.sbo = 128;
                 const uint32_t id = umma_idesc_f16(128, 32, false, false, fmt, fmt);
                 if (F == 16) {
-                    a.hi = slot_addr(g + 8) + 512 * 16; a.lo = a.hi + 256 * 16; a.lbo = 2048; a.sbo = 128;
+                    const SmemOp a = smem_op_k_outer(slot_addr(g + 8) + 512 * 16, 128, 16), bo = smem_op_k_outer(smem_u32(bufY), 32, 128);
                     umma_gemm3_ss<16>(tmem0 + ACC_X, a, bo, id, false);
                     umma_commit(&empty[(g + 8) & (TS_RING - 1)]);
                 } else {
@@ -646,10 +633,8 @@ __global__ void __launch_bounds__(TS_NT, 1) token_stack_kernel(const TokParams p
                     for (int h = 0; h < 2; ++h) {
                         wait_full(g + 10 + h);
                         tc_fence_after();
-                        a.hi = slot_addr(g + 10 + h); a.lo = a.hi + 16384; a.lbo = 2048; a.sbo = 128;
-                        SmemOp bh = bo;
-                        bh.hi += h * 4096; bh.lo += h * 4096;
-                        umma_gemm3_ss<64>(tmem0 + ACC_X, a, bh, id, h > 0);
+                        const SmemOp a = smem_op_k_outer(slot_addr(g + 10 + h), 128, 64), bo = smem_op_k_outer(smem_u32(bufY) + h * 4096, 32, 128);
+                        umma_gemm3_ss<64>(tmem0 + ACC_X, a, bo, id, h > 0);
                         umma_commit(&empty[(g + 10 + h) & (TS_RING - 1)]);
                     }
                 }

@@ -48,8 +48,8 @@ umma_selftest_kernel(const __nv_bfloat16* __restrict__ A, const __nv_bfloat16* _
     tc_fence_after();
     const uint32_t tmem = tmem_slot;
     if (tid == 0) {
-        const uint32_t a_lbo = a_mn ? 16 * 128 : 128 * 16, b_lbo = b_mn ? (N / 8) * 128 : N * 16;
-        umma_gemm(tmem, smem_u32(sA), a_lbo, 128, smem_u32(sB), b_lbo, 128, umma_idesc_f16(128, N, a_mn != 0, b_mn != 0, FMT_BF16, FMT_BF16), K, false);
+        const SmemOp a = smem_op_k_outer(smem_u32(sA), 128, K), b = smem_op_k_outer(smem_u32(sB), N, K);   // either major
+        umma_gemm(tmem, a.hi, a.lbo, a.sbo, b.hi, b.lbo, b.sbo, umma_idesc_f16(128, N, a_mn != 0, b_mn != 0, FMT_BF16, FMT_BF16), K, false);
         umma_commit(&bar);
     }
     mbar_wait(&bar, 0);

@@ -59,9 +59,9 @@ umma_split_selftest_kernel(const float* __restrict__ A, const float* __restrict_
     __syncthreads();
     tc_fence_after();
     const uint32_t idesc = umma_idesc_f16(128, N, false, false, FMT, FMT);
-    SmemOp a, b;
-    a.hi = smem_u32(sAh); a.lo = a_exact ? 0u : smem_u32(sAl); a.lbo = 128 * 16; a.sbo = 128;
-    b.hi = smem_u32(sBh); b.lo = smem_u32(sBl); b.lbo = (uint32_t)N * 16; b.sbo = 128;
+    SmemOp a = smem_op_k_outer(smem_u32(sAh), 128, K);   // lo = sAl
+    if (a_exact) a.lo = 0;
+    const SmemOp b = smem_op_k_outer(smem_u32(sBh), N, K);
     TmemOp at;
     at.hi = tmem + TA_HI; at.lo = a_exact ? NO_PLANE : tmem + TA_LO;
     uint32_t phase = 0;
