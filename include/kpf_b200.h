@@ -294,6 +294,27 @@ int kpf_joints_to_frame(const float* joints, const float* center, const float* c
  * after GFM.rigid_align (similarity Procrustes, 3x3 SVD per sample in fp64 on the device). */
 int kpf_eval_errors(const float* pred, const float* gt, const float* cube, int B, int J, float* err, float* pa_err, cudaStream_t stream);
 
+/* ---- 8f-4 evaluation accumulated on the device: replaces the per-batch .cpu(), per-sample numpy SVD loop and host-side sums of
+ * train.py:330-396 (Trainer.test), :470-488 (xyz2error) and util/generateFeature.py:681-703 (rigid_align).
+ * pred [S,B,J,3] f32 (S joint sets of the same samples, stacked), gt [B,J,3] f32, cube [B,3] f32, valid [B] u8 (0 = padding row,
+ * contributes nothing; NULL = all valid), thresholds [T] f32 mm, strictly increasing.  S <= 8, 3 <= J <= 32, 1 <= T <= 256, else
+ * KPF_ERR_BAD_ARGUMENT before any launch.  One kernel, no other launch; it only ADDS to acc (zero it to start a new evaluation).
+ * acc [S][R] int64, R = 1 + 4J + 2(T+1); row s (joint set s) is
+ *   [0]                samples     valid samples seen
+ *   [1, 1+J)           sum_err     per joint, sum of round(min(e, 2^20) * 2^20) over finite e: fixed point, 2^20 units per mm
+ *   [1+J, 1+2J)        sum_pa      the same for the Procrustes-aligned error
+ *   [1+2J, 1+3J)       nonfinite_err  per joint, count of NaN / inf errors (these add nothing to the sums)
+ *   [1+3J, 1+4J)       nonfinite_pa
+ *   [1+4J, +T+1)       hist_err    bin k < T counts thr[k-1] < e <= thr[k] (bin 0: e <= thr[0]); bin T counts e > thr[T-1] and
+ *                                  non-finite e (fp32 compares)
+ *   [.., +T+1)         hist_pa
+ * e is exactly the fp32 value kpf_eval_errors stores for that (sample, joint); the conversion (double)min(e, 2^20 mm) * 2^20 is
+ * exact in fp64 and rounded to nearest even, so every total is an integer sum: exact and independent of batch order, batch
+ * split, streams in flight or ranks (sum the accumulators of several ranks).  Headroom: a joint adds at most 2^40, so a sum slot
+ * holds 2^23 (~8.4 M) samples even if every error is clamped, and ~8.6 G samples at <= 1 m per joint. */
+int kpf_eval_accumulate(const float* pred, const float* gt, const float* cube, const uint8_t* valid, const float* thresholds, int S, int B,
+                        int J, int T, long long* acc, cudaStream_t stream);
+
 /* ---- bring-up self-test of the tcgen05 primitives (csrc/tcgen05.cuh): D[128,N] f32 = A * B^T with bf16 operands.
  * a_mn == 0: A is [128,K] row-major (K-major operand), else A is given transposed [K,128] (MN-major operand);
  * b_mn == 0: B is [N,K] row-major, else B is given as [K,N]. */

@@ -9,9 +9,10 @@ and :395 (the `loader` helper object).
 
 Conventions: optional OUTPUTS do not exist in the op schema, so an absent tensor result is returned as an empty (numel 0) tensor;
 optional INPUTS are `Optional[Tensor]`.  Packed weights travel as plain tensors (+ ints).  No op aliases an input; `desa_fused`
-declares that it writes into `e` (it appends the joints' rows behind the points of the same buffer).
+declares that it writes into `e` (it appends the joints' rows behind the points of the same buffer), `eval_accumulate` that it
+adds into `acc`.
 """
-from typing import Optional, Tuple
+from typing import List, Optional, Tuple
 
 import torch
 from torch import Tensor
@@ -383,6 +384,17 @@ def eval_errors(pred: Tensor, gt: Tensor, cube: Tensor) -> Tuple[Tensor, Tensor]
 def _(pred, gt, cube):
     B, J = pred.shape[:2]
     return pred.new_empty(B, J, dtype=torch.float32), pred.new_empty(B, J, dtype=torch.float32)
+
+
+@_op("eval_accumulate", mutates=("acc",))
+def eval_accumulate(acc: Tensor, pred: Tensor, gt: Tensor, cube: Tensor, valid: Optional[Tensor], thresholds: List[float]) -> None:
+    """Adds the stacked joint sets pred [S,B,J,3] into the int64 accumulator `acc` (ops.eval_accumulate)."""
+    ops.eval_accumulate(acc, pred, gt, cube, valid, thresholds)
+
+
+@eval_accumulate.register_fake
+def _(acc, pred, gt, cube, valid, thresholds):
+    ops.check_eval_accumulate(acc, pred, gt, cube, valid, ops.eval_thresholds(thresholds))
 
 
 # ------------------------------------------------------------------------------------------------ 8f-3 frame front end

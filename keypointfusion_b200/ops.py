@@ -6,6 +6,7 @@ launches the kernel on `torch.cuda.current_stream()`.  There is NO fallback: non
 import ctypes
 import os
 
+import numpy as np
 import torch
 
 from . import _lib
@@ -999,3 +1000,75 @@ def eval_errors(pred, gt, cube, aligned=True):
     pa = torch.empty(B, J, device=pred.device, dtype=torch.float32) if aligned else None
     _call("kpf_eval_errors", _p(pred), _p(gt), _p(cube), B, J, _p(err), _p(pa))
     return err, pa
+
+
+EVAL_MAX_SETS, EVAL_MAX_JOINTS, EVAL_MAX_THRESHOLDS = 8, 32, 256
+EVAL_SCALE = 2 ** 20   # fixed-point units per mm in the accumulator's error sums (include/kpf_b200.h)
+
+
+def eval_row_length(J, T):
+    """int64 slots per joint set of the eval_accumulate accumulator: samples | sum err [J] | sum pa [J] | nonfinite err [J] |
+    nonfinite pa [J] | hist err [T+1] | hist pa [T+1]."""
+    return 1 + 4 * J + 2 * (T + 1)
+
+
+def eval_thresholds(thresholds):
+    """PCK thresholds in mm (a sequence or a CPU tensor) -> tuple of their fp32 values.  ValueError unless there are 1..256 of them,
+    finite and strictly increasing after rounding to fp32.  Host values only: checking a device tensor would need a synchronising read."""
+    if torch.is_tensor(thresholds):
+        if thresholds.device.type != "cpu":
+            raise ValueError("thresholds must be host values (a sequence or a CPU tensor)")
+        thresholds = thresholds.numpy()   # no torch dispatch: works under FakeTensorMode and during graph capture
+    t = np.asarray(thresholds, dtype=np.float32).reshape(-1)
+    if not 1 <= t.size <= EVAL_MAX_THRESHOLDS:
+        raise ValueError(f"{t.size} thresholds: 1..{EVAL_MAX_THRESHOLDS} are supported")
+    if not np.all(np.isfinite(t)) or not np.all(t[1:] > t[:-1]):
+        raise ValueError("thresholds must be finite and strictly increasing (as fp32 values)")
+    return tuple(float(x) for x in t)
+
+
+def check_eval_accumulate(acc, pred, gt, cube, valid, thresholds):
+    """ValueError for any argument kpf_eval_accumulate would refuse, from shapes and dtypes alone (no device read).
+    pred: the stacked joint sets [S,B,J,3]."""
+    if pred.dim() != 4 or pred.shape[-1] != 3:
+        raise ValueError(f"joint sets {tuple(pred.shape)}: expected [S,B,J,3]")
+    S, B, J = (int(x) for x in pred.shape[:3])
+    if not 1 <= S <= EVAL_MAX_SETS:
+        raise ValueError(f"{S} joint sets: 1..{EVAL_MAX_SETS} are supported")
+    if not 3 <= J <= EVAL_MAX_JOINTS:
+        raise ValueError(f"{J} joints: 3..{EVAL_MAX_JOINTS} are supported")
+    if tuple(gt.shape) != (B, J, 3):
+        raise ValueError(f"gt {tuple(gt.shape)} does not match the joint sets' [B,J,3] = {(B, J, 3)}")
+    if tuple(cube.shape) != (B, 3):
+        raise ValueError(f"cube {tuple(cube.shape)}: expected {(B, 3)}")
+    for name, t in (("joint sets", pred), ("gt", gt), ("cube", cube)):
+        if not t.dtype.is_floating_point:
+            raise ValueError(f"{name}: floating-point dtype expected, got {t.dtype}")
+    if valid is not None and (valid.dtype != torch.uint8 or tuple(valid.shape) != (B,)):
+        raise ValueError(f"valid must be a uint8 tensor of shape {(B,)}, got {valid.dtype} {tuple(valid.shape)}")
+    R = eval_row_length(J, len(thresholds))
+    if acc.dtype != torch.int64 or tuple(acc.shape) != (S, R) or not acc.is_contiguous():
+        raise ValueError(f"acc must be a contiguous int64 tensor of shape {(S, R)}, got {acc.dtype} {tuple(acc.shape)}")
+
+
+_thr_cache = {}
+
+
+def eval_accumulate(acc, pred_sets, gt, cube, valid, thresholds):
+    """Add S joint sets' per-joint errors, aligned errors and threshold histograms into `acc` [S, eval_row_length(J, T)] int64
+    (kpf_eval_accumulate: fixed point, exact and order-independent).  pred_sets: a sequence of S tensors [B,J,3] or one [S,B,J,3];
+    gt [B,J,3] and cube [B,3] as for eval_errors; valid [B] uint8 or None; thresholds: host values in mm (eval_thresholds).
+    Validation raises ValueError before any launch; no host synchronisation (capturable: the thresholds' device copy is made once
+    per distinct grid and device, on the first, uncaptured, call)."""
+    pred = pred_sets if torch.is_tensor(pred_sets) else torch.stack([p.float() for p in pred_sets])
+    thr = eval_thresholds(thresholds)
+    check_eval_accumulate(acc, pred, gt, cube, valid, thr)
+    _need_cuda(acc, valid)
+    pred, gt, cube = _f32(pred), _f32(gt), _f32(cube)
+    S, B, J, _ = pred.shape
+    key = (thr, str(acc.device))
+    dthr = _thr_cache.get(key)
+    if dthr is None:
+        dthr = _thr_cache[key] = torch.tensor(thr, dtype=torch.float32, device=acc.device)
+    _call("kpf_eval_accumulate", _p(pred), _p(gt), _p(cube), _p(valid.contiguous() if valid is not None else None), _p(dthr), S, B, J,
+          len(thr), _p(acc))

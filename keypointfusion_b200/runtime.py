@@ -80,6 +80,31 @@ class GraphedFusionPath(_GraphedPath):
         return dict(joints=res[-1], result=res, spatial_weight=sw, pcl=pcl)
 
 
+class GraphedEvalPath(GraphedFusionPath):
+    """GraphedFusionPath that also evaluates the step inside the same graph: after forward_path, `evaluator.update` adds the joint sets
+    of evaluator.stage_names (evaluation.stage_joints) against the ground truth into the evaluator's device accumulator.  Two more
+    inputs: gt [B,J,3] (normalised xyz) and valid [B] uint8.  A final partial batch is padded to B (any rows) with valid = 0 there.
+    Several paths may share one evaluator (PipelinedRunner, OverlappedSteps): its totals do not depend on the order of the steps.
+    `evaluator.summary(group)` reads the result once at the end.  The warm-up steps run at construction leave the accumulator as
+    they found it."""
+    KEYS = GraphedFusionPath.KEYS + ("gt", "valid")
+
+    def __init__(self, net, loader, example, evaluator, **kw):
+        self.evaluator = evaluator
+        before = evaluator.acc.clone()
+        super().__init__(net, loader, example, **kw)
+        evaluator.acc.copy_(before)
+
+    def _run(self):
+        from .evaluation import stage_joints
+        out = super()._run()
+        s = self.static
+        sets = stage_joints(out["result"], s["img"], s["center"], s["M"], s["cube"], s["cam"], self.loader, self.kernel,
+                            names=self.evaluator.stage_names)
+        self.evaluator.update(sets, s["gt"], s["cube"], s["valid"])
+        return out
+
+
 class GraphedFramePath(_GraphedPath):
     """Frames to keypoints as one captured graph: the crop front end (demo_RGBD.Model_RGBD.prepare_batch), the two stock-PyTorch
     backbones, KPFusion.forward_path and joints_to_frame, over static buffers rgb [F,Hf,Wf,3] uint8, depth [F,Hf,Wf] uint16 (or
@@ -239,8 +264,9 @@ class PipelinedRunner:
     `new_host_inputs()` hands the caller a dict of pinned views (one arena): filling those and passing the dict to `submit`
     uploads a step with a single copy; any other dict of host tensors is uploaded tensor by tensor.
 
-    path_cls: GraphedFusionPath (crops + backbone maps in, normalised joints out) or GraphedFramePath (frames, boxes and
-    frame_index in, keypoints in frame pixels and camera mm out); `example` holds that class's KEYS and `kw` go to it."""
+    path_cls: GraphedFusionPath (crops + backbone maps in, normalised joints out), GraphedEvalPath (the same plus gt / valid in,
+    evaluated into kw["evaluator"]) or GraphedFramePath (frames, boxes and frame_index in, keypoints in frame pixels and camera mm
+    out); `example` holds that class's KEYS and `kw` go to it."""
 
     def __init__(self, net, loader, example, path_cls=GraphedFusionPath, **kw):
         dev = next(net.parameters()).device
